@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torch.distributed.run)
   python bench.py --impl reference ...                     (CPU arm: the oracle port of circKit's path)
+  python bench.py ... --dump-outputs DIR                   (also write the last timed step's results as DIR/*.npy)
 
 A step = one pass of the hot path over one batch of synthetic records:
   config 2 of BASELINE.json (default): `circkit uniq` on 10 M circRNA-length records (log-uniform
@@ -71,7 +72,13 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work per cpu_baseline measurement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs), so that "
+                         "two builds can be compared output for output on the same inputs; B200 arm only")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs: the reference arm times a host-side sample, not the B200 path")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -173,6 +180,46 @@ def cpu_faithful_footnote(w, seed):
 
 
 # ------------------------------------------------------------------------------------------------
+DUMP_RECORDS = 1 << 18      # --dump-outputs: per-record results of at most this many records
+DUMP_BASES = 1 << 21        # --dump-outputs: canonical bytes of at most this many bases
+
+
+def dump_outputs(dirname, prefix, n, per_record, canon=None):
+    """--dump-outputs: the results of the last timed step, for all n records or, above DUMP_RECORDS, for a sample drawn with
+    a fixed seed, as DIR/<prefix><name>.npy:
+      index            the sampled record indices (float64)
+      <name>           per_record[name][index] for each device array of n per-record results (float64: exact below 2^53);
+                       the 64-bit hash as hash_hi and hash_lo, its two 32-bit halves
+      canonical_bytes  (canon given) the canonical bytes of the first sampled records that fit DUMP_BASES, concatenated
+                       (float32); per_record["length"] splits them
+    canon = (out, offsets): the aligned output arena, record i at 32 * ((offsets[i] >> 5) + i)."""
+    import numpy as np
+    import torch
+    idx = np.arange(n) if n <= DUMP_RECORDS else np.sort(np.random.default_rng(0).choice(n, DUMP_RECORDS, replace=False))
+    res = {"index": idx.astype(np.float64)}
+    didx = torch.from_numpy(idx).to(next(iter(per_record.values())).device)
+    for name, t in per_record.items():
+        v = t[:n][didx].cpu().numpy()
+        if name == "hash":
+            u = v.view(np.uint64)
+            res["hash_hi"], res["hash_lo"] = (u >> np.uint64(32)).astype(np.float64), (u & np.uint64(0xFFFFFFFF)).astype(np.float64)
+        else:
+            res[name] = v.astype(np.float64)
+    if canon is not None:
+        out, offsets = canon
+        lens = per_record["length"][:n][didx].long()
+        ends = torch.cumsum(lens, 0)
+        m = int((ends <= DUMP_BASES).sum().item())
+        starts = 32 * ((offsets[didx[:m]] >> 5) + didx[:m])
+        total = int(ends[m - 1].item()) if m else 0
+        pos = torch.repeat_interleave(starts - (ends[:m] - lens[:m]), lens[:m]) + torch.arange(total, device=out.device)
+        res["canonical_bytes"] = out[pos].cpu().numpy().astype(np.float32)
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in res.items():
+        np.save(os.path.join(dirname, prefix + name + ".npy"), a)
+
+
+# ------------------------------------------------------------------------------------------------
 def bench_monomerize(args):
     """`--workload mono`: `monomerize` (SURVEY 8f row 4) on one GPU.  1 M concatemers (2.3 copies of a 250-400 nt unit, 1 %
     substitutions; `--records` overrides), seed 10, min identity 0.95 (the reference CLI's default seed, its tests' identity).
@@ -219,6 +266,8 @@ def bench_monomerize(args):
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "", n, {"end_index": out})       # -1: no monomer found
     # end to end: host buffers in, end indices out
     h_raw = raw.cpu().pin_memory(); h_off = offsets.cpu().pin_memory()
     h_out = torch.empty(n, dtype=torch.int32).pin_memory()
@@ -661,8 +710,9 @@ def global_first_index_check(ctx, D, torch, dist, dev, rank, world, R, hash_loca
     return ok, uniq
 
 
-def b200_arm(args, wname, R, rank, local_rank, world, dev, steps, warmup, want_e2e, want_cpu, scaling):
+def b200_arm(args, wname, R, rank, local_rank, world, dev, steps, warmup, want_e2e, want_cpu, scaling, dump_prefix=""):
     """One workload on this rank's shard of R records: resident measurement (value, roofline), optional e2e and CPU legs.
+    With --dump-outputs, rank 0 writes its shard's results of the last timed step as <dump_prefix><name>.npy.
     Returns the JSON line as a dict on rank 0 (None elsewhere)."""
     import numpy as np
     import torch
@@ -888,6 +938,13 @@ def b200_arm(args, wname, R, rank, local_rank, world, dev, steps, warmup, want_e
     ktimes = D.kernel_times(ctx)
     ctx._lib.ck_kernel_timing(ctx.handle, 0)
     D.check(ctx, ws)
+    if args.dump_outputs and rank == 0:
+        per_record = {"length": lens_out if raw_dev is not None else lens, "start": outs_last.start, "strand": outs_last.strand}
+        if outs_last.hash is not None:
+            per_record["hash"] = outs_last.hash
+        if w["uniq"]:
+            per_record["first_index"] = first
+        dump_outputs(args.dump_outputs, dump_prefix, R, per_record, canon=(outs_last.out, batch.offsets))
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -1050,7 +1107,7 @@ def main():
         total5 = args.c5_records
         R5 = total5 // world
         sub = b200_arm(args, "c5", R5, rank, local_rank, world, dev, max(2, min(args.steps, 5)), 3,
-                       want_e2e=False, want_cpu=False, scaling="strong")
+                       want_e2e=False, want_cpu=False, scaling="strong", dump_prefix="config5_")
         if rank == 0:
             line["config5"] = {k: sub[k] for k in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "scaling",
                                                     "gbases_per_s", "gpu_launches", "global_unique_records", "global_parity")}

@@ -9,15 +9,16 @@ Sources
 * fixtures/            -- byte copies of the reference's tests/examples/<dir>/{in,out}.fasta for
                           the canonicalize/uniq path (test DATA, not source), plus test.fasta and the
                           676-record real-monomer corpus (nim_cated.../out.fasta) used as extra input.
-* xxh3_vectors.json    -- XXH3-64 (seed 0) of deterministic inputs at every length class, produced by
-                          python-xxhash 3.7.0 (libxxhash 0.8.2): an independent implementation of the
-                          algorithm xxhash-rust 0.8.6 implements (src/uniq.rs:45).
+* xxh3_vectors.json    -- XXH3-64 (seed 0) of deterministic inputs at every length class and of seeded
+                          random bytes, produced by python-xxhash 3.7.0 (libxxhash 0.8.2): an independent
+                          implementation of the algorithm xxhash-rust 0.8.6 implements (src/uniq.rs:45).
 * oracle_cli/*.out     -- the ORACLE's byte-exact CLI output for each fixture input (the reference's
                           out.fasta files lack the final newline the program writes, src/canonicalize.rs:37,
                           so byte-exact expectations have to come from the source-following oracle).
 """
 import json
 import os
+import random
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -68,11 +69,18 @@ def xxh3_vectors():
         raw = bytes((i * 131 + 17 + L) & 0xFF for i in range(L))
         vec.append({"len": L, "kind": "dna", "xxh3_64": "%016x" % xxhash.xxh3_64_intdigest(dna)})
         vec.append({"len": L, "kind": "raw", "xxh3_64": "%016x" % xxhash.xxh3_64_intdigest(raw)})
+    # random bytes: one random.Random(11) stream, consumed length after length in this order
+    rng = random.Random(11)
+    rnd = []
+    for L in list(range(0, 300)) + [1023, 1024, 1025, 2048, 4097, 70000]:
+        data = bytes(rng.getrandbits(8) for _ in range(L))
+        rnd.append({"len": L, "xxh3_64": "%016x" % xxhash.xxh3_64_intdigest(data)})
     return {"generator": "python-xxhash %s / libxxhash %s" % (xxhash.VERSION, xxhash.XXHASH_VERSION),
             "dna": "bytes(b'ACGT'[(i*7 + (i>>3)*3 + L) & 3] for i in range(L))",
             "raw": "bytes((i*131 + 17 + L) & 0xFF for i in range(L))",
+            "random": "rng = random.Random(11), then for each length in order: bytes(rng.getrandbits(8) for _ in range(L))",
             "known": {"": "2d06800538d394c2", "AAT": "a6ab697c798b7cdd"},
-            "vectors": vec}
+            "vectors": vec, "random_vectors": rnd}
 
 
 def oracle_cli():

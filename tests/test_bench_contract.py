@@ -31,6 +31,41 @@ def test_reference_arm_line_on_cpu():
     assert j["value"] > 0 and j["ms_per_step"] > 0
 
 
+def test_dump_outputs_format(tmp_path, monkeypatch):
+    """--dump-outputs on host tensors: a seeded sample of the records, exact hash halves, the canonical bytes of the first
+    sampled records cut out of the aligned arena (record i at 32 * ((offsets[i] >> 5) + i)), at most DUMP_BASES of them."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_RECORDS", 700)
+    monkeypatch.setattr(bench, "DUMP_BASES", 30000)
+    rng = np.random.default_rng(5)
+    n = 5000
+    lens = rng.integers(1, 300, n)
+    off = np.zeros(n + 1, np.int64); np.cumsum(lens, out=off[1:])
+    seqs = [rng.integers(0, 256, L).astype(np.uint8) for L in lens]
+    out = np.zeros(32 * ((int(off[-1]) >> 5) + n) + 32, np.uint8)
+    for i, s in enumerate(seqs):
+        a = 32 * ((off[i] >> 5) + i)
+        out[a:a + len(s)] = s
+    h = rng.integers(-2**63, 2**63 - 1, n, dtype=np.int64)
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(str(d), "x_", n, {"length": torch.from_numpy(np.diff(off)), "hash": torch.from_numpy(h)},
+                           canon=(torch.from_numpy(out), torch.from_numpy(off)))
+    r = {f.name[2:-4]: np.load(f) for f in (tmp_path / "a").iterdir()}
+    assert sorted(r) == ["canonical_bytes", "hash_hi", "hash_lo", "index", "length"]
+    assert all(np.array_equal(v, np.load(tmp_path / "b" / ("x_" + k + ".npy"))) for k, v in r.items())   # the same sample
+    idx = r["index"].astype(np.int64)
+    assert len(idx) == 700 and np.all(np.diff(idx) > 0) and r["hash_hi"].dtype == np.float64
+    u = (r["hash_hi"].astype(np.uint64) << np.uint64(32)) | r["hash_lo"].astype(np.uint64)
+    assert np.array_equal(u.view(np.int64), h[idx]) and np.array_equal(r["length"], lens[idx])
+    cb, ln = r["canonical_bytes"], r["length"].astype(np.int64)
+    k = int((np.cumsum(ln) <= 30000).sum())
+    assert cb.dtype == np.float32 and len(cb) == ln[:k].sum()
+    assert np.array_equal(cb, np.concatenate([seqs[i] for i in idx[:k]]))
+
+
 def test_argument_defaults():
     sys.path.insert(0, ROOT)
     import importlib
