@@ -1,11 +1,13 @@
-//! circkit-cuda: the device side of `circkit canonicalize` / `circkit uniq` on B200 (sm_100a).
+//! circkit-cuda: the device side of `circkit canonicalize` / `circkit uniq` / `circkit monomerize` on B200 (sm_100a).
 //!
 //! * [`ffi`] mirrors `include/circkit_b200.h` one to one.
 //! * [`Context`] owns a `ck_ctx` (one device, two in-flight batch slots, the first-occurrence table).
 //! * [`Pump`] is the replacement for `seq_io::parallel::parallel_fasta` as circKit uses it
 //!   (`src/canonicalize.rs:17-45`, `src/uniq.rs:29-79`): the reader thread appends `record.seq()` to a pinned batch, full
 //!   batches are packed to 2 bits per base on the host (`ck_pack2_host`), shipped and processed on alternating slots, and the
-//!   caller's consumer closure sees every record in input order with its canonical bytes / survival decision.
+//!   caller's consumer closure sees every record in input order with its canonical bytes / survival decision.  For
+//!   `circkit monomerize` (`src/monomerize.rs:16-160`) the raw bytes go to the device as they are (`ck_mono_submit`), and the
+//!   closure gets the written records' monomers and the lengths of the `--table` row.
 //! * [`canonicalize`], [`lmsr`], [`lmsr_index`] are the drop-ins for `circkit::canonicalize` (`lib/src/canonicalize.rs:54`),
 //!   `circkit::canonicalize::lmsr` (`:41`) and `lmsr_index` (`:5`): same signatures, same results, a process-wide context.
 //!
@@ -43,6 +45,20 @@ pub mod ffi {
         pub lane_bytes_total: u64,
         pub n_records: u32,
     }
+    /// `ck_mono_options`: the consumer-closure options of `circkit monomerize` (`src/commands.rs:19-90`); every "unset"
+    /// value filters nothing, like the reference's `None`.
+    #[repr(C)]
+    #[derive(Clone, Copy, PartialEq, Debug)]
+    pub struct MonoOptions {
+        pub seed_len: u32,              // 1..63
+        pub flags: u32,                 // CK_MONO_SENSITIVE | CK_MONO_FIRST_ONLY | CK_MONO_KEEP_ALL
+        pub overlap_dist: u64,          // --max-mismatch; 0 = unset
+        pub overlap_min_identity: f64,  // --min-identity; < 0 = unset
+        pub min_length: u64,            // --min-length (default 0)
+        pub max_length: u64,            // --max-length; u64::MAX = unset
+        pub min_overlap: u64,           // --min-overlap; 0 = unset
+        pub min_overlap_percent: f64,   // --min-overlap-percent; NaN = unset
+    }
     pub const CK_OK: c_int = 0;
     pub const CK_F_NORMALIZE: u32 = 1;
     pub const CK_F_NO_BYTES: u32 = 2;
@@ -50,6 +66,10 @@ pub mod ffi {
     pub const CK_F_PACKED_IN: u32 = 8;
     pub const CK_F_SURVIVORS: u32 = 16;
     pub const CK_PEER_HANDLE_BYTES: usize = 64;
+    pub const CK_MONO_SENSITIVE: u32 = 1;
+    pub const CK_MONO_FIRST_ONLY: u32 = 2;
+    pub const CK_MONO_KEEP_ALL: u32 = 4;
+    pub const CK_MONO_NONE: u32 = 0xffff_ffff;
     extern "C" {
         pub fn ck_init(cfg: *const CkConfig, out: *mut *mut CkCtx) -> c_int;
         pub fn ck_destroy(ctx: *mut CkCtx);
@@ -74,6 +94,11 @@ pub mod ffi {
                              lane_bytes_capacity: u64, lane_offsets: *mut u64, lane_bytes_total: *mut u64) -> c_int;
         pub fn ck_canon_submit_packed(ctx: *mut CkCtx, slot: c_int, batch: *const CkPackedBatch, flags: u32) -> c_int;
         pub fn ck_uniq_submit_packed(ctx: *mut CkCtx, slot: c_int, batch: *const CkPackedBatch, flags: u32, base_index: u64) -> c_int;
+        pub fn ck_mono_submit(ctx: *mut CkCtx, slot: c_int, bytes: *const u8, offsets: *const u64, n: u32, flags: u32,
+                              opt: *const MonoOptions) -> c_int;
+        pub fn ck_mono_wait(ctx: *mut CkCtx, slot: c_int, out_n_written: *mut u32, out_index: *mut u32, out_compact_offsets: *mut u64,
+                            out_compact_bytes: *mut u8, out_monomer_len: *mut u32, out_full_len: *mut u32,
+                            out_end_index: *mut u32) -> c_int;
         pub fn ck_peer_export(ctx: *mut CkCtx, world: u32, rank: u32, max_records: u32, handle_out: *mut c_void) -> c_int;
         pub fn ck_peer_attach(ctx: *mut CkCtx, all_handles: *const c_void) -> c_int;
         pub fn ck_lmsr_index(ctx: *mut CkCtx, s: *const u8, n: usize, out_index: *mut usize) -> c_int;
@@ -172,8 +197,10 @@ struct Batch {
     lane_bytes: Pinned<u8>,
     lane_offsets: Pinned<u64>,
     // results
-    out: Pinned<u8>,            // canonicalize: aligned arena; uniq: the survivors' compact arena
-    out_len: Pinned<u32>,
+    out: Pinned<u8>,            // canonicalize: aligned arena; uniq / monomerize: the survivors' / written records' compact arena
+    out_len: Pinned<u32>,       // monomerize: monomer_length
+    full_len: Pinned<u32>,      // monomerize: original_length (length of full_seq)
+    end: Pinned<u32>,           // monomerize: the worker's end index (CK_MONO_NONE = None)
     first: Pinned<u64>,
     sel: Pinned<u32>,
     sel_off: Pinned<u64>,
@@ -189,14 +216,23 @@ pub struct Done<'a> {
     /// global input index of this record and of the first record with the same canonical form (`uniq` only)
     pub index: u64,
     pub first_index: u64,
+    /// `monomerize`: full_seq[..monomer_length] of a record the consumer closure writes (`src/monomerize.rs:139-143`), None
+    /// for a record it drops; None in the other modes
+    pub monomer: Option<&'a [u8]>,
+    /// `monomerize`: the `original_length` / `monomer_length` columns of `--table` (`:145-154`); 0 in the other modes
+    pub original_length: u64,
+    pub monomer_length: u64,
 }
 
-#[derive(Clone, Copy, PartialEq, Eq)]
+#[derive(Clone, Copy, PartialEq)]
 pub enum Mode {
     /// `circkit canonicalize`: every record comes back with its canonical form
     Canonicalize,
     /// `circkit uniq`: `first_index == index` marks the survivors; `canonical_bytes` = the `-c` flag
     Uniq { canonical_bytes: bool },
+    /// `circkit monomerize`: normalisation, the monomer search, the filters and the extraction of the written monomers run
+    /// on the device (`ck_mono_submit`); `Done::monomer` is Some for the records the CLI writes
+    Monomerize(ffi::MonoOptions),
 }
 
 /// The record pump: replacement for `parallel_fasta(reader, threads, 64, W, F)`.
@@ -211,8 +247,8 @@ pub struct Pump {
 }
 
 impl Pump {
-    /// `threads` = the CLI's `--threads` (`src/commands.rs:122,147`): host packer threads.  `table_capacity` = distinct
-    /// canonical forms `uniq` may meet (ignored for canonicalize).
+    /// `threads` = the CLI's `--threads` (`src/commands.rs:122,147`): host packer threads (monomerize does not pack).
+    /// `table_capacity` = distinct canonical forms `uniq` may meet (ignored for canonicalize / monomerize).
     pub fn new(device: i32, mode: Mode, threads: u32, table_capacity: u64) -> Result<Self> {
         const MAX_BYTES: u64 = 256 << 20;
         const MAX_RECORDS: u32 = 1 << 20;
@@ -235,6 +271,8 @@ impl Pump {
                 lane_offsets: Pinned::new(ctx, r + 1)?,
                 out: Pinned::new(ctx, unsafe { ffi::ck_out_arena_bytes(MAX_BYTES, MAX_RECORDS) } as usize)?,
                 out_len: Pinned::new(ctx, r)?,
+                full_len: Pinned::new(ctx, r)?,
+                end: Pinned::new(ctx, r)?,
                 first: Pinned::new(ctx, r)?,
                 sel: Pinned::new(ctx, r)?,
                 sel_off: Pinned::new(ctx, r + 1)?,
@@ -292,6 +330,16 @@ impl Pump {
         let threads = self.threads;
         let mode = self.mode;
         let b = &mut self.batches[slot];
+        if let Mode::Monomerize(opt) = mode {
+            // the raw bytes as the reader appended them: the device normalises them and needs the raw form for full_seq
+            let rc = unsafe {
+                ffi::ck_mono_submit(self.ctx.raw, slot as c_int, b.bytes.as_slice().as_ptr(), b.offsets.as_slice().as_ptr(), b.n as u32,
+                                    ffi::CK_F_NORMALIZE, &opt)
+            };
+            self.ctx.check(rc)?;
+            self.in_flight[slot] = true;
+            return Ok(());
+        }
         let mut lane_total = 0u64;
         // pack on the host: needletail normalisation + symbol lanes + 2 bits per base (a quarter of the bytes cross PCIe)
         let rc = unsafe {
@@ -315,6 +363,7 @@ impl Pump {
         };
         let rc = match mode {
             Mode::Canonicalize => unsafe { ffi::ck_canon_submit_packed(self.ctx.raw, slot as c_int, &pb, ffi::CK_F_ALIGNED_OUT) },
+            Mode::Monomerize(_) => unreachable!(),
             Mode::Uniq { canonical_bytes } => {
                 let flags = ffi::CK_F_SURVIVORS | ffi::CK_F_ALIGNED_OUT | if canonical_bytes { 0 } else { ffi::CK_F_NO_BYTES };
                 unsafe { ffi::ck_uniq_submit_packed(self.ctx.raw, slot as c_int, &pb, flags, b.base_index) }
@@ -351,6 +400,9 @@ impl Pump {
                         canonical: Some(&out[at..at + len[i] as usize]),
                         index: b.base_index + i as u64,
                         first_index: b.base_index + i as u64,
+                        monomer: None,
+                        original_length: 0,
+                        monomer_length: 0,
                     })?;
                 }
             }
@@ -383,6 +435,41 @@ impl Pump {
                         canonical,
                         index: b.base_index + i as u64,
                         first_index: first[i],
+                        monomer: None,
+                        original_length: 0,
+                        monomer_length: 0,
+                    })?;
+                }
+            }
+            Mode::Monomerize(_) => {
+                let mut nw = 0u32;
+                let rc = unsafe {
+                    ffi::ck_mono_wait(raw, slot as c_int, &mut nw, b.sel.as_mut_slice().as_mut_ptr(), b.sel_off.as_mut_slice().as_mut_ptr(),
+                                      b.out.as_mut_slice().as_mut_ptr(), b.out_len.as_mut_slice().as_mut_ptr(),
+                                      b.full_len.as_mut_slice().as_mut_ptr(), b.end.as_mut_slice().as_mut_ptr())
+                };
+                self.ctx.check(rc)?;
+                let b = &self.batches[slot];
+                let (off, out, len, full) = (b.offsets.as_slice(), b.out.as_slice(), b.out_len.as_slice(), b.full_len.as_slice());
+                let (sel, sel_off) = (b.sel.as_slice(), b.sel_off.as_slice());
+                let mut k = 0usize;                                       // next written record
+                for i in 0..n {
+                    let monomer = if k < nw as usize && sel[k] as usize == i {
+                        let at = sel_off[k] as usize;
+                        k += 1;
+                        Some(&out[at..at + len[i] as usize])
+                    } else {
+                        None
+                    };
+                    consume(Done {
+                        head: &b.heads[i],
+                        raw_seq: &b.bytes.as_slice()[off[i] as usize..off[i + 1] as usize],
+                        canonical: None,
+                        index: b.base_index + i as u64,
+                        first_index: b.base_index + i as u64,
+                        monomer,
+                        original_length: full[i] as u64,
+                        monomer_length: len[i] as u64,
                     })?;
                 }
             }

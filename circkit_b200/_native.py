@@ -12,7 +12,7 @@ CK_OK = 0
 CK_ERR_CUDA, CK_ERR_ARG, CK_ERR_STATE, CK_ERR_TOO_LONG, CK_ERR_TABLE_FULL = -1, -2, -3, -4, -5
 CK_F_NORMALIZE, CK_F_NO_BYTES, CK_F_ALIGNED_OUT, CK_F_PACKED_IN, CK_F_SURVIVORS, CK_F_SINGLE_COPY = 1, 2, 4, 8, 16, 32
 CK_PEER_HANDLE_BYTES = 64
-CK_MONO_SENSITIVE, CK_MONO_FIRST_ONLY, CK_MONO_NONE = 1, 2, 0xFFFFFFFF
+CK_MONO_SENSITIVE, CK_MONO_FIRST_ONLY, CK_MONO_KEEP_ALL, CK_MONO_NONE = 1, 2, 4, 0xFFFFFFFF
 CK_CLASS_2BIT_LE_512, CK_CLASS_2BIT_LE_2048, CK_CLASS_2BIT_LE_65536, CK_CLASS_2BIT_LE_425984 = 1, 2, 4, 8
 CK_CLASS_2BIT_LE_4096, CK_CLASS_2BIT_LE_8192 = 1 << 10, 1 << 11
 
@@ -26,6 +26,12 @@ class CkPackedBatch(C.Structure):
     _fields_ = [("packed2", C.c_void_p), ("offsets", C.c_void_p), ("lens", C.c_void_p), ("lane", C.c_void_p),
                 ("lane_bytes", C.c_void_p), ("lane_offsets", C.c_void_p), ("lane_bytes_total", C.c_uint64),
                 ("n_records", C.c_uint32)]
+
+
+class CkMonoOptions(C.Structure):
+    _fields_ = [("seed_len", C.c_uint32), ("flags", C.c_uint32), ("overlap_dist", C.c_uint64),
+                ("overlap_min_identity", C.c_double), ("min_length", C.c_uint64), ("max_length", C.c_uint64),
+                ("min_overlap", C.c_uint64), ("min_overlap_percent", C.c_double)]
 
 
 class NativeLibraryMissing(RuntimeError):
@@ -75,6 +81,8 @@ SIGNATURES = {
     "ck_dev_gather_first": (_i, [_vp, _vp, _vp, _vp, _u32, _vp]),
     "ck_dev_monomerize": (_i, [_vp, _vp, _vp, _vp, _vp, _u32, _u32, _u64, C.c_double, _u32, _vp]),
     "ck_dev_normalize": (_i, [_vp, _vp, _vp, _vp, _u32, _vp, _vp]),
+    "ck_mono_submit": (_i, [_vp, _i, _vp, _vp, _u32, _u32, C.POINTER(CkMonoOptions)]),
+    "ck_mono_wait": (_i, [_vp, _i, C.POINTER(_u32), _vp, _vp, _vp, _vp, _vp, _vp]),
     "ck_launch_count": (_u64, [_vp]),
     "ck_kernel_timing": (_i, [_vp, _i]),
     "ck_kernel_times": (_i, [_vp, _vp, _vp, _u32]),

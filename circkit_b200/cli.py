@@ -1,7 +1,8 @@
-"""`circkit canonicalize` / `circkit uniq` on the B200 path: the host side of the two CLI drivers.
+"""`circkit canonicalize` / `circkit uniq` / `circkit monomerize` on the B200 path: the host side of the CLI drivers.
 
     python -m circkit_b200 canonicalize [INPUT] [-o OUTPUT] [-t THREADS]
     python -m circkit_b200 uniq [INPUT] [-o OUTPUT] [-c] [--table TABLE] [-t THREADS]
+    python -m circkit_b200 monomerize [INPUT] [-o OUTPUT] [--seed-length N] [--max-mismatch N | --min-identity F] ... [--table TABLE]
 
 Mirrors src/canonicalize.rs:7-51 and src/uniq.rs:15-88 with the flags of src/commands.rs:112-149: the host keeps what
 the reference keeps on the host -- reading (with the compression sniffing of src/utils.rs:9-27), FASTA record splitting
@@ -9,7 +10,9 @@ the reference keeps on the host -- reading (with the compression sniffing of src
 table (src/uniq.rs:62-71, src/utils.rs:74-84) and output compression by suffix (src/utils.rs:29-72) -- and hands batches
 of record bytes, packed to 2 bits per base by `--threads` host threads (ck_pack2_host), to the C ABI (ck_*_submit_packed,
 two slots in flight), where LMSR, the canonical form, XXH3-64, the first-occurrence table and the compaction of the
-survivors run on the GPU.  Input and output stream in pieces of 64 MB, so files larger than host memory pass through.
+survivors run on the GPU.  `monomerize` (src/monomerize.rs:16-160) hands the raw record bytes to ck_mono_submit /
+ck_mono_wait the same way; normalisation, the monomer search, the length / overlap filters and the extraction of the written
+monomers run on the GPU.  Input and output stream in pieces of 64 MB, so files larger than host memory pass through.
 Nothing is printed on success (tests/canon_uniq.rs:74-77); an I/O error exits non-zero with the OS message on stderr.
 
 Record splitting and output assembly are numpy-vectorised (no per-record Python on the canonicalize path).
@@ -350,8 +353,9 @@ MAX_BATCH_BYTES = 256 << 20
 MAX_BATCH_RECORDS = 1 << 20
 
 
-def _batches(offsets: np.ndarray):
-    """cuts of the record range into batches of <= MAX_BATCH_BYTES / MAX_BATCH_RECORDS"""
+def _batches(offsets: np.ndarray, oversize: bool = False):
+    """cuts of the record range into batches of <= MAX_BATCH_BYTES / MAX_BATCH_RECORDS; oversize=True: a record longer than
+    MAX_BATCH_BYTES is a batch of its own (else FastaError)"""
     n = len(offsets) - 1
     cuts = [0]
     while cuts[-1] < n:
@@ -361,7 +365,9 @@ def _batches(offsets: np.ndarray):
         if int(offsets[hi]) > limit:
             hi = int(np.searchsorted(offsets, limit, side="right")) - 1
         if hi <= lo:
-            raise FastaError("record longer than the batch size")
+            if not oversize:
+                raise FastaError("record longer than the batch size")
+            hi = lo + 1
         cuts.append(hi)
     return cuts
 
@@ -443,6 +449,13 @@ def run_canonicalize(pieces, write, threads: int = 0) -> None:
             ctx.close()
 
 
+def _csv_field(f: bytes, delim: bytes) -> bytes:
+    """csv 1.2.2 defaults (QuoteStyle::Necessary, double_quote, terminator '\\n')"""
+    if any(c in f for c in (delim, b'"', b"\n", b"\r")):
+        return b'"' + f.replace(b'"', b'""') + b'"'
+    return f
+
+
 def _check_ids(recs: "Records", which: np.ndarray) -> None:
     """record.id().unwrap() (src/uniq.rs:48,67): the id -- head up to the first ' ' -- must be UTF-8"""
     heads = recs.gather(recs.head_lo[which], recs.head_hi[which]).tobytes()
@@ -464,11 +477,6 @@ def run_uniq(pieces, write, canonical: bool = False, table_write=None, table_ext
     first_ids = {}                                             # global index of a first occurrence -> its id (for --table only)
     delim = b"\t" if table_ext == "tsv" else b","
     wrote_header = False
-
-    def field(f: bytes) -> bytes:
-        if any(c in f for c in (delim, b'"', b"\n", b"\r")):
-            return b'"' + f.replace(b'"', b'""') + b'"'
-        return f
     try:
         for recs in pieces:
             n = len(recs)
@@ -498,7 +506,7 @@ def run_uniq(pieces, write, canonical: bool = False, table_write=None, table_ext
                     if not wrote_header:
                         rows += b"id" + delim + b"duplicate_id\n"
                         wrote_header = True
-                    rows += field(first_ids[int(first[i])]) + delim + field(rec_id(i)) + b"\n"
+                    rows += _csv_field(first_ids[int(first[i])], delim) + delim + _csv_field(rec_id(i), delim) + b"\n"
                 table_write(bytes(rows))
             base += n
     finally:
@@ -526,82 +534,111 @@ class CliError(ValueError):
     """argument combinations the reference rejects with `bail!` (src/monomerize.rs:35-45)"""
 
 
-def monomerize(fasta: bytes, sensitive: bool = False, seed_length: int = 10, max_mismatch=None, min_identity=None,
-               min_overlap=None, min_overlap_percent=None, min_length: int = 0, max_length=None, keep_all: bool = False,
-               table_ext: str | None = None):
-    """bytes of a FASTA file -> (bytes `circkit monomerize` writes, bytes of the --table file or None)
-    (src/monomerize.rs:16-160).  Normalisation (`ck_dev_normalize`) and the monomer search (`ck_dev_monomerize`) run on
-    the device over the whole file as one batch; the length / overlap filters of the consumer closure (:102-135) and the
-    framing (:139-143: '>' head, full_seq[..end]) are vectorised on the host."""
-    import torch
-    from .monomerize import Monomerizer
+def mono_options(sensitive: bool = False, seed_length: int = 10, max_mismatch=None, min_identity=None, min_overlap=None,
+                 min_overlap_percent=None, min_length: int = 0, max_length=None, keep_all: bool = False):
+    """the options of `circkit monomerize` (src/commands.rs:19-90) as ck_mono_options, checked like the CLI's bail!s
+    (src/monomerize.rs:35-45) and the builder (lib/src/monomerize.rs:20-40) before anything touches the device"""
+    from ._native import CK_MONO_KEEP_ALL, CK_MONO_SENSITIVE, CkMonoOptions
     if max_mismatch is not None and min_identity is not None:
         raise CliError("cannot specify both max_mismatch and min_identity")
     if min_identity is not None and not 0.0 <= min_identity <= 1.0:
         raise CliError("min_identity must be between 0.0 and 1.0")
-    recs = Records(fasta)
-    n = len(recs)
-    table = bytearray() if table_ext is not None else None
-    if n == 0:
-        return b"", (bytes(table) if table is not None else None)
-    seq_len = (recs.seq_hi - recs.seq_lo).astype(np.int64)
-    off = np.zeros(n + 1, dtype=np.int64)
-    np.cumsum(seq_len, out=off[1:])
-    arena = np.ascontiguousarray(recs.gather(recs.seq_lo, recs.seq_hi))
-    m = Monomerizer(seed_length, max_mismatch, min_identity)
-    ctx = m._context()
-    try:
-        dev = torch.device("cuda", ctx.device)
-        raw = torch.from_numpy(arena if len(arena) else np.zeros(1, dtype=np.uint8)).to(dev)
-        offs = torch.from_numpy(off).to(dev)
-        norm, nlens = m.normalize_device(raw, offs, n)
-        end = m.end_indices_device(norm, offs, n, sensitive=sensitive, lens=nlens)
-        idx = end.cpu().numpy().astype(np.int64)             # -1 = None
-        nl = nlens.cpu().numpy().astype(np.int64)
-    finally:
-        ctx.close()
-    idx[(nl < seed_length) | (nl < min_length)] = -1        # worker closure, src/monomerize.rs:92-96
-    # record.full_seq(): the lines of seq joined, each without its '\n' and one trailing '\r'
-    is_nl, is_cr = arena == 10, arena == 13
-    before_nl = np.append(is_nl[1:], False)
-    at_end = np.zeros(len(arena), dtype=bool)
-    nonempty = seq_len > 0
-    at_end[off[1:][nonempty] - 1] = True
-    kept = ~(is_nl | (is_cr & (before_nl | at_end)))
-    c = np.zeros(len(arena) + 1, dtype=np.int64)
-    np.cumsum(kept, out=c[1:])
-    full_len = c[off[1:]] - c[off[:-1]]
-    ok = idx >= 0                                            # consumer closure, :107-135
-    ok &= ~(idx < min_length)
-    if max_length is not None:
-        ok &= ~(idx > max_length)
-    if min_overlap is not None:
-        ok &= ~((full_len - idx) < min_overlap)
-    if min_overlap_percent is not None:
-        with np.errstate(divide="ignore", invalid="ignore"):
-            ok &= ~(((full_len - idx).astype(np.float64) / idx.astype(np.float64)) < min_overlap_percent)
-    write = ok | keep_all
-    end_idx = np.minimum(np.where(ok, idx, full_len), full_len)
-    rec_of = np.repeat(np.arange(n, dtype=np.int64), seq_len)
-    rank = c[:-1] - c[off[:-1]][rec_of]
-    sel = kept & (rank < end_idx[rec_of]) & write[rec_of]
-    heads = recs.gather(recs.head_lo[write], recs.head_hi[write])
-    out = _assemble(heads, (recs.head_hi - recs.head_lo)[write], arena[sel], end_idx[write])
-    if table is not None:                                    # :145-154, csv 1.2.2 defaults: header with the first row
-        delim = b"\t" if table_ext == "tsv" else b","
+    if not 1 <= seed_length <= 63:
+        raise CliError("Seed length must be at least 1 and at most 63 but was set to %d." % seed_length)
+    for name, v in (("max_mismatch", max_mismatch), ("min_overlap", min_overlap), ("min_length", min_length),
+                    ("max_length", max_length)):
+        if v is not None and v < 0:                          # usize in the reference
+            raise CliError("%s must not be negative" % name)
+    return CkMonoOptions(seed_length, (CK_MONO_SENSITIVE if sensitive else 0) | (CK_MONO_KEEP_ALL if keep_all else 0),
+                         max_mismatch or 0, -1.0 if min_identity is None else float(min_identity), min_length,
+                         2**64 - 1 if max_length is None else max_length, min_overlap or 0,
+                         float("nan") if min_overlap_percent is None else float(min_overlap_percent))
 
-        def field(f: bytes) -> bytes:
-            if any(x in f for x in (delim, b'"', b"\n", b"\r")):
-                return b'"' + f.replace(b'"', b'""') + b'"'
-            return f
-        rows = np.flatnonzero(write)
-        if len(rows):
-            table += delim.join([b"id", b"original_length", b"monomer_length"]) + b"\n"
-        for i in rows.tolist():
-            head = recs.data[recs.head_lo[i]: recs.head_hi[i]].tobytes()
-            head.decode("utf-8")                             # std::str::from_utf8(record.head()).unwrap()
-            table += delim.join([field(head), b"%d" % full_len[i], b"%d" % end_idx[i]]) + b"\n"
-    return out, (bytes(table) if table is not None else None)
+
+def _pump_mono(ctx: Context, big: "Context | None", arena: np.ndarray, offsets: np.ndarray, opts):
+    """All batches of one piece through the two slots (ck_mono_submit / ck_mono_wait): the submit of batch b runs while
+    batch b - 1 is collected.  A record longer than MAX_BATCH_BYTES is a batch of its own on `big`, a context whose staging
+    fits it.  -> (indices of the written records, increasing; their bytes, concatenated; monomer_len[n]; full_len[n])"""
+    n = len(offsets) - 1
+    cuts = _batches(offsets, oversize=True)
+    mono_len = np.zeros(n, dtype=np.int64)
+    full_len = np.zeros(n, dtype=np.int64)
+    idxs, outs = [], []
+    nb = len(cuts) - 1
+    pend = {}
+    for b in range(nb + 1):
+        if b < nb:
+            lo, hi = cuts[b], cuts[b + 1]
+            rel = (offsets[lo: hi + 1] - offsets[lo]).astype(np.uint64)
+            sub = arena[int(offsets[lo]): int(offsets[hi])]
+            c = big if int(rel[-1]) > MAX_BATCH_BYTES else ctx
+            c.mono_submit(b & 1, sub, rel, opts)
+            pend[b] = (c, sub, rel)                              # keeps the host arrays alive until the wait
+        if b >= 1:
+            lo, hi = cuts[b - 1], cuts[b]
+            c, _, rel = pend.pop(b - 1)
+            r = c.mono_wait((b - 1) & 1, hi - lo, int(rel[-1]))
+            mono_len[lo:hi] = r["monomer_len"]
+            full_len[lo:hi] = r["full_len"]
+            if r["n_written"]:
+                idx = r["index"].astype(np.int64)
+                st = r["offsets"][:-1].astype(np.int64)
+                idxs.append(idx + lo)
+                outs.append(r["bytes"][_region_mask(len(r["bytes"]), st, st + mono_len[lo + idx])])
+    written = np.concatenate(idxs) if idxs else np.zeros(0, dtype=np.int64)
+    body = np.concatenate(outs) if outs else np.zeros(0, dtype=np.uint8)
+    return written, body, mono_len, full_len
+
+
+def run_monomerize(pieces, write, opts, table_write=None, table_ext: str | None = None) -> None:
+    """`circkit monomerize` over a stream of Records pieces (src/monomerize.rs:16-160): `opts` from mono_options; normalisation,
+    the monomer search, the length / overlap filters of the consumer closure and the extraction of full_seq[..end] run on the
+    device; `write(bytes)` gets the output ('>' head '\\n' monomer '\\n'), `table_write` the --table rows as pieces complete."""
+    ctx = big = None
+    delim = b"\t" if table_ext == "tsv" else b","
+    wrote_header = False
+    try:
+        for recs in pieces:
+            n = len(recs)
+            if n == 0:
+                continue
+            arena, offsets, seq_len = _piece_arena(recs)
+            longest = int(seq_len.max())
+            if ctx is None:
+                ctx = _context(0)
+            if longest > MAX_BATCH_BYTES and (big is None or big.max_batch_bytes < longest):
+                if big is not None:
+                    big.close()
+                big = Context(max_batch_bytes=longest, max_batch_records=1)
+            written, body, mono_len, full_len = _pump_mono(ctx, big, arena, offsets, opts)
+            heads = recs.gather(recs.head_lo[written], recs.head_hi[written])
+            write(_assemble(heads, (recs.head_hi - recs.head_lo)[written], body, mono_len[written]))
+            if table_write is not None and len(written):      # :145-154, csv 1.2.2 defaults: header with the first row
+                rows = bytearray()
+                if not wrote_header:
+                    rows += delim.join([b"id", b"original_length", b"monomer_length"]) + b"\n"
+                    wrote_header = True
+                for i in written.tolist():
+                    head = recs.data[recs.head_lo[i]: recs.head_hi[i]].tobytes()
+                    head.decode("utf-8")                         # std::str::from_utf8(record.head()).unwrap()
+                    rows += delim.join([_csv_field(head, delim), b"%d" % full_len[i], b"%d" % mono_len[i]]) + b"\n"
+                table_write(bytes(rows))
+    finally:
+        for c in (ctx, big):
+            if c is not None:
+                c.close()
+
+
+def monomerize(fasta: bytes, sensitive: bool = False, seed_length: int = 10, max_mismatch=None, min_identity=None,
+               min_overlap=None, min_overlap_percent=None, min_length: int = 0, max_length=None, keep_all: bool = False,
+               table_ext: str | None = None):
+    """bytes of a FASTA file -> (bytes `circkit monomerize` writes, bytes of the --table file or None)
+    (src/monomerize.rs:16-160), through run_monomerize"""
+    opts = mono_options(sensitive, seed_length, max_mismatch, min_identity, min_overlap, min_overlap_percent, min_length,
+                        max_length, keep_all)
+    out, table = [], ([] if table_ext is not None else None)
+    run_monomerize(iter_records([fasta] if fasta else []), out.append, opts, table.append if table is not None else None, table_ext)
+    return b"".join(out), (b"".join(table) if table is not None else None)
 
 
 # ------------------------------------------------------------------------------------------------ entry point
@@ -638,19 +675,11 @@ def main(argv=None) -> int:
     args = ap.parse_args(argv)
     try:
         threads = max(1, args.threads or 1)
-        if args.command == "monomerize":
-            data = read_input(args.input)
-            ext = None
-            if args.table is not None:
-                ext = "tsv" if args.table.endswith(".tsv") else "csv"
-            out, table = monomerize(data, args.sensitive, args.seed_length, args.max_mismatch, args.min_identity, args.min_overlap,
-                                    args.min_overlap_percent, args.min_length, args.max_length, args.keep_all, ext)
-            write_output(args.output, out)
-            if args.table is not None:
-                with open(args.table, "wb") as f:
-                    f.write(table)
-            return 0
-        # canonicalize / uniq stream: decompress, split, pack, process and write piece by piece (src/utils.rs:9-72)
+        opts = None
+        if args.command == "monomerize":                      # argument errors before any file is opened
+            opts = mono_options(args.sensitive, args.seed_length, args.max_mismatch, args.min_identity, args.min_overlap,
+                                args.min_overlap_percent, args.min_length, args.max_length, args.keep_all)
+        # every subcommand streams: decompress, split, (pack,) process and write piece by piece (src/utils.rs:9-72)
         pieces = iter_records(iter_input(args.input))
         first = next(pieces, None)                              # open the input (and fail on it) before the output is created
 
@@ -661,13 +690,15 @@ def main(argv=None) -> int:
         w = Writer(args.output)
         tf = None
         try:
+            ext = None
+            if getattr(args, "table", None) is not None:           # uniq / monomerize --table
+                ext = "tsv" if args.table.endswith(".tsv") else "csv"
+                tf = open(args.table, "wb")
             if args.command in ("canonicalize", "canon"):
                 run_canonicalize(chain(), w.write, threads=threads)
+            elif args.command == "monomerize":
+                run_monomerize(chain(), w.write, opts, tf.write if tf else None, ext)
             else:
-                ext = None
-                if args.table is not None:
-                    ext = "tsv" if args.table.endswith(".tsv") else "csv"
-                    tf = open(args.table, "wb")
                 cap = 1 << 24
                 if args.input is not None:
                     # distinct canonical forms the table must hold: bounded by the record count, itself bounded by the input size

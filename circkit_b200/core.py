@@ -222,6 +222,28 @@ class Context:
         k = int(ns.value)
         return dict(n_survivors=k, index=index[:k], offsets=offs[:k + 1], bytes=out, lens=lens[:n], hash=h[:n], first=first[:n])
 
+    def mono_submit(self, slot: int, arena: np.ndarray, offsets: np.ndarray, opts: "N.CkMonoOptions", normalize: bool = True,
+                    want_bytes: bool = True):
+        """ck_mono_submit: `circkit monomerize`'s worker and consumer closures over a batch of raw record bytes"""
+        flags = (N.CK_F_NORMALIZE if normalize else 0) | (0 if want_bytes else N.CK_F_NO_BYTES)
+        self._check(self._lib.ck_mono_submit(self._h, slot, _ptr(arena), _ptr(offsets), len(offsets) - 1, flags, C.byref(opts)))
+
+    def mono_wait(self, slot: int, n: int, total: int, want_bytes: bool = True):
+        """ck_mono_wait -> dict(n_written, index[nw], offsets[nw + 1], bytes (compact arena), monomer_len[n], full_len[n],
+        end[n] (CK_MONO_NONE = None))"""
+        nw = C.c_uint32(0)
+        index = np.zeros(max(n, 1), dtype=np.uint32)
+        offs = np.zeros(max(n, 0) + 1, dtype=np.uint64)
+        out = np.empty(max(total + 16 * n, 1), dtype=np.uint8) if want_bytes else None   # read only where written
+        mono_len = np.zeros(max(n, 1), dtype=np.uint32)
+        full_len = np.zeros(max(n, 1), dtype=np.uint32)
+        end = np.zeros(max(n, 1), dtype=np.uint32)
+        self._check(self._lib.ck_mono_wait(self._h, slot, C.byref(nw), _ptr(index), _ptr(offs), _ptr(out), _ptr(mono_len),
+                                           _ptr(full_len), _ptr(end)))
+        k = int(nw.value)
+        return dict(n_written=k, index=index[:k], offsets=offs[:k + 1], bytes=out, monomer_len=mono_len[:n], full_len=full_len[:n],
+                    end=end[:n])
+
     def uniq_batch(self, arena: np.ndarray, offsets: np.ndarray, base_index: int = 0, *, normalize: bool = False,
                    want_bytes=True, aligned=False):
         """Worker + consumer closures over a batch (src/uniq.rs:33-78): dict(out, lens, hash, first)."""

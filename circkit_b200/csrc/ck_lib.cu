@@ -98,7 +98,7 @@ struct Slot {
     u64 *d_dense = nullptr; u64 *d_laneoff = nullptr;   // CK_F_PACKED_IN: the host packer's dense 2-bit layout, byte-lane offsets
     u32 *h_counts = nullptr;            // pinned
     ExecScratch scr;
-    bool busy = false, uniq = false;
+    bool busy = false, uniq = false, mono = false;   // mono: ck_mono_submit's batch (ck_mono_wait collects it)
     u32 dbl = 1;                        // packed2 layout of the batch in flight
     u64 longest = 0;                    // longest raw record of the batch in flight
     u32 *sel = nullptr; u64 *coff = nullptr;    // CK_F_SURVIVORS: survivor indices / compact offsets of the batch in flight
@@ -576,8 +576,13 @@ int peer_first_index(ck_ctx *ctx, cudaStream_t st, u32 slot, const u64 *hash, u3
     return CK_OK;
 }
 
+// Longest record of a monomerize batch: every kernel of that path keeps lengths and in-record positions in u32 and steps
+// through a record 512 bytes at a time, so positions up to length + 511 must fit.  (Canonicalize / uniq: 2^30 symbols.)
+constexpr u64 kMonoMaxRecord = (1ull << 32) - 1024;
+
 // shared front of every submit: slot and batch checks.  Returns CK_OK with s.busy still false; n_records == 0 is complete.
-int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_records, uint32_t flags, bool uniq, bool have_bytes)
+int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_records, uint32_t flags, bool uniq, bool have_bytes,
+                 bool mono = false)
 {
     if (!ctx) return CK_ERR_ARG;
     if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
@@ -587,7 +592,7 @@ int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_reco
     if (n_records && (!offsets || (!have_bytes && offsets[n_records] != offsets[0])))
         return fail(ctx, CK_ERR_ARG, "null batch pointers");
     if (uniq && !ctx->table) return fail(ctx, CK_ERR_STATE, "context was created with table_capacity 0");
-    s.n = n_records; s.flags = flags; s.uniq = uniq; s.total = 0;
+    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.total = 0;
     if (n_records == 0) return CK_OK;
     if (offsets[0] != 0) return fail(ctx, CK_ERR_ARG, "offsets[0] must be 0");
     const u64 total = offsets[n_records];
@@ -597,46 +602,119 @@ int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_reco
         if (offsets[i + 1] < offsets[i]) return fail(ctx, CK_ERR_ARG, "offsets must be non-decreasing");
         longest = std::max<u64>(longest, offsets[i + 1] - offsets[i]);
     }
-    if (longest > (1ull << 30)) return fail(ctx, CK_ERR_TOO_LONG, "record longer than 2^30 symbols");
+    if (mono && longest > kMonoMaxRecord) return fail(ctx, CK_ERR_TOO_LONG, "record longer than 2^32 - 1024 bytes");
+    if (!mono && longest > (1ull << 30)) return fail(ctx, CK_ERR_TOO_LONG, "record longer than 2^30 symbols");
     s.total = total;
     s.longest = longest;
     s.dbl = longest > 512 ? 1u : 0u;     // batches of short records: single-copy arena (ck_device.cuh)
     return CK_OK;
 }
 
-// CK_F_SURVIVORS: compact the batch's survivors on the device (indices, 16-byte-aligned compact offsets, canonical bytes).  The
-// sort workspace of the batch is free by now (stream order): indices | lengths / offsets | flags | cub temporaries live in it;
-// the compact bytes go to the byte arena d_norm (no byte-lane kernel is running any more).
-int enqueue_compaction(ck_ctx *ctx, Slot &s, uint64_t base_index)
+// Order-preserving compaction of the records a batch writes (uniq's survivors, monomerize's written records): a flag per
+// record -> cub::DeviceSelect (their indices, increasing) -> their lengths rounded up to 16 -> exclusive scan = 16-byte-aligned
+// compact offsets.  The sort workspace of the batch is free by now (stream order): indices | lengths / offsets | flags | cub
+// temporaries live in it.  compaction_carve lays it out (the caller fills `flags` in stream order); compaction_select_scan
+// selects and scans, copies the count to h_counts[20] and leaves s.sel / s.coff for the wait; the caller gathers the bytes.
+struct Compaction {
+    u32 *sel; u64 *len16; u64 *coff; u8 *flags; u32 *n_sel; void *tmp; size_t tmp_bytes;
+};
+int compaction_carve(ck_ctx *ctx, Slot &s, Compaction &c)
 {
-    cudaStream_t st = s.stream;
     const u32 n = s.n;
     u8 *w = reinterpret_cast<u8 *>(s.d_lists);
-    u32 *sel = reinterpret_cast<u32 *>(w); w += ((size_t)n * 4 + 255) & ~(size_t)255;
-    u64 *len16 = reinterpret_cast<u64 *>(w); w += ((size_t)(n + 1) * 8 + 255) & ~(size_t)255;
-    u64 *coff = reinterpret_cast<u64 *>(w); w += ((size_t)(n + 1) * 8 + 255) & ~(size_t)255;
-    u8 *flags = w; w += ((size_t)n + 255) & ~(size_t)255;
-    u32 *n_sel = reinterpret_cast<u32 *>(w); w += 256;
-    void *tmp = w;
+    c.sel = reinterpret_cast<u32 *>(w); w += ((size_t)n * 4 + 255) & ~(size_t)255;
+    c.len16 = reinterpret_cast<u64 *>(w); w += ((size_t)(n + 1) * 8 + 255) & ~(size_t)255;
+    c.coff = reinterpret_cast<u64 *>(w); w += ((size_t)(n + 1) * 8 + 255) & ~(size_t)255;
+    c.flags = w; w += ((size_t)n + 255) & ~(size_t)255;
+    c.n_sel = reinterpret_cast<u32 *>(w); w += 256;
+    c.tmp = w;
     const size_t used = (size_t)(w - reinterpret_cast<u8 *>(s.d_lists));
     const size_t have = lists_bytes_for(ctx->cfg.max_batch_records);
     size_t need_a = 0, need_b = 0;
     cub::CountingInputIterator<u32> ids(0);
-    cub::DeviceSelect::Flagged(nullptr, need_a, ids, flags, sel, n_sel, (int)n, st);
-    cub::DeviceScan::ExclusiveSum(nullptr, need_b, len16, coff, (int)n + 1, st);
+    cub::DeviceSelect::Flagged(nullptr, need_a, ids, c.flags, c.sel, c.n_sel, (int)n, s.stream);
+    cub::DeviceScan::ExclusiveSum(nullptr, need_b, c.len16, c.coff, (int)n + 1, s.stream);
     if (used + std::max(need_a, need_b) > have) return fail(ctx, CK_ERR_ARG, "sort workspace too small for the compaction");
-    size_t tb = have - used;
-    k_survivor_flags<<<(n + 255) / 256, 256, 0, st>>>(s.d_first, base_index, n, flags);
-    CK_CUDA(ctx, cub::DeviceSelect::Flagged(tmp, tb, ids, flags, sel, n_sel, (int)n, st));
-    k_survivor_lens<<<(n + 256) / 256, 256, 0, st>>>(sel, n_sel, s.d_len, n, len16);
-    tb = have - used;
-    CK_CUDA(ctx, cub::DeviceScan::ExclusiveSum(tmp, tb, len16, coff, (int)n + 1, st));
+    c.tmp_bytes = have - used;
+    return CK_OK;
+}
+int compaction_select_scan(ck_ctx *ctx, Slot &s, const Compaction &c, const u32 *lens)
+{
+    cudaStream_t st = s.stream;
+    const u32 n = s.n;
+    size_t tb = c.tmp_bytes;
+    cub::CountingInputIterator<u32> ids(0);
+    CK_CUDA(ctx, cub::DeviceSelect::Flagged(c.tmp, tb, ids, c.flags, c.sel, c.n_sel, (int)n, st));
+    k_survivor_lens<<<(n + 256) / 256, 256, 0, st>>>(c.sel, c.n_sel, lens, n, c.len16);
+    tb = c.tmp_bytes;
+    CK_CUDA(ctx, cub::DeviceScan::ExclusiveSum(c.tmp, tb, c.len16, c.coff, (int)n + 1, st));
+    ctx->launches += 3;
+    CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 20, c.n_sel, 4, cudaMemcpyDeviceToHost, st));
+    s.sel = c.sel; s.coff = c.coff;
+    return CK_OK;
+}
+
+// CK_F_SURVIVORS: compact the batch's survivors on the device (indices, 16-byte-aligned compact offsets, canonical bytes); the
+// compact bytes go to the byte arena d_norm (no byte-lane kernel is running any more).
+int enqueue_compaction(ck_ctx *ctx, Slot &s, uint64_t base_index)
+{
+    cudaStream_t st = s.stream;
+    const u32 n = s.n;
+    Compaction c;
+    int rc = compaction_carve(ctx, s, c);
+    if (rc) return rc;
+    k_survivor_flags<<<(n + 255) / 256, 256, 0, st>>>(s.d_first, base_index, n, c.flags);
+    rc = compaction_select_scan(ctx, s, c, s.d_len);
+    if (rc) return rc;
     if (!(s.flags & CK_F_NO_BYTES))
-        k_gather_survivors<<<std::min<u32>((n + 7) / 8, 32u * (u32)ctx->num_sms), 256, 0, st>>>(sel, n_sel, s.d_len, s.d_off, s.d_out,
-                                                                                               (s.flags & CK_F_ALIGNED_OUT) ? 1u : 0u, coff, s.d_norm);
-    ctx->launches += 5;
-    CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 20, n_sel, 4, cudaMemcpyDeviceToHost, st));
-    s.sel = sel; s.coff = coff;
+        k_gather_survivors<<<std::min<u32>((n + 7) / 8, 32u * (u32)ctx->num_sms), 256, 0, st>>>(c.sel, c.n_sel, s.d_len, s.d_off, s.d_out,
+                                                                                               (s.flags & CK_F_ALIGNED_OUT) ? 1u : 0u, c.coff, s.d_norm);
+    ctx->launches += 2;
+    CK_CUDA(ctx, cudaGetLastError());
+    return CK_OK;
+}
+
+// ck_mono_submit's device path, in stream order on the slot's stream: H2D of the raw bytes and offsets to d_raw / d_off;
+// normalise (k_prepare as ck_dev_normalize runs it: bytes to d_norm, lengths to d_len) -> k_monomerize -> k_mono_select ->
+// compaction -> k_mono_gather.  Per record: the worker's end index in d_start, full_len in d_slotof and monomer_len in d_hash
+// (as u32; no canonical form is computed for a monomerize batch).  The compact bytes go to d_out: they need up to
+// offsets[n] + 15 n bytes, and d_out holds out_bytes_total(B, R) >= B + 32 R.
+// The compaction workspace is checked before anything is enqueued, so a refused batch leaves nothing running on the slot.
+int enqueue_mono(ck_ctx *ctx, Slot &s, const uint8_t *bytes, const uint64_t *offsets, const ck_mono_options &o)
+{
+    cudaStream_t st = s.stream;
+    const u32 n = s.n;
+    const bool norm = s.flags & CK_F_NORMALIZE;
+    u32 *end = s.d_start, *full_len = reinterpret_cast<u32 *>(s.d_slotof), *mono_len = reinterpret_cast<u32 *>(s.d_hash);
+    Compaction c;
+    int rc = compaction_carve(ctx, s, c);
+    if (rc) return rc;
+    CK_CUDA(ctx, cudaMemcpyAsync(s.d_off, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, st));
+    if (s.total) CK_CUDA(ctx, cudaMemcpyAsync(s.d_raw, bytes, s.total, cudaMemcpyHostToDevice, st));
+    if (norm) {
+        PrepareArgs pa{s.d_raw, s.d_off, n, 1u | 2u | 4u, nullptr, s.d_norm, s.d_len, nullptr};
+        k_prepare<<<ctx->num_sms * 32, 256, 0, st>>>(pa);
+        ctx->launches++;
+    }
+    MonoArgs ma{};
+    ma.bytes = norm ? s.d_norm : s.d_raw; ma.offsets = s.d_off; ma.lens = norm ? s.d_len : nullptr; ma.n_records = n;
+    ma.seed_len = o.seed_len; ma.use_identity = o.overlap_min_identity >= 0.0 ? 1u : 0u; ma.overlap_dist = o.overlap_dist;
+    ma.identity = o.overlap_min_identity; ma.flags = o.flags & (CK_MONO_SENSITIVE | CK_MONO_FIRST_ONLY); ma.out_end = end;
+    k_monomerize<<<std::min<u32>((n + 7) / 8, 16u * (u32)ctx->num_sms), 256, 0, st>>>(ma);
+    MonoSelectArgs sa{};
+    sa.raw = s.d_raw; sa.offsets = s.d_off; sa.lens = norm ? s.d_len : nullptr; sa.n_records = n; sa.normalize = norm ? 1u : 0u;
+    sa.keep_all = (o.flags & CK_MONO_KEEP_ALL) ? 1u : 0u; sa.seed_len = o.seed_len; sa.min_length = o.min_length;
+    sa.max_length = o.max_length; sa.min_overlap = o.min_overlap; sa.min_overlap_percent = o.min_overlap_percent;
+    sa.end = end; sa.full_len = full_len; sa.monomer_len = mono_len; sa.written = c.flags;
+    const u32 grid = std::min<u32>((n + 7) / 8, 32u * (u32)ctx->num_sms);
+    k_mono_select<<<grid, 256, 0, st>>>(sa);
+    ctx->launches += 2;
+    rc = compaction_select_scan(ctx, s, c, mono_len);
+    if (rc) return rc;
+    if (!(s.flags & CK_F_NO_BYTES)) {
+        k_mono_gather<<<grid, 256, 0, st>>>(s.d_raw, s.d_off, c.sel, c.n_sel, mono_len, c.coff, norm ? 1u : 0u, s.d_out);
+        ctx->launches++;
+    }
     CK_CUDA(ctx, cudaGetLastError());
     return CK_OK;
 }
@@ -759,7 +837,7 @@ int wait_common(ck_ctx *ctx, int slot, bool uniq, uint8_t *out_bytes, uint32_t *
     if (!ctx) return CK_ERR_ARG;
     if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
     Slot &s = ctx->slot[slot];
-    if (!s.busy || s.uniq != uniq) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    if (!s.busy || s.uniq != uniq || s.mono) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
     s.busy = false;
     if (s.n == 0) {
         if (uniq && ctx->peer.attached && ctx->peer.world > 1) CK_CUDA(ctx, cudaStreamSynchronize(s.stream));
@@ -1040,6 +1118,58 @@ int ck_uniq_reset(ck_ctx *ctx)
     CK_CUDA(ctx, cudaMemset(ctx->d_overflow, 0, 4));
     CK_CUDA(ctx, cudaDeviceSynchronize());
     ctx->have_last_insert = false;
+    return CK_OK;
+}
+
+int ck_mono_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, const uint64_t *offsets, uint32_t n_records, uint32_t flags,
+                   const ck_mono_options *opt)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (!opt) return fail(ctx, CK_ERR_ARG, "null options");
+    if (opt->seed_len < 1 || opt->seed_len > 63) return fail(ctx, CK_ERR_ARG, "Seed length must be at least 1 and at most 63");
+    if (opt->overlap_min_identity >= 0.0 && opt->overlap_dist)
+        return fail(ctx, CK_ERR_ARG, "Both overlap_dist and overlap_min_identity are set. They are mutually exclusive");
+    if (opt->flags & ~(CK_MONO_SENSITIVE | CK_MONO_FIRST_ONLY | CK_MONO_KEEP_ALL)) return fail(ctx, CK_ERR_ARG, "unknown option flags");
+    if (flags & ~(CK_F_NORMALIZE | CK_F_NO_BYTES)) return fail(ctx, CK_ERR_ARG, "flags must be CK_F_NORMALIZE / CK_F_NO_BYTES");
+    int rc = submit_check(ctx, slot, offsets, n_records, flags, false, bytes != nullptr, true);
+    if (rc) return rc;
+    Slot &s = ctx->slot[slot];
+    s.mono = true;
+    if (n_records == 0) return submit_empty(ctx, s, 0);
+    CK_CUDA(ctx, cudaSetDevice(ctx->device));
+    rc = enqueue_mono(ctx, s, bytes, offsets, *opt);
+    if (rc) return rc;
+    s.busy = true;
+    return CK_OK;
+}
+int ck_mono_wait(ck_ctx *ctx, int slot, uint32_t *out_n_written, uint32_t *out_index, uint64_t *out_compact_offsets,
+                 uint8_t *out_compact_bytes, uint32_t *out_monomer_len, uint32_t *out_full_len, uint32_t *out_end_index)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    Slot &s = ctx->slot[slot];
+    if (!s.busy || !s.mono) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    s.busy = false;
+    if (out_n_written) *out_n_written = 0;
+    const size_t n = s.n;
+    if (n == 0) return CK_OK;
+    cudaStream_t st = s.stream;
+    if (out_monomer_len) CK_CUDA(ctx, cudaMemcpyAsync(out_monomer_len, s.d_hash, n * 4, cudaMemcpyDeviceToHost, st));
+    if (out_full_len) CK_CUDA(ctx, cudaMemcpyAsync(out_full_len, s.d_slotof, n * 4, cudaMemcpyDeviceToHost, st));
+    if (out_end_index) CK_CUDA(ctx, cudaMemcpyAsync(out_end_index, s.d_start, n * 4, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(ctx, cudaStreamSynchronize(st));
+    const u32 nw = s.h_counts[20];
+    if (out_n_written) *out_n_written = nw;
+    if (nw == 0) return CK_OK;
+    u64 bytes = 0;
+    if (out_index) CK_CUDA(ctx, cudaMemcpyAsync(out_index, s.sel, (size_t)nw * 4, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(ctx, cudaMemcpyAsync(&bytes, s.coff + nw, 8, cudaMemcpyDeviceToHost, st));
+    if (out_compact_offsets) CK_CUDA(ctx, cudaMemcpyAsync(out_compact_offsets, s.coff, ((size_t)nw + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(ctx, cudaStreamSynchronize(st));
+    if (out_compact_bytes && !(s.flags & CK_F_NO_BYTES) && bytes) {
+        CK_CUDA(ctx, cudaMemcpyAsync(out_compact_bytes, s.d_out, bytes, cudaMemcpyDeviceToHost, st));
+        CK_CUDA(ctx, cudaStreamSynchronize(st));
+    }
     return CK_OK;
 }
 

@@ -13,6 +13,7 @@
 // view that reads the monomer backwards through bio's complement table (no reverse complement is materialised).
 #pragma once
 #include "ck_device.cuh"
+#include "ck_kernels.cuh"
 
 namespace ck {
 
@@ -112,6 +113,139 @@ __global__ void __launch_bounds__(256) k_monomerize(MonoArgs a)
             }
         }
         if (lane_id() == 0) a.out_end[rec] = idx;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// The consumer closure of `circkit monomerize` (src/monomerize.rs:102-143) on the device, for the batch API
+// (ck_mono_submit): k_mono_select decides per record what is written and how long it is, the compaction of ck_lib.cu
+// (the one uniq's survivors use) lays the written records out, k_mono_gather writes full_seq[.. monomer_len] of each.
+//
+// full_seq (seq_io 0.3.2 Record::full_seq) is the record without its '\n's and without a '\r' that ends a line or the
+// record.  k_monomerize's index counts normalised symbols but is applied to full_seq, which keeps the ' ' / '\t' that
+// normalisation drops: that is what the reference does.
+struct MonoSelectArgs {
+    const u8 *raw; const u64 *offsets; const u32 *lens;   // lens: normalised lengths (CK_F_NORMALIZE), else nullptr
+    u32 n_records; u32 normalize; u32 keep_all; u32 seed_len;
+    u64 min_length, max_length, min_overlap;                // max_length: ~0 = unset; min_overlap: 0 = unset
+    double min_overlap_percent;                             // NaN = unset
+    u32 *end;              // in: k_monomerize's answer; out: the worker's result (CK_MONO_NONE = None)
+    u32 *full_len, *monomer_len; u8 *written;
+};
+
+// the 16 record bytes src[p .. p + 16) (bytes at or past len read as anything) from aligned 16-byte words
+__device__ __forceinline__ uint4 mono_load16(const u8 *src, u32 p, u32 len)
+{
+    const u8 *b = src + p;
+    const u32 sh = (u32)((size_t)b & 15u);
+    return prep_load16(reinterpret_cast<const uint4 *>(b - sh), sh, sh != 0 && p + 16u - sh < len, p < len);
+}
+__device__ __forceinline__ u32 mono_mask4(u32 w, u32 c)    // bit k: byte k of w equals c
+{
+    return (((__vcmpeq4(w, c) & 0x01010101u) * 0x01020408u) >> 24) & 15u;
+}
+// bit k: byte p + k exists and is not part of full_seq.  Every lane of the warp calls it (lane l + 1 holds the byte after
+// lane l's sixteen; lane 31 reads it).
+__device__ __forceinline__ u32 mono_fullseq_drop(uint4 q, const u8 *src, u32 p, u32 len)
+{
+    const u32 valid = p >= len ? 0u : len - p >= 16 ? 0xffffu : (1u << (len - p)) - 1u;
+    const u32 nl = (mono_mask4(q.x, 0x0a0a0a0au) | mono_mask4(q.y, 0x0a0a0a0au) << 4 | mono_mask4(q.z, 0x0a0a0a0au) << 8
+                    | mono_mask4(q.w, 0x0a0a0a0au) << 12) & valid;
+    const u32 cr = (mono_mask4(q.x, 0x0d0d0d0du) | mono_mask4(q.y, 0x0d0d0d0du) << 4 | mono_mask4(q.z, 0x0d0d0d0du) << 8
+                    | mono_mask4(q.w, 0x0d0d0d0du) << 12) & valid;
+    u32 nxt = __shfl_down_sync(CK_FULL, nl & 1u, 1);
+    if (lane_id() == 31) nxt = p + 16 < len && src[p + 16] == '\n';
+    const u32 last = p < len && len - p <= 16 ? 1u << (len - p - 1) : 0u;
+    return nl | (cr & ((nl >> 1) | (nxt << 15) | last));
+}
+
+__global__ void __launch_bounds__(256) k_mono_select(MonoSelectArgs a)
+{
+    const u32 lane = lane_id();
+    const u32 gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
+    for (u32 rec = gw; rec < a.n_records; rec += nw) {
+        const u64 off = a.offsets[rec];
+        const u32 rawlen = (u32)(a.offsets[rec + 1] - off);
+        u32 full = rawlen;                                  // library semantics: the bytes as they are
+        if (a.normalize) {
+            const u8 *src = a.raw + off;
+            u32 drop = 0;
+            for (u32 base = 0; base < rawlen; base += 512) {
+                const u32 p = base + 16 * lane;
+                drop += __popc(mono_fullseq_drop(mono_load16(src, p, rawlen), src, p, rawlen));
+            }
+            full = rawlen - __reduce_add_sync(CK_FULL, drop);
+        }
+        if (lane == 0) {
+            const u32 n = a.lens ? a.lens[rec] : rawlen;
+            u32 idx = a.end[rec];
+            if (n < a.seed_len || n < a.min_length) idx = CK_MONO_NONE;     // worker closure, src/monomerize.rs:92-96
+            bool ok = idx != CK_MONO_NONE;
+            if (ok) {                                       // consumer closure, :107-135
+                const long long diff = (long long)full - (long long)idx;
+                if (idx < a.min_length || idx > a.max_length) ok = false;
+                if (a.min_overlap && (diff < 0 || (u64)diff < a.min_overlap)) ok = false;
+                if (__ddiv_rn((double)diff, (double)idx) < a.min_overlap_percent) ok = false;   // NaN: false
+            }
+            a.end[rec] = idx;
+            a.full_len[rec] = full;
+            a.monomer_len[rec] = ok ? min(idx, full) : full;
+            a.written[rec] = ok || a.keep_all;
+        }
+    }
+}
+
+#define CK_MONO_STAGE 544u     // 15 carried bytes + 512 + the rounding of the last store, per warp
+
+// One warp per written record k: full_seq[.. monomer_len] (CK_F_NORMALIZE; else the raw bytes) to compact + compact_off[k].
+// The warp reads 512 raw bytes per step (16 per lane), packs the kept ones into a per-warp stage through a warp prefix sum
+// and stores the stage as whole 16-byte vectors (compact_off is 16-byte aligned; the last vector may run into the record's
+// 16-byte rounding); it stops reading once monomer_len bytes are out.
+__global__ void __launch_bounds__(256) k_mono_gather(const u8 *raw, const u64 *offsets, const u32 *sel, const u32 *n_sel,
+                                                     const u32 *monomer_len, const u64 *compact_off, u32 normalize, u8 *compact)
+{
+    __shared__ __align__(16) u8 stage_all[8][CK_MONO_STAGE];
+    u8 *stage = stage_all[threadIdx.x >> 5];
+    const u32 lane = lane_id();
+    const u32 gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
+    const u32 ns = *n_sel;
+    for (u32 k = gw; k < ns; k += nw) {
+        const u32 rec = sel[k], want = monomer_len[rec];
+        const u64 off = offsets[rec];
+        const u32 rawlen = (u32)(offsets[rec + 1] - off);
+        const u8 *src = raw + off;
+        u8 *dst = compact + compact_off[k];
+        u32 done = 0, carry = 0;                            // bytes staged so far / of them still in the stage
+        for (u32 base = 0; done < want && base < rawlen; base += 512) {
+            const u32 p = base + 16 * lane;
+            const uint4 q = mono_load16(src, p, rawlen);
+            u32 keep = p >= rawlen ? 0u : rawlen - p >= 16 ? 0xffffu : (1u << (rawlen - p)) - 1u;
+            if (normalize) keep &= ~mono_fullseq_drop(q, src, p, rawlen);
+            const u32 cnt = __popc(keep);
+            u32 incl = cnt;
+#pragma unroll
+            for (u32 d = 1; d < 32; d <<= 1) {
+                const u32 t = __shfl_up_sync(CK_FULL, incl, d);
+                if (lane >= d) incl += t;
+            }
+            const u32 tot = __shfl_sync(CK_FULL, incl, 31);
+            const u32 room = want - done;
+            u32 j = incl - cnt;
+            for (u32 m = keep; m && j < room; m &= m - 1u) stage[carry + j++] = (u8)prep_byte(q, __ffs(m) - 1);
+            const u32 got = min(tot, room);
+            __syncwarp();
+            const u32 fill = carry + got;
+            const bool last = done + got >= want;
+            const u32 vecs = last ? (fill + 15) / 16 : fill / 16;
+            u8 *out = dst + (done - carry);                 // done - carry: bytes stored so far, a multiple of 16
+            for (u32 c = lane; c < vecs; c += 32) reinterpret_cast<uint4 *>(out)[c] = reinterpret_cast<const uint4 *>(stage)[c];
+            __syncwarp();
+            const u32 rest = last ? 0u : fill - 16 * vecs;
+            if (lane < rest) stage[lane] = stage[16 * vecs + lane];
+            __syncwarp();
+            carry = rest;
+            done += got;
+        }
     }
 }
 

@@ -37,7 +37,7 @@ extern "C" {
 #define CK_ERR_CUDA (-1)       /* a CUDA runtime call failed (no device, out of memory, ...) */
 #define CK_ERR_ARG (-2)        /* bad argument */
 #define CK_ERR_STATE (-3)      /* wait without submit, slot busy, ... */
-#define CK_ERR_TOO_LONG (-4)   /* a record exceeds the supported length (2^30 symbols) */
+#define CK_ERR_TOO_LONG (-4)   /* a record exceeds the supported length (2^30 symbols; ck_mono_submit: 2^32 - 1024 bytes) */
 #define CK_ERR_TABLE_FULL (-5) /* first-occurrence table capacity exhausted */
 
 /* flags of ck_canon_submit / ck_uniq_submit */
@@ -262,6 +262,42 @@ int ck_dev_monomerize(ck_ctx *ctx, void *stream, const uint8_t *bytes, const uin
  * dropped, so out_len[i] <= offsets[i+1] - offsets[i]); feed both to ck_dev_monomerize (`lens`) for the CLI's semantics. */
 int ck_dev_normalize(ck_ctx *ctx, void *stream, const uint8_t *bytes, const uint64_t *offsets, uint32_t n_records,
                      uint8_t *out_bytes, uint32_t *out_len);
+/* Batch API of `circkit monomerize` (host buffers, the two slots of the context, like ck_canon_submit / ck_uniq_submit; a
+ * monomerize batch may be in flight on one slot while a canonicalize / uniq batch is on the other).  ck_mono_submit copies
+ * the raw record bytes in and, in order on the slot's stream: normalises them (flags CK_F_NORMALIZE: the CLI's semantics,
+ * as ck_dev_normalize), runs the monomer search, then the worker and consumer closures' rules (src/monomerize.rs:83-143):
+ *   idx      = None when the (normalised) record is shorter than seed_len or min_length, else the monomer search's answer;
+ *   ok       = idx is not None and none of idx < min_length, idx > max_length, full_len - idx < min_overlap,
+ *              (double)(full_len - idx) / idx < min_overlap_percent holds;
+ *   written  = ok or CK_MONO_KEEP_ALL;   monomer_len = ok ? min(idx, full_len) : full_len;
+ * full_len = length of seq_io's full_seq (the record without '\n' and without a '\r' that ends a line or the record) with
+ * CK_F_NORMALIZE, else the raw length.  The written records' bytes (full_seq[.. monomer_len], or the raw bytes without
+ * CK_F_NORMALIZE) are compacted on the device; CK_F_NO_BYTES skips them.  idx counts normalised symbols and is applied to
+ * full_seq, which keeps the ' ' / '\t' that normalisation drops: the reference does the same.
+ * Every "unset" value below filters nothing, like the reference's None.  seed_len outside 1..63, or identity and a
+ * non-zero distance together -> CK_ERR_ARG (the builder's rules, lib/src/monomerize.rs:20-40).  A record may be up to
+ * 2^32 - 1024 bytes long (lengths are 32-bit; the 2^30 limit of canonicalize / uniq does not apply); a longer one ->
+ * CK_ERR_TOO_LONG. */
+#define CK_MONO_KEEP_ALL 4u
+typedef struct ck_mono_options {
+    uint32_t seed_len;             /* 1..63 */
+    uint32_t flags;                /* CK_MONO_SENSITIVE | CK_MONO_FIRST_ONLY | CK_MONO_KEEP_ALL */
+    uint64_t overlap_dist;         /* --max-mismatch; 0 = unset */
+    double overlap_min_identity;   /* --min-identity; < 0 = unset */
+    uint64_t min_length;           /* --min-length (default 0) */
+    uint64_t max_length;           /* --max-length; UINT64_MAX = unset */
+    uint64_t min_overlap;          /* --min-overlap; 0 = unset */
+    double min_overlap_percent;    /* --min-overlap-percent; NaN = unset */
+} ck_mono_options;
+int ck_mono_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, const uint64_t *offsets, uint32_t n_records,
+                   uint32_t flags /* CK_F_NORMALIZE, CK_F_NO_BYTES */, const ck_mono_options *opt);
+/* Per record of the batch: out_monomer_len, out_full_len and out_end_index (idx above, before the filters; CK_MONO_NONE =
+ * None).  The written records only: *out_n_written; out_index[k] = position in the batch of written record k (increasing);
+ * its bytes at out_compact_bytes[out_compact_offsets[k]] (16-byte aligned, out_monomer_len[out_index[k]] bytes;
+ * out_compact_offsets has n_written + 1 entries, the last one = bytes to expect).  Any out pointer may be NULL.
+ * Size out_index for n_records entries, out_compact_offsets for n_records + 1 and out_compact_bytes for offsets[n] + 16 n_records. */
+int ck_mono_wait(ck_ctx *ctx, int slot, uint32_t *out_n_written, uint32_t *out_index, uint64_t *out_compact_offsets,
+                 uint8_t *out_compact_bytes, uint32_t *out_monomer_len, uint32_t *out_full_len, uint32_t *out_end_index);
 /* number of kernels this context has launched so far (bench.py's gpu_launches) */
 uint64_t ck_launch_count(const ck_ctx *ctx);
 /* per-class kernel timing for the roofline: when enabled, every length/alphabet-class launch is bracketed
