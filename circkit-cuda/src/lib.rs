@@ -70,6 +70,11 @@ pub mod ffi {
     pub const CK_MONO_FIRST_ONLY: u32 = 2;
     pub const CK_MONO_KEEP_ALL: u32 = 4;
     pub const CK_MONO_NONE: u32 = 0xffff_ffff;
+    // FASTA text batches (ck_fasta_submit / ck_fasta_wait): the commands, and uniq -c's body
+    pub const CK_CMD_CANONICALIZE: u32 = 1;
+    pub const CK_CMD_UNIQ: u32 = 2;
+    pub const CK_CMD_MONOMERIZE: u32 = 3;
+    pub const CK_F_CANONICAL_BODY: u32 = 64;
     extern "C" {
         pub fn ck_init(cfg: *const CkConfig, out: *mut *mut CkCtx) -> c_int;
         pub fn ck_destroy(ctx: *mut CkCtx);
@@ -99,6 +104,14 @@ pub mod ffi {
         pub fn ck_mono_wait(ctx: *mut CkCtx, slot: c_int, out_n_written: *mut u32, out_index: *mut u32, out_compact_offsets: *mut u64,
                             out_compact_bytes: *mut u8, out_monomer_len: *mut u32, out_full_len: *mut u32,
                             out_end_index: *mut u32) -> c_int;
+        // FASTA text in, the CLI's output bytes out; `mono` may be null except for CK_CMD_MONOMERIZE, any out pointer may be
+        // null.  Declared from the header; this crate has no Pump over them (callers drive the two slots themselves).
+        pub fn ck_fasta_out_bytes(text_bytes: u64, n_records: u32) -> u64;
+        pub fn ck_fasta_submit(ctx: *mut CkCtx, slot: c_int, text: *const u8, text_bytes: u64, command: u32, flags: u32,
+                               base_index: u64, mono: *const MonoOptions, out_n_records: *mut u32) -> c_int;
+        pub fn ck_fasta_wait(ctx: *mut CkCtx, slot: c_int, out_fasta: *mut u8, out_fasta_bytes: *mut u64, out_n_written: *mut u32,
+                             out_index: *mut u32, out_head: *mut u64, out_first_index: *mut u64, out_full_len: *mut u32,
+                             out_monomer_len: *mut u32) -> c_int;
         pub fn ck_peer_export(ctx: *mut CkCtx, world: u32, rank: u32, max_records: u32, handle_out: *mut c_void) -> c_int;
         pub fn ck_peer_attach(ctx: *mut CkCtx, all_handles: *const c_void) -> c_int;
         pub fn ck_lmsr_index(ctx: *mut CkCtx, s: *const u8, n: usize, out_index: *mut usize) -> c_int;

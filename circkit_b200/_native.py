@@ -13,6 +13,8 @@ CK_ERR_CUDA, CK_ERR_ARG, CK_ERR_STATE, CK_ERR_TOO_LONG, CK_ERR_TABLE_FULL = -1, 
 CK_F_NORMALIZE, CK_F_NO_BYTES, CK_F_ALIGNED_OUT, CK_F_PACKED_IN, CK_F_SURVIVORS, CK_F_SINGLE_COPY = 1, 2, 4, 8, 16, 32
 CK_PEER_HANDLE_BYTES = 64
 CK_MONO_SENSITIVE, CK_MONO_FIRST_ONLY, CK_MONO_KEEP_ALL, CK_MONO_NONE = 1, 2, 4, 0xFFFFFFFF
+CK_CMD_CANONICALIZE, CK_CMD_UNIQ, CK_CMD_MONOMERIZE = 1, 2, 3
+CK_F_CANONICAL_BODY = 64
 CK_CLASS_2BIT_LE_512, CK_CLASS_2BIT_LE_2048, CK_CLASS_2BIT_LE_65536, CK_CLASS_2BIT_LE_425984 = 1, 2, 4, 8
 CK_CLASS_2BIT_LE_4096, CK_CLASS_2BIT_LE_8192 = 1 << 10, 1 << 11
 
@@ -83,6 +85,9 @@ SIGNATURES = {
     "ck_dev_normalize": (_i, [_vp, _vp, _vp, _vp, _u32, _vp, _vp]),
     "ck_mono_submit": (_i, [_vp, _i, _vp, _vp, _u32, _u32, C.POINTER(CkMonoOptions)]),
     "ck_mono_wait": (_i, [_vp, _i, C.POINTER(_u32), _vp, _vp, _vp, _vp, _vp, _vp]),
+    "ck_fasta_out_bytes": (_u64, [_u64, _u32]),
+    "ck_fasta_submit": (_i, [_vp, _i, _vp, _u64, _u32, _u32, _u64, C.POINTER(CkMonoOptions), C.POINTER(_u32)]),
+    "ck_fasta_wait": (_i, [_vp, _i, _vp, C.POINTER(_u64), C.POINTER(_u32), _vp, _vp, _vp, _vp, _vp]),
     "ck_launch_count": (_u64, [_vp]),
     "ck_kernel_timing": (_i, [_vp, _i]),
     "ck_kernel_times": (_i, [_vp, _vp, _vp, _u32]),

@@ -4,18 +4,18 @@
     python -m circkit_b200 uniq [INPUT] [-o OUTPUT] [-c] [--table TABLE] [-t THREADS]
     python -m circkit_b200 monomerize [INPUT] [-o OUTPUT] [--seed-length N] [--max-mismatch N | --min-identity F] ... [--table TABLE]
 
-Mirrors src/canonicalize.rs:7-51 and src/uniq.rs:15-88 with the flags of src/commands.rs:112-149: the host keeps what
-the reference keeps on the host -- reading (with the compression sniffing of src/utils.rs:9-27), FASTA record splitting
-(seq_io 0.3.2 rules), writing in the reference's framing (src/canonicalize.rs:33-37, src/uniq.rs:50-61), the duplicate
-table (src/uniq.rs:62-71, src/utils.rs:74-84) and output compression by suffix (src/utils.rs:29-72) -- and hands batches
-of record bytes, packed to 2 bits per base by `--threads` host threads (ck_pack2_host), to the C ABI (ck_*_submit_packed,
-two slots in flight), where LMSR, the canonical form, XXH3-64, the first-occurrence table and the compaction of the
-survivors run on the GPU.  `monomerize` (src/monomerize.rs:16-160) hands the raw record bytes to ck_mono_submit /
-ck_mono_wait the same way; normalisation, the monomer search, the length / overlap filters and the extraction of the written
-monomers run on the GPU.  Input and output stream in pieces of 64 MB, so files larger than host memory pass through.
-Nothing is printed on success (tests/canon_uniq.rs:74-77); an I/O error exits non-zero with the OS message on stderr.
+Mirrors src/canonicalize.rs:7-51, src/uniq.rs:15-88 and src/monomerize.rs:16-160 with the flags of src/commands.rs:19-149.
+The host reads (with the compression sniffing of src/utils.rs:9-27), cuts the decompressed text into pieces and batches of
+whole records at '\n>' boundaries, writes (output compression by suffix, src/utils.rs:29-72) and builds the --table rows;
+each batch of FASTA text goes to the C ABI's text entries (ck_fasta_submit / ck_fasta_wait, two slots in flight), where
+seq_io 0.3.2's record split, normalisation, LMSR, the canonical form, XXH3-64, the first-occurrence table, the monomer
+search and its filters, and the framing of the written records ('>' head '\n' body '\n', src/canonicalize.rs:33-37,
+src/uniq.rs:50-61) run on the GPU.  What comes back is the bytes to write, plus the head ranges, first indices and
+lengths the id checks and the tables need.  Input and output stream in pieces of 64 MB, so files larger than host memory
+pass through.  Nothing is printed on success (tests/canon_uniq.rs:74-77); an I/O error exits non-zero with the OS message
+on stderr.
 
-Record splitting and output assembly are numpy-vectorised (no per-record Python on the canonicalize path).
+`Records` and `_assemble` state the record split and the framing on the host (seq_io's rules, vectorised with numpy).
 """
 from __future__ import annotations
 
@@ -324,28 +324,46 @@ class Writer:
             self.f.close()
 
 
-def iter_records(chunks):
-    """Records objects over a stream of chunks: every yield holds whole records only (the tail of a chunk that may belong to
-    an unfinished record is carried into the next one).  seq_io's leading-blank-line rule applies to the first piece only."""
+def iter_text(chunks):
+    """Pieces of whole records over a stream of chunks: each piece is cut before the last '\\n>' of what has been read (the
+    record that follows may be unfinished and is carried into the next piece).  Every piece but the first begins with '>';
+    the first keeps seq_io's leading blank lines (see _piece_text)."""
     carry = b""
     first = True
     for c in chunks:
         data = carry + c if carry else c
-        d = np.frombuffer(data, dtype=np.uint8)
-        gt = np.flatnonzero(d == ord(">"))
-        gt = gt[(gt > 0)]
-        gt = gt[d[gt - 1] == 10]
-        if len(gt) == 0:                                     # no record start after the first byte: keep accumulating
+        cut = data.rfind(b"\n>") + 1
+        if cut == 0:                                         # no record start after the first byte: keep accumulating
             carry = data
             continue
-        cut = int(gt[-1])                                    # the last record of the piece may be unfinished: hold it back
         piece, carry = data[:cut], data[cut:]
         if not first and piece[:1] != b">":
             raise FastaError("expected '>' at record start")
         first = False
-        yield Records(piece)
+        yield piece
     if carry or first:
-        yield Records(carry)
+        yield carry
+
+
+def iter_records(chunks):
+    """Records objects over a stream of chunks, cut as iter_text cuts them: every yield holds whole records only.  seq_io's
+    leading-blank-line rule applies to the first piece only."""
+    for piece in iter_text(chunks):
+        yield Records(piece)
+
+
+def _piece_text(piece) -> bytes:
+    """the text of a piece from its first record's '>' on: a Records piece's data, or a text piece of iter_text with seq_io's
+    leading empty lines ("" or "\\r") skipped; any other first line -> FastaError"""
+    if isinstance(piece, Records):
+        return piece.data[int(piece.head_lo[0]) - 1:].tobytes() if len(piece) else b""
+    pos, n = 0, len(piece)
+    while pos < n and piece[pos] != 62:
+        end = piece.find(b"\n", pos)
+        if piece[pos:end if end >= 0 else n] not in (b"", b"\r"):
+            raise FastaError("expected '>' at record start")
+        pos = n if end < 0 else end + 1
+    return piece[pos:] if pos else piece
 
 
 # ------------------------------------------------------------------------------------------------ GPU pump
@@ -353,100 +371,114 @@ MAX_BATCH_BYTES = 256 << 20
 MAX_BATCH_RECORDS = 1 << 20
 
 
-def _batches(offsets: np.ndarray, oversize: bool = False):
-    """cuts of the record range into batches of <= MAX_BATCH_BYTES / MAX_BATCH_RECORDS; oversize=True: a record longer than
-    MAX_BATCH_BYTES is a batch of its own (else FastaError)"""
-    n = len(offsets) - 1
-    cuts = [0]
-    while cuts[-1] < n:
-        lo = cuts[-1]
-        hi = min(n, lo + MAX_BATCH_RECORDS)
-        limit = int(offsets[lo]) + MAX_BATCH_BYTES
-        if int(offsets[hi]) > limit:
-            hi = int(np.searchsorted(offsets, limit, side="right")) - 1
+def _text_batches(text: bytes, max_bytes: int, max_records: int, oversize: bool = False):
+    """(lo, hi) cuts of a piece of whole records (text[0] == '>') at '\\n>' boundaries, each of at most max_bytes bytes and
+    max_records records; a record longer than max_bytes is a cut of its own with oversize=True, else a FastaError"""
+    n, lo = len(text), 0
+    while lo < n:
+        hi = n if n - lo <= max_bytes else text.rfind(b"\n>", lo, lo + max_bytes + 1) + 1
         if hi <= lo:
             if not oversize:
                 raise FastaError("record longer than the batch size")
-            hi = lo + 1
-        cuts.append(hi)
-    return cuts
-
-
-def _pump(ctx: Context, arena: np.ndarray, offsets: np.ndarray, uniq: bool, want_bytes: bool = True, base_index: int = 0,
-          threads: int = 0):
-    """All batches of one piece of the input through the two slots of the C ABI (the bounded queue of parallel_fasta): the
-    host packer (ck_pack2_host, `threads` threads) and the submit of batch b run while batch b - 1 is collected.
-    canonicalize -> (canonical bytes of every record, compact; normalised lengths; None; None)
-    uniq         -> (canonical bytes of the SURVIVORS only, compact -- the device compacts them, CK_F_SURVIVORS; lengths;
-                     first_index of every record; indices of the survivors)"""
-    from .core import pack2_host
-    n = len(offsets) - 1
-    cuts = _batches(offsets)
-    lens = np.zeros(n, dtype=np.uint32)
-    first = np.zeros(n, dtype=np.uint64) if uniq else None
-    outs, keeps = [], []
-    nb = len(cuts) - 1
-    pend = {}
-    for b in range(nb + 1):
-        if b < nb:
-            lo, hi = cuts[b], cuts[b + 1]
-            rel = (offsets[lo: hi + 1] - offsets[lo]).astype(np.uint64)
-            sub = arena[int(offsets[lo]): int(offsets[hi])]
-            pb = pack2_host(sub, rel, normalize=True, threads=threads)
-            if uniq:
-                ctx.uniq_submit_packed(b & 1, pb, base_index + lo, no_bytes=not want_bytes, aligned=True, survivors=True)
-            else:
-                ctx.canon_submit_packed(b & 1, pb, aligned=True)
-            pend[b] = pb                                       # keeps the pinned / host arrays alive until the wait
-        if b >= 1:
-            lo, hi = cuts[b - 1], cuts[b]
-            pb = pend.pop(b - 1)
-            if uniq:
-                r = ctx.uniq_wait_survivors((b - 1) & 1, hi - lo, pb.total, want_bytes=want_bytes)
-                first[lo:hi] = r["first"]
-                lens[lo:hi] = r["lens"]
-                idx = r["index"].astype(np.int64)
-                keeps.append(idx + lo)
-                if want_bytes and len(idx):
-                    st = r["offsets"][:-1].astype(np.int64)
-                    outs.append(r["bytes"][_region_mask(len(r["bytes"]), st, st + r["lens"][idx].astype(np.int64))])
-            else:
-                r = ctx.canon_wait((b - 1) & 1, hi - lo, pb.total, aligned=True)
-                lens[lo:hi] = r["lens"]
-                st = ctx.aligned_starts(pb.offsets).astype(np.int64)
-                outs.append(r["out"][_region_mask(len(r["out"]), st, st + r["lens"].astype(np.int64))])
-    body = np.concatenate(outs) if outs else np.zeros(0, dtype=np.uint8)
-    keep = (np.concatenate(keeps) if keeps else np.zeros(0, dtype=np.int64)) if uniq else None
-    return body, lens, first, keep
+            hi = text.find(b"\n>", lo) + 1 or n
+        if text.count(b"\n>", lo, hi) >= max_records:       # more records than a batch takes: cut after max_records of them
+            d = np.frombuffer(text, dtype=np.uint8, count=hi - lo, offset=lo)
+            hi = lo + int(np.flatnonzero((d[:-1] == 10) & (d[1:] == 62))[max_records - 1]) + 1
+        yield lo, hi
+        lo = hi
 
 
 def _context(table_capacity: int) -> Context:
     return Context(max_batch_bytes=MAX_BATCH_BYTES, max_batch_records=MAX_BATCH_RECORDS, table_capacity=table_capacity)
 
 
-def _piece_arena(recs: "Records"):
-    seq_len = recs.seq_hi - recs.seq_lo
-    offsets = np.zeros(len(recs) + 1, dtype=np.uint64)
-    np.cumsum(seq_len, out=offsets[1:])
-    return np.ascontiguousarray(recs.gather(recs.seq_lo, recs.seq_hi)), offsets, seq_len
+class _Pump:
+    """Text batches through the two slots of a context (ck_fasta_submit / ck_fasta_wait): batch b is copied into slot
+    b & 1's pinned buffer and submitted (the submit returns once the device has split it), then batch b - 1 is collected
+    and handed to done(text, lo, result, base_index, tag); the record split, the command and the output framing run on the
+    device.  Batches come from pieces fed in input order.  A record longer than MAX_BATCH_BYTES (monomerize: oversize=True)
+    is a batch of its own on a second context sized for it."""
+
+    def __init__(self, command: str, done, table_capacity: int = 0, oversize: bool = False, **submit_kw):
+        self.command, self.done, self.oversize, self.kw = command, done, oversize, submit_kw
+        self.ctx, self.big = _context(table_capacity), None
+        self.pinned = {}                                     # (slot, 0 in / 1 out) -> (pointer, uint8 array)
+        self.pend, self.b, self.base = None, 0, 0
+
+    def _buf(self, slot: int, which: int, size: int) -> np.ndarray:
+        p = self.pinned.get((slot, which))
+        if p is None or len(p[1]) < size:
+            if p is not None:
+                self.ctx._lib.ck_free_pinned(self.ctx.handle, p[0])
+            size = (size + (16 << 20) - 1) & ~((16 << 20) - 1)
+            ptr = self.ctx._lib.ck_alloc_pinned(self.ctx.handle, size)
+            if not ptr:
+                raise MemoryError("cannot allocate %d bytes of pinned host memory" % size)
+            p = (ptr, np.ctypeslib.as_array((ctypes.c_uint8 * size).from_address(ptr)))
+            self.pinned[(slot, which)] = p
+        return p[1]
+
+    def feed(self, text: bytes, tag=None):
+        for lo, hi in _text_batches(text, MAX_BATCH_BYTES, MAX_BATCH_RECORDS, self.oversize):
+            slot, size, ctx = self.b & 1, hi - lo, self.ctx
+            if size > MAX_BATCH_BYTES:
+                if self.big is None or self.big.max_batch_bytes < size:
+                    if self.pend is not None and self.pend[0] is self.big:
+                        self._finish()
+                    if self.big is not None:
+                        self.big.close()
+                    self.big = Context(max_batch_bytes=size, max_batch_records=1)
+                ctx = self.big
+            buf = self._buf(slot, 0, size)[:size]
+            buf[:] = np.frombuffer(text, dtype=np.uint8, count=size, offset=lo)
+            n = ctx.fasta_submit(slot, buf, self.command, base_index=self.base, **self.kw)
+            if self.pend is not None:
+                self._finish()
+            self.pend = (ctx, slot, text, lo, self.base, tag, ctx.fasta_out_bytes(size, n))
+            self.base += n
+            self.b += 1
+
+    def _finish(self):
+        ctx, slot, text, lo, base, tag, out_bytes = self.pend
+        self.pend = None
+        self.done(text, lo, ctx.fasta_wait(slot, self._buf(slot, 1, out_bytes)), base, tag)
+
+    def close(self, ok: bool = True):
+        try:
+            if ok and self.pend is not None:
+                self._finish()
+        finally:
+            for p, _ in self.pinned.values():
+                self.ctx._lib.ck_free_pinned(self.ctx.handle, p)
+            self.pinned = {}
+            for c in (self.ctx, self.big):
+                if c is not None:
+                    c.close()
+
+
+def _drive(pieces, command: str, done, piece_tag=None, **kw):
+    """every piece's text through a _Pump (created at the first non-empty piece); piece_tag(text) goes to `done` with each
+    of the piece's batches"""
+    pump = None
+    ok = False
+    try:
+        for piece in pieces:
+            text = _piece_text(piece)
+            if not text:
+                continue
+            if pump is None:
+                pump = _Pump(command, done, **kw)
+            pump.feed(text, piece_tag(text) if piece_tag else None)
+        ok = True
+    finally:
+        if pump is not None:
+            pump.close(ok)
 
 
 def run_canonicalize(pieces, write, threads: int = 0) -> None:
-    """`circkit canonicalize` over a stream of Records pieces (src/canonicalize.rs:7-51); `write(bytes)` gets the output"""
-    ctx = None
-    try:
-        for recs in pieces:
-            if len(recs) == 0:
-                continue
-            if ctx is None:
-                ctx = _context(0)
-            arena, offsets, _ = _piece_arena(recs)
-            body, lens, _, _ = _pump(ctx, arena, offsets, False, threads=threads)
-            heads = recs.gather(recs.head_lo, recs.head_hi)
-            write(_assemble(heads, recs.head_hi - recs.head_lo, body, lens.astype(np.int64)))
-    finally:
-        if ctx is not None:
-            ctx.close()
+    """`circkit canonicalize` over a stream of pieces (text pieces of iter_text or Records; src/canonicalize.rs:7-51):
+    `write(bytes)` gets the output.  `threads` is accepted for the command line's sake: the host does no per-record work."""
+    _drive(pieces, "canonicalize", lambda text, lo, r, base, tag: write(r["fasta"]))
 
 
 def _csv_field(f: bytes, delim: bytes) -> bytes:
@@ -456,68 +488,45 @@ def _csv_field(f: bytes, delim: bytes) -> bytes:
     return f
 
 
-def _check_ids(recs: "Records", which: np.ndarray) -> None:
-    """record.id().unwrap() (src/uniq.rs:48,67): the id -- head up to the first ' ' -- must be UTF-8"""
-    heads = recs.gather(recs.head_lo[which], recs.head_hi[which]).tobytes()
-    try:
-        heads.decode("utf-8")                                 # every head valid => every id valid (the common case)
-        return
-    except UnicodeDecodeError:
-        pass
-    for a, b in zip(recs.head_lo[which].tolist(), recs.head_hi[which].tolist()):
-        recs.data[a:b].tobytes().split(b" ", 1)[0].decode("utf-8")
+def _rec_id(text: bytes, lo: int, head: np.ndarray, i: int) -> bytes:
+    """record.id(): head up to the first ' ' (src/uniq.rs:48,67 unwrap it as UTF-8)"""
+    return text[lo + int(head[i, 0]): lo + int(head[i, 1])].split(b" ", 1)[0]
 
 
 def run_uniq(pieces, write, canonical: bool = False, table_write=None, table_ext: str | None = None, table_capacity: int = 1 << 24,
              threads: int = 0) -> None:
-    """`circkit uniq` over a stream of Records pieces (src/uniq.rs:15-88): one first-occurrence table on the device for the whole
-    input, survivors written piece by piece in input order, duplicate rows to `table_write` as they are met."""
-    ctx = None
-    base = 0
+    """`circkit uniq` over a stream of pieces (src/uniq.rs:15-88): one first-occurrence table on the device for the whole
+    input, survivors written batch by batch in input order, duplicate rows to `table_write` as they are met."""
     first_ids = {}                                             # global index of a first occurrence -> its id (for --table only)
     delim = b"\t" if table_ext == "tsv" else b","
-    wrote_header = False
-    try:
-        for recs in pieces:
-            n = len(recs)
-            if n == 0:
-                continue
-            if ctx is None:
-                ctx = _context(table_capacity)
-            arena, offsets, seq_len = _piece_arena(recs)
-            body, lens, first, keep_idx = _pump(ctx, arena, offsets, True, want_bytes=canonical, base_index=base, threads=threads)
-            keep = np.zeros(n, dtype=bool)
-            keep[keep_idx] = True                               # first occurrence in input order (src/uniq.rs:47-48)
-            _check_ids(recs, np.ones(n, dtype=bool) if table_write is not None else keep)
-            head_len = (recs.head_hi - recs.head_lo)[keep]
-            heads = recs.gather(recs.head_lo[keep], recs.head_hi[keep])
-            if canonical:                                       # src/uniq.rs:53-56: the device returned the survivors' bytes only
-                bodies, body_len = body, lens.astype(np.int64)[keep]
-            else:                                               # raw record.seq(), internal line breaks included (:57-59)
-                bodies, body_len = recs.gather(recs.seq_lo[keep], recs.seq_hi[keep]), seq_len[keep]
-            write(_assemble(heads, head_len, bodies, body_len))
-            if table_write is not None:                         # src/uniq.rs:62-71, csv 1.2.2 defaults
-                def rec_id(i):
-                    return recs.data[recs.head_lo[i]: recs.head_hi[i]].tobytes().split(b" ", 1)[0]
-                for i in keep_idx.tolist():
-                    first_ids[base + i] = rec_id(i)
-                rows = bytearray()
-                for i in np.flatnonzero(~keep).tolist():
-                    if not wrote_header:
-                        rows += b"id" + delim + b"duplicate_id\n"
-                        wrote_header = True
-                    rows += _csv_field(first_ids[int(first[i])], delim) + delim + _csv_field(rec_id(i), delim) + b"\n"
-                table_write(bytes(rows))
-            base += n
-    finally:
-        if ctx is not None:
-            ctx.close()
+    state = {"header": False}
+
+    def done(text, lo, r, base, ascii_text):
+        head, keep_idx = r["head"], r["index"]
+        if not ascii_text:                                     # record.id().unwrap(): survivors, or every record with --table
+            for i in (range(len(head)) if table_write is not None else keep_idx.tolist()):
+                _rec_id(text, lo, head, i).decode("utf-8")
+        write(r["fasta"])
+        if table_write is not None:                            # src/uniq.rs:62-71, csv 1.2.2 defaults
+            for i in keep_idx.tolist():
+                first_ids[base + i] = _rec_id(text, lo, head, i)
+            keep = np.zeros(len(head), dtype=bool)
+            keep[keep_idx] = True
+            rows = bytearray()
+            for i in np.flatnonzero(~keep).tolist():
+                if not state["header"]:
+                    rows += b"id" + delim + b"duplicate_id\n"
+                    state["header"] = True
+                rows += _csv_field(first_ids[int(r["first"][i])], delim) + delim + _csv_field(_rec_id(text, lo, head, i), delim) + b"\n"
+            table_write(bytes(rows))
+
+    _drive(pieces, "uniq", done, bytes.isascii, table_capacity=table_capacity, canonical_body=canonical)
 
 
 def canonicalize(fasta: bytes) -> bytes:
     """bytes of a FASTA file -> bytes `circkit canonicalize` writes (src/canonicalize.rs:7-51)"""
     out = []
-    run_canonicalize(iter_records([fasta] if fasta else []), out.append)
+    run_canonicalize(iter_text([fasta] if fasta else []), out.append)
     return b"".join(out)
 
 
@@ -525,7 +534,7 @@ def uniq(fasta: bytes, canonical: bool = False, table_ext: str | None = None):
     """bytes of a FASTA file -> (bytes `circkit uniq` writes, bytes of the --table file or None) (src/uniq.rs:15-88)"""
     out, table = [], ([] if table_ext is not None else None)
     n_upper = fasta.count(b">") + 1
-    run_uniq(iter_records([fasta] if fasta else []), out.append, canonical, table.append if table is not None else None, table_ext,
+    run_uniq(iter_text([fasta] if fasta else []), out.append, canonical, table.append if table is not None else None, table_ext,
              table_capacity=n_upper)
     return b"".join(out), (b"".join(table) if table is not None else None)
 
@@ -555,78 +564,29 @@ def mono_options(sensitive: bool = False, seed_length: int = 10, max_mismatch=No
                          float("nan") if min_overlap_percent is None else float(min_overlap_percent))
 
 
-def _pump_mono(ctx: Context, big: "Context | None", arena: np.ndarray, offsets: np.ndarray, opts):
-    """All batches of one piece through the two slots (ck_mono_submit / ck_mono_wait): the submit of batch b runs while
-    batch b - 1 is collected.  A record longer than MAX_BATCH_BYTES is a batch of its own on `big`, a context whose staging
-    fits it.  -> (indices of the written records, increasing; their bytes, concatenated; monomer_len[n]; full_len[n])"""
-    n = len(offsets) - 1
-    cuts = _batches(offsets, oversize=True)
-    mono_len = np.zeros(n, dtype=np.int64)
-    full_len = np.zeros(n, dtype=np.int64)
-    idxs, outs = [], []
-    nb = len(cuts) - 1
-    pend = {}
-    for b in range(nb + 1):
-        if b < nb:
-            lo, hi = cuts[b], cuts[b + 1]
-            rel = (offsets[lo: hi + 1] - offsets[lo]).astype(np.uint64)
-            sub = arena[int(offsets[lo]): int(offsets[hi])]
-            c = big if int(rel[-1]) > MAX_BATCH_BYTES else ctx
-            c.mono_submit(b & 1, sub, rel, opts)
-            pend[b] = (c, sub, rel)                              # keeps the host arrays alive until the wait
-        if b >= 1:
-            lo, hi = cuts[b - 1], cuts[b]
-            c, _, rel = pend.pop(b - 1)
-            r = c.mono_wait((b - 1) & 1, hi - lo, int(rel[-1]))
-            mono_len[lo:hi] = r["monomer_len"]
-            full_len[lo:hi] = r["full_len"]
-            if r["n_written"]:
-                idx = r["index"].astype(np.int64)
-                st = r["offsets"][:-1].astype(np.int64)
-                idxs.append(idx + lo)
-                outs.append(r["bytes"][_region_mask(len(r["bytes"]), st, st + mono_len[lo + idx])])
-    written = np.concatenate(idxs) if idxs else np.zeros(0, dtype=np.int64)
-    body = np.concatenate(outs) if outs else np.zeros(0, dtype=np.uint8)
-    return written, body, mono_len, full_len
-
-
 def run_monomerize(pieces, write, opts, table_write=None, table_ext: str | None = None) -> None:
-    """`circkit monomerize` over a stream of Records pieces (src/monomerize.rs:16-160): `opts` from mono_options; normalisation,
-    the monomer search, the length / overlap filters of the consumer closure and the extraction of full_seq[..end] run on the
-    device; `write(bytes)` gets the output ('>' head '\\n' monomer '\\n'), `table_write` the --table rows as pieces complete."""
-    ctx = big = None
+    """`circkit monomerize` over a stream of pieces (src/monomerize.rs:16-160): `opts` from mono_options; normalisation,
+    the monomer search, the length / overlap filters of the consumer closure, the extraction of full_seq[..end] and the
+    framing run on the device; `write(bytes)` gets the output ('>' head '\\n' monomer '\\n'), `table_write` the --table rows
+    as batches complete."""
     delim = b"\t" if table_ext == "tsv" else b","
-    wrote_header = False
-    try:
-        for recs in pieces:
-            n = len(recs)
-            if n == 0:
-                continue
-            arena, offsets, seq_len = _piece_arena(recs)
-            longest = int(seq_len.max())
-            if ctx is None:
-                ctx = _context(0)
-            if longest > MAX_BATCH_BYTES and (big is None or big.max_batch_bytes < longest):
-                if big is not None:
-                    big.close()
-                big = Context(max_batch_bytes=longest, max_batch_records=1)
-            written, body, mono_len, full_len = _pump_mono(ctx, big, arena, offsets, opts)
-            heads = recs.gather(recs.head_lo[written], recs.head_hi[written])
-            write(_assemble(heads, (recs.head_hi - recs.head_lo)[written], body, mono_len[written]))
-            if table_write is not None and len(written):      # :145-154, csv 1.2.2 defaults: header with the first row
-                rows = bytearray()
-                if not wrote_header:
-                    rows += delim.join([b"id", b"original_length", b"monomer_length"]) + b"\n"
-                    wrote_header = True
-                for i in written.tolist():
-                    head = recs.data[recs.head_lo[i]: recs.head_hi[i]].tobytes()
-                    head.decode("utf-8")                         # std::str::from_utf8(record.head()).unwrap()
-                    rows += delim.join([_csv_field(head, delim), b"%d" % full_len[i], b"%d" % mono_len[i]]) + b"\n"
-                table_write(bytes(rows))
-    finally:
-        for c in (ctx, big):
-            if c is not None:
-                c.close()
+    state = {"header": False}
+
+    def done(text, lo, r, base, tag):
+        write(r["fasta"])
+        if table_write is not None and r["n_written"]:       # :145-154, csv 1.2.2 defaults: header with the first row
+            rows = bytearray()
+            if not state["header"]:
+                rows += delim.join([b"id", b"original_length", b"monomer_length"]) + b"\n"
+                state["header"] = True
+            head, full_len, mono_len = r["head"], r["full_len"], r["monomer_len"]
+            for i in r["index"].tolist():
+                h = text[lo + int(head[i, 0]): lo + int(head[i, 1])]
+                h.decode("utf-8")                             # std::str::from_utf8(record.head()).unwrap()
+                rows += delim.join([_csv_field(h, delim), b"%d" % full_len[i], b"%d" % mono_len[i]]) + b"\n"
+            table_write(bytes(rows))
+
+    _drive(pieces, "monomerize", done, oversize=True, mono=opts)
 
 
 def monomerize(fasta: bytes, sensitive: bool = False, seed_length: int = 10, max_mismatch=None, min_identity=None,
@@ -637,7 +597,7 @@ def monomerize(fasta: bytes, sensitive: bool = False, seed_length: int = 10, max
     opts = mono_options(sensitive, seed_length, max_mismatch, min_identity, min_overlap, min_overlap_percent, min_length,
                         max_length, keep_all)
     out, table = [], ([] if table_ext is not None else None)
-    run_monomerize(iter_records([fasta] if fasta else []), out.append, opts, table.append if table is not None else None, table_ext)
+    run_monomerize(iter_text([fasta] if fasta else []), out.append, opts, table.append if table is not None else None, table_ext)
     return b"".join(out), (b"".join(table) if table is not None else None)
 
 
@@ -679,9 +639,12 @@ def main(argv=None) -> int:
         if args.command == "monomerize":                      # argument errors before any file is opened
             opts = mono_options(args.sensitive, args.seed_length, args.max_mismatch, args.min_identity, args.min_overlap,
                                 args.min_overlap_percent, args.min_length, args.max_length, args.keep_all)
-        # every subcommand streams: decompress, split, (pack,) process and write piece by piece (src/utils.rs:9-72)
-        pieces = iter_records(iter_input(args.input))
+        # every subcommand streams: decompress, cut into pieces of whole records, process and write batch by batch
+        # (src/utils.rs:9-72); the record split is the device's
+        pieces = iter_text(iter_input(args.input))
         first = next(pieces, None)                              # open the input (and fail on it) before the output is created
+        if first is not None:
+            first = _piece_text(first)
 
         def chain():
             if first is not None:

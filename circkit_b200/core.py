@@ -81,6 +81,7 @@ class Context:
         self.device = device
         self.max_batch_bytes = max_batch_bytes
         self.max_batch_records = max_batch_records
+        self._text_batch = {}           # slot -> (records, text bytes) of its text batch in flight
 
     # -- plumbing
     @property
@@ -243,6 +244,45 @@ class Context:
         k = int(nw.value)
         return dict(n_written=k, index=index[:k], offsets=offs[:k + 1], bytes=out, monomer_len=mono_len[:n], full_len=full_len[:n],
                     end=end[:n])
+
+    # -- FASTA text batches (ck_fasta_submit / ck_fasta_wait): record split, the command and the output framing on the device
+    _COMMANDS = {"canonicalize": N.CK_CMD_CANONICALIZE, "uniq": N.CK_CMD_UNIQ, "monomerize": N.CK_CMD_MONOMERIZE}
+
+    def fasta_out_bytes(self, text_bytes: int, n_records: int) -> int:
+        return int(self._lib.ck_fasta_out_bytes(text_bytes, n_records))
+
+    def fasta_submit(self, slot: int, text, command: str, *, base_index: int = 0, canonical_body: bool = False,
+                     mono: "N.CkMonoOptions | None" = None) -> int:
+        """ck_fasta_submit: `text` (bytes-like or a uint8 array, e.g. pinned) holds whole FASTA records and begins with '>';
+        `command` is "canonicalize", "uniq" or "monomerize" (`mono`: mono_options).  -> number of records in the text"""
+        a = text if isinstance(text, np.ndarray) else np.frombuffer(text, dtype=np.uint8)
+        n = C.c_uint32(0)
+        flags = N.CK_F_CANONICAL_BODY if canonical_body else 0
+        rc = self._lib.ck_fasta_submit(self._h, slot, a.ctypes.data if len(a) else None, len(a), self._COMMANDS[command], flags,
+                                       base_index, C.byref(mono) if mono is not None else None, C.byref(n))
+        self._check(rc)
+        self._text_batch[slot] = (int(n.value), len(a))
+        return int(n.value)
+
+    def fasta_wait(self, slot: int, out: "np.ndarray | None" = None) -> dict:
+        """ck_fasta_wait -> dict(fasta = the bytes the CLI writes for the batch, n_written, index[nw] (positions of the written
+        records in the batch), head[n, 2] (head ranges in the text), first[n] (uniq), full_len[n] / monomer_len[n]
+        (monomerize)).  `out`: optional uint8 buffer (pinned, for speed) of at least fasta_out_bytes(text_bytes, n) bytes."""
+        n, text_bytes = self._text_batch.pop(slot, (0, 0))
+        need = self.fasta_out_bytes(text_bytes, n)
+        if out is None or len(out) < need:
+            out = np.empty(need, dtype=np.uint8)
+        nbytes, nw = C.c_uint64(0), C.c_uint32(0)
+        index = np.zeros(max(n, 1), dtype=np.uint32)
+        head = np.zeros((max(n, 1), 2), dtype=np.uint64)
+        first = np.zeros(max(n, 1), dtype=np.uint64)
+        full_len = np.zeros(max(n, 1), dtype=np.uint32)
+        mono_len = np.zeros(max(n, 1), dtype=np.uint32)
+        self._check(self._lib.ck_fasta_wait(self._h, slot, out.ctypes.data, C.byref(nbytes), C.byref(nw), _ptr(index), _ptr(head),
+                                            _ptr(first), _ptr(full_len), _ptr(mono_len)))
+        k = int(nw.value)
+        return dict(fasta=out[:int(nbytes.value)].tobytes(), n_written=k, index=index[:k], head=head[:n], first=first[:n],
+                    full_len=full_len[:n], monomer_len=mono_len[:n])
 
     def uniq_batch(self, arena: np.ndarray, offsets: np.ndarray, base_index: int = 0, *, normalize: bool = False,
                    want_bytes=True, aligned=False):

@@ -24,6 +24,7 @@
 #include "ck_lane4.cuh"
 #include "ck_synth.cuh"
 #include "ck_monomerize.cuh"
+#include "ck_fasta.cuh"
 
 using namespace ck;
 
@@ -99,6 +100,13 @@ struct Slot {
     u32 *h_counts = nullptr;            // pinned
     ExecScratch scr;
     bool busy = false, uniq = false, mono = false;   // mono: ck_mono_submit's batch (ck_mono_wait collects it)
+    bool text = false;                  // ck_fasta_submit's batch (ck_fasta_wait collects it)
+    u32 cmd = 0;                        // its CK_CMD_*
+    // text batches, allocated by the first ck_fasta_submit on the slot: the text, the framed output, the record starts,
+    // head / seq ranges (2 per record), 64-bit lengths (seq, then framed), framed offsets, tile counts / offsets, the longest seq
+    u8 *d_text = nullptr, *d_frame = nullptr;
+    u64 *d_rstart = nullptr, *d_head = nullptr, *d_seq = nullptr, *d_len64 = nullptr, *d_fofs = nullptr, *d_meta = nullptr;
+    u32 *d_tiles = nullptr;
     u32 dbl = 1;                        // packed2 layout of the batch in flight
     u64 longest = 0;                    // longest raw record of the batch in flight
     u32 *sel = nullptr; u64 *coff = nullptr;    // CK_F_SURVIVORS: survivor indices / compact offsets of the batch in flight
@@ -580,6 +588,17 @@ int peer_first_index(ck_ctx *ctx, cudaStream_t st, u32 slot, const u64 *hash, u3
 // through a record 512 bytes at a time, so positions up to length + 511 must fit.  (Canonicalize / uniq: 2^30 symbols.)
 constexpr u64 kMonoMaxRecord = (1ull << 32) - 1024;
 
+// the builder's rules (lib/src/monomerize.rs:20-40) and the known option flags
+int mono_options_check(ck_ctx *ctx, const ck_mono_options *opt)
+{
+    if (!opt) return fail(ctx, CK_ERR_ARG, "null options");
+    if (opt->seed_len < 1 || opt->seed_len > 63) return fail(ctx, CK_ERR_ARG, "Seed length must be at least 1 and at most 63");
+    if (opt->overlap_min_identity >= 0.0 && opt->overlap_dist)
+        return fail(ctx, CK_ERR_ARG, "Both overlap_dist and overlap_min_identity are set. They are mutually exclusive");
+    if (opt->flags & ~(CK_MONO_SENSITIVE | CK_MONO_FIRST_ONLY | CK_MONO_KEEP_ALL)) return fail(ctx, CK_ERR_ARG, "unknown option flags");
+    return CK_OK;
+}
+
 // shared front of every submit: slot and batch checks.  Returns CK_OK with s.busy still false; n_records == 0 is complete.
 int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_records, uint32_t flags, bool uniq, bool have_bytes,
                  bool mono = false)
@@ -592,7 +611,7 @@ int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_reco
     if (n_records && (!offsets || (!have_bytes && offsets[n_records] != offsets[0])))
         return fail(ctx, CK_ERR_ARG, "null batch pointers");
     if (uniq && !ctx->table) return fail(ctx, CK_ERR_STATE, "context was created with table_capacity 0");
-    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.total = 0;
+    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.text = false; s.total = 0;
     if (n_records == 0) return CK_OK;
     if (offsets[0] != 0) return fail(ctx, CK_ERR_ARG, "offsets[0] must be 0");
     const u64 total = offsets[n_records];
@@ -674,23 +693,20 @@ int enqueue_compaction(ck_ctx *ctx, Slot &s, uint64_t base_index)
     return CK_OK;
 }
 
-// ck_mono_submit's device path, in stream order on the slot's stream: H2D of the raw bytes and offsets to d_raw / d_off;
-// normalise (k_prepare as ck_dev_normalize runs it: bytes to d_norm, lengths to d_len) -> k_monomerize -> k_mono_select ->
+// The device path of a monomerize batch whose raw bytes and offsets are in d_raw / d_off (ck_mono_submit copies them in,
+// ck_fasta_submit splits them out of the text), in stream order on the slot's stream: normalise (k_prepare as ck_dev_normalize runs it: bytes to d_norm, lengths to d_len) -> k_monomerize -> k_mono_select ->
 // compaction -> k_mono_gather.  Per record: the worker's end index in d_start, full_len in d_slotof and monomer_len in d_hash
 // (as u32; no canonical form is computed for a monomerize batch).  The compact bytes go to d_out: they need up to
 // offsets[n] + 15 n bytes, and d_out holds out_bytes_total(B, R) >= B + 32 R.
-// The compaction workspace is checked before anything is enqueued, so a refused batch leaves nothing running on the slot.
-int enqueue_mono(ck_ctx *ctx, Slot &s, const uint8_t *bytes, const uint64_t *offsets, const ck_mono_options &o)
+// The callers carve the compaction workspace (`c`) before they enqueue anything, so a refused batch leaves nothing running
+// on the slot.
+int enqueue_mono(ck_ctx *ctx, Slot &s, const Compaction &c, const ck_mono_options &o)
 {
     cudaStream_t st = s.stream;
     const u32 n = s.n;
     const bool norm = s.flags & CK_F_NORMALIZE;
     u32 *end = s.d_start, *full_len = reinterpret_cast<u32 *>(s.d_slotof), *mono_len = reinterpret_cast<u32 *>(s.d_hash);
-    Compaction c;
-    int rc = compaction_carve(ctx, s, c);
-    if (rc) return rc;
-    CK_CUDA(ctx, cudaMemcpyAsync(s.d_off, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, st));
-    if (s.total) CK_CUDA(ctx, cudaMemcpyAsync(s.d_raw, bytes, s.total, cudaMemcpyHostToDevice, st));
+    int rc;
     if (norm) {
         PrepareArgs pa{s.d_raw, s.d_off, n, 1u | 2u | 4u, nullptr, s.d_norm, s.d_len, nullptr};
         k_prepare<<<ctx->num_sms * 32, 256, 0, st>>>(pa);
@@ -781,6 +797,19 @@ int submit_empty(ck_ctx *ctx, Slot &s, uint64_t base_index)
     return CK_OK;
 }
 
+// canonicalize / uniq over raw bytes and offsets already in d_raw / d_off (ck_canon_submit / ck_uniq_submit copy them in,
+// ck_fasta_submit splits them out of the text): k_prepare -> k_extend_packed2 -> submit_tail
+int enqueue_canon(ck_ctx *ctx, Slot &s, uint64_t base_index)
+{
+    cudaStream_t st = s.stream;
+    const u32 n_records = s.n, flags = s.flags;
+    PrepareArgs pa{s.d_raw, s.d_off, n_records, (flags & CK_F_NORMALIZE) | (s.dbl << 2), s.d_p2, s.d_norm, s.d_len, s.d_lane};
+    k_prepare<<<ctx->num_sms * 32, 256, 0, st>>>(pa);
+    k_extend_packed2<<<extend_grid(ctx, n_records), 256, 0, st>>>(s.d_p2, s.d_off, s.d_len, s.d_lane, n_records, nullptr, s.dbl);
+    ctx->launches += 2;
+    return submit_tail(ctx, s, (flags & CK_F_NORMALIZE) != 0, base_index);
+}
+
 int submit_common(ck_ctx *ctx, int slot, const uint8_t *bytes, const uint64_t *offsets, uint32_t n_records,
                   uint32_t flags, bool uniq, uint64_t base_index)
 {
@@ -793,11 +822,7 @@ int submit_common(ck_ctx *ctx, int slot, const uint8_t *bytes, const uint64_t *o
     CK_CUDA(ctx, cudaSetDevice(ctx->device));
     CK_CUDA(ctx, cudaMemcpyAsync(s.d_off, offsets, (size_t)(n_records + 1) * 8, cudaMemcpyHostToDevice, st));
     if (total) CK_CUDA(ctx, cudaMemcpyAsync(s.d_raw, bytes, total, cudaMemcpyHostToDevice, st));
-    PrepareArgs pa{s.d_raw, s.d_off, n_records, (flags & CK_F_NORMALIZE) | (s.dbl << 2), s.d_p2, s.d_norm, s.d_len, s.d_lane};
-    k_prepare<<<ctx->num_sms * 32, 256, 0, st>>>(pa);
-    k_extend_packed2<<<extend_grid(ctx, n_records), 256, 0, st>>>(s.d_p2, s.d_off, s.d_len, s.d_lane, n_records, nullptr, s.dbl);
-    ctx->launches += 2;
-    return submit_tail(ctx, s, (flags & CK_F_NORMALIZE) != 0, base_index);
+    return enqueue_canon(ctx, s, base_index);
 }
 
 // CK_F_PACKED_IN: the batch arrives as the host packer (ck_pack2_host) left it -- 2 bits per base for the A/C/G/T records,
@@ -837,7 +862,7 @@ int wait_common(ck_ctx *ctx, int slot, bool uniq, uint8_t *out_bytes, uint32_t *
     if (!ctx) return CK_ERR_ARG;
     if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
     Slot &s = ctx->slot[slot];
-    if (!s.busy || s.uniq != uniq || s.mono) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    if (!s.busy || s.uniq != uniq || s.mono || s.text) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
     s.busy = false;
     if (s.n == 0) {
         if (uniq && ctx->peer.attached && ctx->peer.world > 1) CK_CUDA(ctx, cudaStreamSynchronize(s.stream));
@@ -961,7 +986,8 @@ void ck_destroy(ck_ctx *ctx)
     for (int k = 0; k < 2; k++) {
         Slot &s = ctx->slot[k];
         void *ptrs[] = {s.d_raw, s.d_off, s.d_p2, s.d_norm, s.d_len, s.d_lane, s.d_out, s.d_start, s.d_strand,
-                        s.d_hash, s.d_first, s.d_slotof, s.d_lists, s.d_counts, s.d_dense, s.d_laneoff, s.d_p4};
+                        s.d_hash, s.d_first, s.d_slotof, s.d_lists, s.d_counts, s.d_dense, s.d_laneoff, s.d_p4,
+                        s.d_text, s.d_frame, s.d_rstart, s.d_head, s.d_seq, s.d_len64, s.d_fofs, s.d_meta, s.d_tiles};
         for (void *p : ptrs) if (p) cudaFree(p);
         if (s.h_counts) cudaFreeHost(s.h_counts);
         if (s.stream) cudaStreamDestroy(s.stream);
@@ -1077,7 +1103,7 @@ int ck_uniq_wait_survivors(ck_ctx *ctx, int slot, uint32_t *out_n_survivors, uin
     if (!ctx) return CK_ERR_ARG;
     if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
     Slot &s = ctx->slot[slot];
-    if (!s.busy || !s.uniq) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    if (!s.busy || !s.uniq || s.text) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
     if (!out_n_survivors) return fail(ctx, CK_ERR_ARG, "null argument");
     if (s.n && !(s.flags & CK_F_SURVIVORS)) return fail(ctx, CK_ERR_STATE, "the batch was not submitted with CK_F_SURVIVORS");
     *out_n_survivors = 0;
@@ -1125,19 +1151,21 @@ int ck_mono_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, const uint64_t *
                    const ck_mono_options *opt)
 {
     if (!ctx) return CK_ERR_ARG;
-    if (!opt) return fail(ctx, CK_ERR_ARG, "null options");
-    if (opt->seed_len < 1 || opt->seed_len > 63) return fail(ctx, CK_ERR_ARG, "Seed length must be at least 1 and at most 63");
-    if (opt->overlap_min_identity >= 0.0 && opt->overlap_dist)
-        return fail(ctx, CK_ERR_ARG, "Both overlap_dist and overlap_min_identity are set. They are mutually exclusive");
-    if (opt->flags & ~(CK_MONO_SENSITIVE | CK_MONO_FIRST_ONLY | CK_MONO_KEEP_ALL)) return fail(ctx, CK_ERR_ARG, "unknown option flags");
+    int rc = mono_options_check(ctx, opt);
+    if (rc) return rc;
     if (flags & ~(CK_F_NORMALIZE | CK_F_NO_BYTES)) return fail(ctx, CK_ERR_ARG, "flags must be CK_F_NORMALIZE / CK_F_NO_BYTES");
-    int rc = submit_check(ctx, slot, offsets, n_records, flags, false, bytes != nullptr, true);
+    rc = submit_check(ctx, slot, offsets, n_records, flags, false, bytes != nullptr, true);
     if (rc) return rc;
     Slot &s = ctx->slot[slot];
     s.mono = true;
     if (n_records == 0) return submit_empty(ctx, s, 0);
     CK_CUDA(ctx, cudaSetDevice(ctx->device));
-    rc = enqueue_mono(ctx, s, bytes, offsets, *opt);
+    Compaction c;
+    if ((rc = compaction_carve(ctx, s, c))) return rc;
+    cudaStream_t st = s.stream;
+    CK_CUDA(ctx, cudaMemcpyAsync(s.d_off, offsets, (size_t)(n_records + 1) * 8, cudaMemcpyHostToDevice, st));
+    if (s.total) CK_CUDA(ctx, cudaMemcpyAsync(s.d_raw, bytes, s.total, cudaMemcpyHostToDevice, st));
+    rc = enqueue_mono(ctx, s, c, *opt);
     if (rc) return rc;
     s.busy = true;
     return CK_OK;
@@ -1148,7 +1176,7 @@ int ck_mono_wait(ck_ctx *ctx, int slot, uint32_t *out_n_written, uint32_t *out_i
     if (!ctx) return CK_ERR_ARG;
     if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
     Slot &s = ctx->slot[slot];
-    if (!s.busy || !s.mono) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    if (!s.busy || !s.mono || s.text) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
     s.busy = false;
     if (out_n_written) *out_n_written = 0;
     const size_t n = s.n;
@@ -1170,6 +1198,167 @@ int ck_mono_wait(ck_ctx *ctx, int slot, uint32_t *out_n_written, uint32_t *out_i
         CK_CUDA(ctx, cudaMemcpyAsync(out_compact_bytes, s.d_out, bytes, cudaMemcpyDeviceToHost, st));
         CK_CUDA(ctx, cudaStreamSynchronize(st));
     }
+    return CK_OK;
+}
+
+// ---- FASTA text batches (ck_fasta_submit / ck_fasta_wait; csrc/ck_fasta.cuh) -----------------------
+uint64_t ck_fasta_out_bytes(uint64_t text_bytes, uint32_t n_records) { return text_bytes + 2ull * n_records + 64; }
+
+static int text_alloc(ck_ctx *ctx, Slot &s)
+{
+    const u64 B = ctx->cfg.max_batch_bytes, R = ctx->cfg.max_batch_records;
+    const u64 tiles = (B + CK_FASTA_TILE - 1) / CK_FASTA_TILE + 1;
+    // 64 bytes of slack past the text: the start masks read whole 16-byte words, the copies read one aligned word ahead
+    if (!s.d_text) CK_CUDA(ctx, cudaMalloc(&s.d_text, B + 64));
+    if (!s.d_frame) CK_CUDA(ctx, cudaMalloc(&s.d_frame, ck_fasta_out_bytes(B, (u32)R)));
+    if (!s.d_rstart) CK_CUDA(ctx, cudaMalloc(&s.d_rstart, (R + 1) * 8));
+    if (!s.d_head) CK_CUDA(ctx, cudaMalloc(&s.d_head, (R + 1) * 16));
+    if (!s.d_seq) CK_CUDA(ctx, cudaMalloc(&s.d_seq, (R + 1) * 16));
+    if (!s.d_len64) CK_CUDA(ctx, cudaMalloc(&s.d_len64, (R + 1) * 8));
+    if (!s.d_fofs) CK_CUDA(ctx, cudaMalloc(&s.d_fofs, (R + 1) * 8));
+    if (!s.d_meta) CK_CUDA(ctx, cudaMalloc(&s.d_meta, 64));
+    if (!s.d_tiles) CK_CUDA(ctx, cudaMalloc(&s.d_tiles, 2 * tiles * 4));
+    return CK_OK;
+}
+
+// Record split of the text in d_text (nbytes >= 1): starts, ranges, the record count to h_counts[24] and the longest seq to
+// h_counts[26..27]; the caller synchronises.  Scan temporaries live in the slot's sort workspace (free: the slot is idle).
+static int enqueue_split(ck_ctx *ctx, Slot &s, u64 nbytes)
+{
+    cudaStream_t st = s.stream;
+    const u32 R = ctx->cfg.max_batch_records;
+    const u64 tiles = (nbytes + CK_FASTA_TILE - 1) / CK_FASTA_TILE;
+    u32 *count = s.d_tiles, *off = s.d_tiles + tiles + 1;
+    const size_t have = lists_bytes_for(R);
+    size_t need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, count, off, (int)(tiles + 1), st);
+    if (need > have) return fail(ctx, CK_ERR_ARG, "sort workspace too small for the record split");
+    k_fasta_count<<<(u32)tiles, 256, 0, st>>>(s.d_text, nbytes, count);
+    CK_CUDA(ctx, cub::DeviceScan::ExclusiveSum(s.d_lists, need, count, off, (int)(tiles + 1), st));
+    k_fasta_starts<<<(u32)tiles, 256, 0, st>>>(s.d_text, nbytes, off, R, s.d_rstart);
+    CK_CUDA(ctx, cudaMemsetAsync(s.d_meta, 0, 8, st));
+    FastaRangeArgs ra{s.d_text, nbytes, s.d_rstart, off + tiles, R, s.d_head, s.d_seq, s.d_len64, s.d_meta};
+    k_fasta_ranges<<<std::min<u32>((R + 7) / 8, 32u * (u32)ctx->num_sms), 256, 0, st>>>(ra);
+    ctx->launches += 4;
+    CK_CUDA(ctx, cudaGetLastError());
+    CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 24, off + tiles, 4, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 26, s.d_meta, 8, cudaMemcpyDeviceToHost, st));
+    return CK_OK;
+}
+
+// Framing of the written records: c.sel / c.n_sel hold them (selected already), d_len64 takes the framed lengths, d_fofs their
+// exclusive scan, d_frame the bytes; the byte count goes to h_counts[22..23].
+static int enqueue_frame(ck_ctx *ctx, Slot &s, const Compaction &c, u32 body, const u64 *coff)
+{
+    cudaStream_t st = s.stream;
+    const u32 n = s.n;
+    FastaFrameArgs fa{};
+    fa.text = s.d_text; fa.head = s.d_head; fa.seq = s.d_seq; fa.sel = c.sel; fa.n_sel = c.n_sel; fa.n = n; fa.body = body;
+    fa.arena = s.d_out; fa.off = s.d_off; fa.coff = coff;
+    fa.lens = body == CK_FRAME_COMPACT ? reinterpret_cast<const u32 *>(s.d_hash) : s.d_len;
+    fa.flen = s.d_len64; fa.fofs = s.d_fofs; fa.frame = s.d_frame;
+    k_fasta_frame_lens<<<(n + 256) / 256, 256, 0, st>>>(fa);
+    size_t tb = c.tmp_bytes;
+    CK_CUDA(ctx, cub::DeviceScan::ExclusiveSum(c.tmp, tb, s.d_len64, s.d_fofs, (int)n + 1, st));
+    k_fasta_frame<<<std::min<u32>((n + 7) / 8, 32u * (u32)ctx->num_sms), 256, 0, st>>>(fa);
+    ctx->launches += 3;
+    CK_CUDA(ctx, cudaGetLastError());
+    CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 22, s.d_fofs + n, 8, cudaMemcpyDeviceToHost, st));
+    return CK_OK;
+}
+
+int ck_fasta_submit(ck_ctx *ctx, int slot, const uint8_t *text, uint64_t text_bytes, uint32_t command, uint32_t flags,
+                    uint64_t base_index, const ck_mono_options *mono, uint32_t *out_n_records)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (out_n_records) *out_n_records = 0;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    if (command < CK_CMD_CANONICALIZE || command > CK_CMD_MONOMERIZE) return fail(ctx, CK_ERR_ARG, "unknown command");
+    const bool uniq = command == CK_CMD_UNIQ, is_mono = command == CK_CMD_MONOMERIZE;
+    if (flags & ~(uniq ? CK_F_CANONICAL_BODY : 0u)) return fail(ctx, CK_ERR_ARG, "flags must be 0 (CK_F_CANONICAL_BODY: uniq only)");
+    if (text_bytes && !text) return fail(ctx, CK_ERR_ARG, "null text");
+    if (text_bytes && text[0] != '>') return fail(ctx, CK_ERR_ARG, "text must begin with '>'");
+    if (text_bytes > ctx->cfg.max_batch_bytes) return fail(ctx, CK_ERR_ARG, "text exceeds max_batch_bytes");
+    Slot &s = ctx->slot[slot];
+    if (!s.stream) return fail(ctx, CK_ERR_STATE, "context was created without batch slots");
+    if (s.busy) return fail(ctx, CK_ERR_STATE, "slot already holds a batch; call the matching wait first");
+    if (uniq && !ctx->table) return fail(ctx, CK_ERR_STATE, "context was created with table_capacity 0");
+    if (uniq && ctx->peer.attached) return fail(ctx, CK_ERR_STATE, "text batches do not run in a peer group");
+    int rc;
+    if (is_mono && (rc = mono_options_check(ctx, mono))) return rc;
+    CK_CUDA(ctx, cudaSetDevice(ctx->device));
+    if ((rc = text_alloc(ctx, s))) return rc;
+    s.n = 0; s.total = 0; s.uniq = uniq; s.mono = is_mono; s.text = true; s.cmd = command;
+    s.flags = CK_F_NORMALIZE | (is_mono ? 0u : CK_F_ALIGNED_OUT) | (uniq && !(flags & CK_F_CANONICAL_BODY) ? CK_F_NO_BYTES : 0u);
+    if (text_bytes == 0) return submit_empty(ctx, s, base_index);
+    cudaStream_t st = s.stream;
+    CK_CUDA(ctx, cudaMemcpyAsync(s.d_text, text, text_bytes, cudaMemcpyHostToDevice, st));
+    if ((rc = enqueue_split(ctx, s, text_bytes))) return rc;
+    CK_CUDA(ctx, cudaStreamSynchronize(st));
+    const u32 n = s.h_counts[24];
+    u64 longest;
+    memcpy(&longest, s.h_counts + 26, 8);
+    if (out_n_records) *out_n_records = n;
+    if (n > ctx->cfg.max_batch_records) return fail(ctx, CK_ERR_ARG, "text holds more records than max_batch_records");
+    if (is_mono && longest > kMonoMaxRecord) return fail(ctx, CK_ERR_TOO_LONG, "record longer than 2^32 - 1024 bytes");
+    if (!is_mono && longest > (1ull << 30)) return fail(ctx, CK_ERR_TOO_LONG, "record longer than 2^30 symbols");
+    s.n = n; s.longest = longest; s.dbl = longest > 512 ? 1u : 0u;   // as submit_check
+    Compaction c;
+    if ((rc = compaction_carve(ctx, s, c))) return rc;
+    // the arena of the seq bytes, as the host-buffer entries receive it
+    size_t tb = c.tmp_bytes;
+    CK_CUDA(ctx, cub::DeviceScan::ExclusiveSum(c.tmp, tb, s.d_len64, s.d_off, (int)n + 1, st));
+    k_fasta_gather<<<std::min<u32>((n + 7) / 8, 32u * (u32)ctx->num_sms), 256, 0, st>>>(s.d_text, s.d_seq, s.d_off, n, s.d_raw);
+    ctx->launches += 2;
+    if (is_mono) {
+        if ((rc = enqueue_mono(ctx, s, c, *mono))) return rc;
+        if ((rc = enqueue_frame(ctx, s, c, CK_FRAME_COMPACT, c.coff))) return rc;
+    } else {
+        if ((rc = enqueue_canon(ctx, s, base_index))) return rc;   // leaves the slot busy
+        // the written records: all (canonicalize) or the first occurrences (uniq)
+        if (uniq) { k_survivor_flags<<<(n + 255) / 256, 256, 0, st>>>(s.d_first, base_index, n, c.flags); ctx->launches++; }
+        else CK_CUDA(ctx, cudaMemsetAsync(c.flags, 1, n, st));
+        size_t sb = c.tmp_bytes;
+        cub::CountingInputIterator<u32> ids(0);
+        CK_CUDA(ctx, cub::DeviceSelect::Flagged(c.tmp, sb, ids, c.flags, c.sel, c.n_sel, (int)n, st));
+        CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 20, c.n_sel, 4, cudaMemcpyDeviceToHost, st));
+        s.sel = c.sel;
+        ctx->launches++;
+        if ((rc = enqueue_frame(ctx, s, c, (s.flags & CK_F_NO_BYTES) ? CK_FRAME_RAW : CK_FRAME_CANON, nullptr))) return rc;
+    }
+    s.busy = true;
+    return CK_OK;
+}
+
+int ck_fasta_wait(ck_ctx *ctx, int slot, uint8_t *out_fasta, uint64_t *out_fasta_bytes, uint32_t *out_n_written,
+                  uint32_t *out_index, uint64_t *out_head, uint64_t *out_first_index, uint32_t *out_full_len,
+                  uint32_t *out_monomer_len)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    Slot &s = ctx->slot[slot];
+    if (!s.busy || !s.text) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    s.busy = false;
+    if (out_fasta_bytes) *out_fasta_bytes = 0;
+    if (out_n_written) *out_n_written = 0;
+    const size_t n = s.n;
+    if (n == 0) return CK_OK;
+    cudaStream_t st = s.stream;
+    if (out_head) CK_CUDA(ctx, cudaMemcpyAsync(out_head, s.d_head, n * 16, cudaMemcpyDeviceToHost, st));
+    if (out_first_index && s.uniq) CK_CUDA(ctx, cudaMemcpyAsync(out_first_index, s.d_first, n * 8, cudaMemcpyDeviceToHost, st));
+    if (out_full_len && s.mono) CK_CUDA(ctx, cudaMemcpyAsync(out_full_len, s.d_slotof, n * 4, cudaMemcpyDeviceToHost, st));
+    if (out_monomer_len && s.mono) CK_CUDA(ctx, cudaMemcpyAsync(out_monomer_len, s.d_hash, n * 4, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(ctx, cudaStreamSynchronize(st));
+    if (!s.mono && s.h_counts[CLS_HUGE]) return fail(ctx, CK_ERR_TOO_LONG, "batch holds a record beyond the staged-length classes");
+    if (s.uniq && s.h_counts[16]) return fail(ctx, CK_ERR_TABLE_FULL, "uniq table is full; raise table_capacity");
+    const u32 nw = s.h_counts[20];
+    u64 bytes;
+    memcpy(&bytes, s.h_counts + 22, 8);
+    if (out_n_written) *out_n_written = nw;
+    if (out_fasta_bytes) *out_fasta_bytes = bytes;
+    if (out_index && nw) CK_CUDA(ctx, cudaMemcpyAsync(out_index, s.sel, (size_t)nw * 4, cudaMemcpyDeviceToHost, st));
+    if (out_fasta && bytes) CK_CUDA(ctx, cudaMemcpyAsync(out_fasta, s.d_frame, bytes, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(ctx, cudaStreamSynchronize(st));
     return CK_OK;
 }
 

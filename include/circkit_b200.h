@@ -53,6 +53,7 @@ extern "C" {
 
 #define CK_F_SURVIVORS 16u  /* uniq: also compact the survivors on the device, for ck_uniq_wait_survivors */
 #define CK_F_SINGLE_COPY 32u /* device-resident API: the packed2 arena is in the single-copy layout (batches of records <= 512 bases) */
+/* 64u: CK_F_CANONICAL_BODY of ck_fasta_submit (below) */
 #define CK_F_PACKED_IN 8u   /* (set by the *_submit_packed entries) the batch came through ck_pack2_host */
 
 typedef struct ck_ctx ck_ctx;
@@ -298,6 +299,43 @@ int ck_mono_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, const uint64_t *
  * Size out_index for n_records entries, out_compact_offsets for n_records + 1 and out_compact_bytes for offsets[n] + 16 n_records. */
 int ck_mono_wait(ck_ctx *ctx, int slot, uint32_t *out_n_written, uint32_t *out_index, uint64_t *out_compact_offsets,
                  uint8_t *out_compact_bytes, uint32_t *out_monomer_len, uint32_t *out_full_len, uint32_t *out_end_index);
+
+/* ---- FASTA text batches: `circkit canonicalize` / `uniq` / `monomerize` from decompressed text to written bytes ----------
+ * ck_fasta_submit takes FASTA text as it comes out of the decompressor, on one of the two slots, and does on the slot's
+ * stream everything the CLI's worker and consumer closures do, with seq_io 0.3.2's record split before and the CLI's output
+ * framing after:
+ *   text         whole records; text[0] must be '>' (leading blank lines are the caller's to strip) -> else CK_ERR_ARG;
+ *                a record starts at a '>' at position 0 or after a '\n'; head = the header line without '>' and without
+ *                one trailing '\r'; seq = from after the header's '\n' to the record's last '\n' (or the end of the
+ *                text), one trailing '\r' trimmed; the last record ends at text_bytes.
+ *   command      CK_CMD_CANONICALIZE: every record, '>' head '\n' canonical '\n' (src/canonicalize.rs:33-37);
+ *                CK_CMD_UNIQ: the first occurrences only, '>' head '\n' record.seq() '\n' (internal line breaks kept), or
+ *                the canonical form with CK_F_CANONICAL_BODY (src/uniq.rs:50-61).  The table is the context's, across
+ *                batches, as for ck_uniq_submit; base_index = input-order index of the batch's first record;
+ *                CK_CMD_MONOMERIZE: the written records, '>' head '\n' full_seq[.. monomer_len] '\n', with the rules and
+ *                options of ck_mono_submit (`mono`).
+ * Normalisation is always the CLI's (CK_F_NORMALIZE).  *out_n_records = records in the text (the next batch's base_index
+ * follows from it).  Refused before anything is left running on the slot: text_bytes > max_batch_bytes or more records than
+ * max_batch_records -> CK_ERR_ARG (the slot stays usable); a seq over 2^30 symbols (canonicalize / uniq) or over
+ * 2^32 - 1024 bytes (monomerize) -> CK_ERR_TOO_LONG; uniq on a context with table_capacity 0 or with a peer group attached
+ * -> CK_ERR_STATE.  The submit waits for its record count (a small copy after the split); the other slot keeps running.
+ * The first text batch of a slot allocates its text and framing buffers (about 2 max_batch_bytes + 2 max_batch_records).
+ *
+ * ck_fasta_wait: out_fasta (ck_fasta_out_bytes(text_bytes, n_records) bytes) receives exactly the bytes the CLI writes for
+ * this batch, *out_fasta_bytes of them; *out_n_written records, out_index[k] = position in the batch of written record k
+ * (increasing).  Per record of the batch: out_head[2 i], out_head[2 i + 1] = its head range [lo, hi) in the text;
+ * out_first_index (uniq, as ck_uniq_wait); out_full_len / out_monomer_len (monomerize, as ck_mono_wait).  Any out pointer
+ * may be NULL. */
+#define CK_CMD_CANONICALIZE 1
+#define CK_CMD_UNIQ 2
+#define CK_CMD_MONOMERIZE 3
+#define CK_F_CANONICAL_BODY 64u   /* uniq -c: write the canonical form, not record.seq() */
+uint64_t ck_fasta_out_bytes(uint64_t text_bytes, uint32_t n_records);   /* text_bytes + 2 n_records + 64 */
+int ck_fasta_submit(ck_ctx *ctx, int slot, const uint8_t *text, uint64_t text_bytes, uint32_t command, uint32_t flags,
+                    uint64_t base_index, const ck_mono_options *mono, uint32_t *out_n_records);
+int ck_fasta_wait(ck_ctx *ctx, int slot, uint8_t *out_fasta, uint64_t *out_fasta_bytes, uint32_t *out_n_written,
+                  uint32_t *out_index, uint64_t *out_head, uint64_t *out_first_index, uint32_t *out_full_len,
+                  uint32_t *out_monomer_len);
 /* number of kernels this context has launched so far (bench.py's gpu_launches) */
 uint64_t ck_launch_count(const ck_ctx *ctx);
 /* per-class kernel timing for the roofline: when enabled, every length/alphabet-class launch is bracketed

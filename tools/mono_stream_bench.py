@@ -1,10 +1,11 @@
-"""End-to-end measurement of `python -m circkit_b200 monomerize` on a FASTA file (one GPU).
+"""End-to-end measurement of `python -m circkit_b200 monomerize` (or canonicalize / uniq) on a FASTA file (one GPU).
 
-    python tools/mono_stream_bench.py --out DIR [--parent TREE] [--records 1000000] [--scale 4]
+    python tools/mono_stream_bench.py --out DIR [--command canonicalize|uniq|monomerize] [--parent TREE] [--records 1000000]
+                                      [--scale 4]
 
 Writes data of bench.py's `--workload mono` shape (1 M concatemers: 2.3 copies of a 250-400 nt unit, 1 % substitutions;
 bench.py's unit lengths and base hash, generated on the device in blocks) as FASTA with 70-column lines to a temporary
-directory, runs the CLI on it with seed 10 and min identity 0.95, and prints one JSON line per run: wall time, records/s, input MB/s and the child's peak RSS, with the card's name and
+directory, runs the CLI's --command on it (monomerize, the default: with seed 10 and min identity 0.95), and prints one JSON line per run: wall time, records/s, input MB/s and the child's peak RSS, with the card's name and
 power limit read in the same process.  --parent TREE: the CLI of another source tree (e.g. an exported copy of an earlier
 commit, built in place) runs on the same file and the two outputs are compared byte for byte.  --scale K: a second file K
 times as large goes through this tree's CLI only, to show whether peak RSS grows with the input.
@@ -65,9 +66,11 @@ def write_fasta(path: str, n: int, seed_offset: int = 0) -> int:
     return os.path.getsize(path)
 
 
-def run_cli(tree: str, src: str, dst: str) -> dict:
-    """one `python -m circkit_b200 monomerize` child in `tree`: wall time and peak RSS (its own rusage, from wait4)"""
-    cmd = [sys.executable, "-m", "circkit_b200", "monomerize", src, "-o", dst, "--seed-length", "10", "--min-identity", "0.95"]
+def run_cli(tree: str, command: str, src: str, dst: str) -> dict:
+    """one `python -m circkit_b200 COMMAND` child in `tree`: wall time and peak RSS (its own rusage, from wait4)"""
+    cmd = [sys.executable, "-m", "circkit_b200", command, src, "-o", dst]
+    if command == "monomerize":
+        cmd += ["--seed-length", "10", "--min-identity", "0.95"]
     env = dict(os.environ, PYTHONPATH=tree)
     t0 = time.perf_counter()
     p = subprocess.Popen(cmd, cwd=tree, env=env)
@@ -77,9 +80,9 @@ def run_cli(tree: str, src: str, dst: str) -> dict:
     return {"exit": p.returncode, "wall_s": wall, "peak_rss_mb": ru.ru_maxrss / 1024}
 
 
-def report(label: str, tree: str, src: str, n: int, size: int, dst: str) -> dict:
-    r = run_cli(tree, src, dst)
-    line = {"run": label, "tree": os.path.basename(os.path.abspath(tree)), "records": n, "input_mb": size / 1e6, **r,
+def report(label: str, tree: str, command: str, src: str, n: int, size: int, dst: str) -> dict:
+    r = run_cli(tree, command, src, dst)
+    line = {"run": label, "command": command, "tree": os.path.basename(os.path.abspath(tree)), "records": n, "input_mb": size / 1e6, **r,
             "records_per_s": n / r["wall_s"], "input_mb_per_s": size / 1e6 / r["wall_s"], **gpu_info()}
     print(json.dumps(line), flush=True)
     return line
@@ -88,6 +91,7 @@ def report(label: str, tree: str, src: str, n: int, size: int, dst: str) -> dict
 def main() -> int:
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--out", required=True, help="directory for the JSON lines")
+    ap.add_argument("--command", choices=["canonicalize", "uniq", "monomerize"], default="monomerize")
     ap.add_argument("--parent", help="source tree of the CLI to compare with (built in place)")
     ap.add_argument("--records", type=int, default=1_000_000)
     ap.add_argument("--scale", type=int, default=4)
@@ -102,9 +106,9 @@ def main() -> int:
     try:
         src = os.path.join(tmp, "mono_1x.fa")
         size = write_fasta(src, args.records)
-        lines = [report("new", ROOT, src, args.records, size, os.path.join(tmp, "new_1x.fa"))]
+        lines = [report("new", ROOT, args.command, src, args.records, size, os.path.join(tmp, "new_1x.fa"))]
         if args.parent:
-            lines.append(report("parent", args.parent, src, args.records, size, os.path.join(tmp, "parent_1x.fa")))
+            lines.append(report("parent", args.parent, args.command, src, args.records, size, os.path.join(tmp, "parent_1x.fa")))
             same = filecmp.cmp(os.path.join(tmp, "new_1x.fa"), os.path.join(tmp, "parent_1x.fa"), shallow=False)
             print(json.dumps({"outputs_identical": same}), flush=True)
             lines.append({"outputs_identical": same})
@@ -113,11 +117,12 @@ def main() -> int:
         if args.scale > 1:
             big = os.path.join(tmp, "mono_%dx.fa" % args.scale)
             bsize = write_fasta(big, args.records * args.scale)
-            lines.append(report("new_%dx" % args.scale, ROOT, big, args.records * args.scale, bsize,
+            lines.append(report("new_%dx" % args.scale, ROOT, args.command, big, args.records * args.scale, bsize,
                                 os.path.join(tmp, "new_%dx.fa" % args.scale)))
     finally:
         shutil.rmtree(tmp, ignore_errors=True)
-    with open(os.path.join(args.out, "mono_stream_bench.jsonl"), "w") as f:
+    name = "mono_stream_bench.jsonl" if args.command == "monomerize" else "mono_stream_bench_%s.jsonl" % args.command
+    with open(os.path.join(args.out, name), "w") as f:
         f.write("".join(json.dumps(x) + "\n" for x in lines))
     return 0 if all(x.get("exit", 0) == 0 for x in lines) and all(x.get("outputs_identical", True) for x in lines) else 1
 
