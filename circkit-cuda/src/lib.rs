@@ -93,6 +93,8 @@ pub mod ffi {
                                       out_compact_offsets: *mut u64, out_compact_bytes: *mut u8, out_len: *mut u32,
                                       out_hash64: *mut u64, out_first_index: *mut u64) -> c_int;
         pub fn ck_uniq_reset(ctx: *mut CkCtx) -> c_int;
+        pub fn ck_uniq_grow(ctx: *mut CkCtx, max_keys: u64) -> c_int;
+        pub fn ck_uniq_table_info(ctx: *mut CkCtx, out_keys: *mut u64, out_capacity_keys: *mut u64, out_grows: *mut u64) -> c_int;
         pub fn ck_pack2_words(total_bytes: u64, n_records: u32) -> u64;
         pub fn ck_pack2_host(bytes: *const u8, offsets: *const u64, n_records: u32, flags: u32, threads: u32,
                              packed2_dense: *mut u64, lens: *mut u32, lane: *mut u8, lane_bytes: *mut u8,
@@ -149,6 +151,17 @@ impl Context {
     /// Forget every key (a new input file).
     pub fn uniq_reset(&self) -> Result<()> {
         self.check(unsafe { ffi::ck_uniq_reset(self.raw) })
+    }
+    /// Let the uniq table grow on the device as distinct keys arrive, up to `max_keys` keys (None: as many as device
+    /// memory allows).  Not with a peer group.
+    pub fn uniq_grow(&self, max_keys: Option<u64>) -> Result<()> {
+        self.check(unsafe { ffi::ck_uniq_grow(self.raw, max_keys.unwrap_or(u64::MAX)) })
+    }
+    /// (distinct keys in the uniq table, keys it holds at 2/3 load, growths so far); synchronises both slots.
+    pub fn uniq_table_info(&self) -> Result<(u64, u64, u64)> {
+        let (mut keys, mut cap, mut grows) = (0u64, 0u64, 0u64);
+        self.check(unsafe { ffi::ck_uniq_table_info(self.raw, &mut keys, &mut cap, &mut grows) })?;
+        Ok((keys, cap, grows))
     }
     /// Multi-GPU uniq, step 1: this rank's exchange block as a CUDA IPC handle (send it to every rank).
     pub fn peer_export(&self, world: u32, rank: u32, max_records: u32) -> Result<[u8; ffi::CK_PEER_HANDLE_BYTES]> {
@@ -261,12 +274,16 @@ pub struct Pump {
 
 impl Pump {
     /// `threads` = the CLI's `--threads` (`src/commands.rs:122,147`): host packer threads (monomerize does not pack).
-    /// `table_capacity` = distinct canonical forms `uniq` may meet (ignored for canonicalize / monomerize).
+    /// `table_capacity` = the initial size of `uniq`'s table in distinct canonical forms; it grows on the device as they
+    /// arrive (ignored for canonicalize / monomerize).
     pub fn new(device: i32, mode: Mode, threads: u32, table_capacity: u64) -> Result<Self> {
         const MAX_BYTES: u64 = 256 << 20;
         const MAX_RECORDS: u32 = 1 << 20;
         let uniq = matches!(mode, Mode::Uniq { .. });
-        let ctx = Context::new(device, MAX_BYTES, MAX_RECORDS, if uniq { table_capacity } else { 0 })?;
+        let ctx = Context::new(device, MAX_BYTES, MAX_RECORDS, if uniq { table_capacity.max(1) } else { 0 })?;
+        if uniq {
+            ctx.uniq_grow(None)?;
+        }
         let mk = |ctx: &Context| -> Result<Batch> {
             let r = MAX_RECORDS as usize;
             let b = MAX_BYTES as usize;

@@ -55,6 +55,8 @@ SIGNATURES = {
     "ck_uniq_wait": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "ck_uniq_wait_survivors": (_i, [_vp, _i, C.POINTER(_u32), _vp, _vp, _vp, _vp, _vp, _vp]),
     "ck_uniq_reset": (_i, [_vp]),
+    "ck_uniq_grow": (_i, [_vp, _u64]),
+    "ck_uniq_table_info": (_i, [_vp, C.POINTER(_u64), C.POINTER(_u64), C.POINTER(_u64)]),
     "ck_peer_export": (_i, [_vp, _u32, _u32, _u32, _vp]),
     "ck_peer_attach": (_i, [_vp, _vp]),
     "ck_dev_peer_first_index": (_i, [_vp, _vp, _vp, _u32, _u64, _vp, _u64, _vp]),

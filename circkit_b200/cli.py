@@ -369,6 +369,8 @@ def _piece_text(piece) -> bytes:
 # ------------------------------------------------------------------------------------------------ GPU pump
 MAX_BATCH_BYTES = 256 << 20
 MAX_BATCH_RECORDS = 1 << 20
+# distinct records uniq's table holds when it is created (about 25 MB of device memory); it grows on the device as they arrive
+UNIQ_TABLE_KEYS = 1 << 20
 
 
 def _text_batches(text: bytes, max_bytes: int, max_records: int, oversize: bool = False):
@@ -402,6 +404,8 @@ class _Pump:
     def __init__(self, command: str, done, table_capacity: int = 0, oversize: bool = False, **submit_kw):
         self.command, self.done, self.oversize, self.kw = command, done, oversize, submit_kw
         self.ctx, self.big = _context(table_capacity), None
+        if command == "uniq":
+            self.ctx.uniq_grow()
         self.pinned = {}                                     # (slot, 0 in / 1 out) -> (pointer, uint8 array)
         self.pend, self.b, self.base = None, 0, 0
 
@@ -493,10 +497,13 @@ def _rec_id(text: bytes, lo: int, head: np.ndarray, i: int) -> bytes:
     return text[lo + int(head[i, 0]): lo + int(head[i, 1])].split(b" ", 1)[0]
 
 
-def run_uniq(pieces, write, canonical: bool = False, table_write=None, table_ext: str | None = None, table_capacity: int = 1 << 24,
-             threads: int = 0) -> None:
+def run_uniq(pieces, write, canonical: bool = False, table_write=None, table_ext: str | None = None,
+             table_capacity: int | None = None, threads: int = 0) -> None:
     """`circkit uniq` over a stream of pieces (src/uniq.rs:15-88): one first-occurrence table on the device for the whole
-    input, survivors written batch by batch in input order, duplicate rows to `table_write` as they are met."""
+    input, survivors written batch by batch in input order, duplicate rows to `table_write` as they are met.
+    `table_capacity`: the table's initial size in keys (default UNIQ_TABLE_KEYS); it grows as distinct records arrive."""
+    if table_capacity is None:
+        table_capacity = UNIQ_TABLE_KEYS
     first_ids = {}                                             # global index of a first occurrence -> its id (for --table only)
     delim = b"\t" if table_ext == "tsv" else b","
     state = {"header": False}
@@ -662,13 +669,7 @@ def main(argv=None) -> int:
             elif args.command == "monomerize":
                 run_monomerize(chain(), w.write, opts, tf.write if tf else None, ext)
             else:
-                cap = 1 << 24
-                if args.input is not None:
-                    # distinct canonical forms the table must hold: bounded by the record count, itself bounded by the input size
-                    # (a record needs >= 4 bytes; compressed DNA rarely beats 4x)
-                    sz = os.path.getsize(args.input)
-                    cap = max(1 << 16, min(1 << 30, sz if args.input.rsplit(".", 1)[-1] in ("gz", "bz2", "xz", "zst") else sz // 4))
-                run_uniq(chain(), w.write, args.canonicalize, tf.write if tf else None, ext, table_capacity=cap, threads=threads)
+                run_uniq(chain(), w.write, args.canonicalize, tf.write if tf else None, ext, threads=threads)
         finally:
             w.close()
             if tf is not None:

@@ -308,6 +308,17 @@ class Context:
     def uniq_reset(self):
         self._check(self._lib.ck_uniq_reset(self._h))
 
+    def uniq_grow(self, max_keys: Optional[int] = None):
+        """ck_uniq_grow: the uniq table grows on the device as distinct keys arrive, up to max_keys keys (None: as many as
+        device memory allows; 0: growth off)"""
+        self._check(self._lib.ck_uniq_grow(self._h, 2**64 - 1 if max_keys is None else max_keys))
+
+    def table_info(self) -> "tuple[int, int, int]":
+        """ck_uniq_table_info -> (distinct keys in the table, keys it holds at 2/3 load, growths so far)"""
+        keys, cap, grows = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
+        self._check(self._lib.ck_uniq_table_info(self._h, C.byref(keys), C.byref(cap), C.byref(grows)))
+        return int(keys.value), int(cap.value), int(grows.value)
+
 
 _default: Optional[Context] = None
 

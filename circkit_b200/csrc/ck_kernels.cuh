@@ -7,6 +7,7 @@
 //   k_canon_cta    CTA-per-record, same algorithm                        (plasmid / mtDNA sizes)
 //   k_table_insert first-occurrence table: CAS the key, atomicMin the input index
 //   k_table_first  read back first_index per record
+//   k_table_rehash move a context's table into a larger one (ck_uniq_grow)
 #pragma once
 #include "ck_hash.cuh"
 
@@ -653,6 +654,7 @@ struct TableArgs {
     u64 *slot_of;                        // out: slot found per record (for k_table_first)
     u64 *first_out;                      // out (k_table_first)
     u32 *overflow;                       // set if the table is full
+    u64 *keys;                           // optional: += keys this launch adds to the table (a context's table; ck_uniq_grow)
 };
 __global__ void __launch_bounds__(256) k_table_insert(TableArgs a)
 {
@@ -668,6 +670,10 @@ __global__ void __launch_bounds__(256) k_table_insert(TableArgs a)
         if (prev == CK_EMPTY_KEY || prev == key) {
             atomicMin(&a.slots[s].first, idx);
             a.slot_of[i] = s;
+            if (a.keys && prev == CK_EMPTY_KEY) {     // claimed a free slot: one add per group of lanes that got here together
+                const u32 m = __activemask();
+                if ((threadIdx.x & 31) == (u32)(__ffs(m) - 1)) atomicAdd(a.keys, (u64)__popc(m));
+            }
             return;
         }
         s = s + 1 == a.nslots ? 0 : s + 1;
@@ -687,6 +693,19 @@ __global__ void k_table_clear(TableSlot *slots, u64 n, u64 *side_first)
         slots[i].key = CK_EMPTY_KEY; slots[i].first = ~0ULL;
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) *side_first = ~0ULL;
+}
+// Growth of a context's table (ck_uniq_grow): every key of the old table moves to its home in the new one, with the same
+// probing.  Keys are unique, so each move claims a free slot and carries its minimum index over as it is; the new table
+// starts all ones (empty key, empty first) and is larger than the old one, so the probe always ends.
+__global__ void __launch_bounds__(256) k_table_rehash(const TableSlot *old, u64 old_slots, TableSlot *slots, u64 nslots)
+{
+    for (u64 i = blockIdx.x * (u64)blockDim.x + threadIdx.x; i < old_slots; i += (u64)gridDim.x * blockDim.x) {
+        const TableSlot e = old[i];
+        if (e.key == CK_EMPTY_KEY) continue;
+        u64 s = table_home(e.key, nslots);
+        while (atomicCAS(&slots[s].key, CK_EMPTY_KEY, e.key) != CK_EMPTY_KEY) s = s + 1 == nslots ? 0 : s + 1;
+        slots[s].first = e.first;
+    }
 }
 
 // ---------------------------------------------------------------------------------------------

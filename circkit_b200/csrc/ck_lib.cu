@@ -111,6 +111,7 @@ struct Slot {
     u64 longest = 0;                    // longest raw record of the batch in flight
     u32 *sel = nullptr; u64 *coff = nullptr;    // CK_F_SURVIVORS: survivor indices / compact offsets of the batch in flight
     u32 n = 0, flags = 0; u64 total = 0;
+    u64 rec_mark = 0;                   // uniq batch in flight: ck_ctx::submitted_rec once it was counted (0: not counted)
 };
 
 // Multi-GPU uniq through the C ABI: this rank's exchange block (exported by CUDA IPC) and every peer's, mapped here.
@@ -138,7 +139,14 @@ struct ck_ctx {
     cudaEvent_t last_insert = nullptr;  // insert event of the most recently submitted uniq batch
     bool have_last_insert = false;
     TableSlot *table = nullptr; u64 table_slots = 0; u64 *side = nullptr; u32 *d_overflow = nullptr;
-    PeerGroup peer;                     // world > 1 after ck_peer_attach: uniq runs the hash-range exchange
+    u64 *d_keys = nullptr;              // keys in `table` (k_table_insert counts its claims); 8 bytes after d_overflow, so one
+                                        // 16-byte copy brings both back to h_counts[16] / h_counts[18..19]
+    // ck_uniq_grow: grow_max = most keys the table may grow to hold (0: fixed size).  table_reserve bounds the keys in the table
+    // from above by known_keys (the device's count as collected with the batch that ended at known_rec uniq records) plus the
+    // uniq records submitted since (submitted_rec counts them all).
+    u64 grow_max = 0, grows = 0;
+    u64 known_keys = 0, known_rec = 0, submitted_rec = 0;
+    PeerGroup peer;                    // world > 1 after ck_peer_attach: uniq runs the hash-range exchange
     // library drop-ins (ck_lmsr_index / ck_lmsr / ck_canonicalize): persistent staging + stream, one call at a time per
     // context (any number of host threads may call; lib/src/canonicalize.rs:54 is called from T worker threads)
     std::mutex lib_mu;
@@ -519,10 +527,10 @@ u32 extend_grid(const ck_ctx *ctx, u32 n_records) { return std::max(1u, std::min
 u64 table_slots_for(u64 keys) { return std::max<u64>(1024, keys + keys / 2 + 16); }
 
 int table_insert(ck_ctx *ctx, cudaStream_t st, TableSlot *slots, u64 nslots, u64 *side, u32 *overflow,
-                 const u64 *hash, const u64 *index, u64 base, u32 n, u64 *slot_of, u32 stride = 1)
+                 const u64 *hash, const u64 *index, u64 base, u32 n, u64 *slot_of, u32 stride = 1, u64 *keys = nullptr)
 {
     if (!n) return CK_OK;
-    TableArgs t{slots, nslots, side, hash, index, stride, base, n, slot_of, nullptr, overflow};
+    TableArgs t{slots, nslots, side, hash, index, stride, base, n, slot_of, nullptr, overflow, keys};
     k_table_insert<<<(n + 255) / 256, 256, 0, st>>>(t);
     ctx->launches++;
     CK_CUDA(ctx, cudaGetLastError());
@@ -536,6 +544,67 @@ int table_first(ck_ctx *ctx, cudaStream_t st, TableSlot *slots, u64 nslots, u64 
     ctx->launches++;
     CK_CUDA(ctx, cudaGetLastError());
     return CK_OK;
+}
+
+// keys a table of `slots` slots holds at load <= 2/3
+u64 table_capacity_keys(u64 slots) { return slots * 2 / 3; }
+
+// Growth (ck_uniq_grow): a table of `slots` slots, the context's keys rehashed into it on `st`, the old table freed.  The
+// caller has synchronised both slot streams: no insert or k_table_first of an earlier batch still refers to the old table.
+int table_grow(ck_ctx *ctx, cudaStream_t st, u64 slots)
+{
+    TableSlot *t = nullptr;
+    cudaError_t e = cudaMalloc(&t, slots * sizeof(TableSlot));
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ctx, CK_ERR_TABLE_FULL, "uniq table cannot grow: its new size cannot be allocated", e);
+    }
+    e = cudaMemsetAsync(t, 0xff, slots * sizeof(TableSlot), st);   // empty key and empty first are both all ones
+    if (e == cudaSuccess) {
+        const u64 grid = std::min<u64>((ctx->table_slots + 255) / 256, 32ull * (u64)ctx->num_sms);
+        k_table_rehash<<<(u32)grid, 256, 0, st>>>(ctx->table, ctx->table_slots, t, slots);
+        ctx->launches++;
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) { cudaFree(t); return fail(ctx, CK_ERR_CUDA, "uniq table growth", e); }
+    cudaFree(ctx->table);
+    ctx->table = t; ctx->table_slots = slots; ctx->grows++;
+    return CK_OK;
+}
+
+// Every uniq batch of n records calls this before it enqueues anything (not in a peer group).  With growth on, the table is
+// grown here whenever the batch could take it past 2/3 load: the host's bound on the keys decides when to look, the device's
+// exact count whether to grow.  The new size leaves room for twice the keys and two more batches of this size, so growths
+// are O(log keys) and a stream of duplicates near the bound does not synchronise on every batch.  A refused batch leaves the
+// table as it was.
+int table_reserve(ck_ctx *ctx, Slot &s, u64 n)
+{
+    const u64 cap = table_capacity_keys(ctx->table_slots);
+    if (ctx->grow_max && ctx->known_keys + (ctx->submitted_rec - ctx->known_rec) + n > cap) {
+        // the other slot's insert and k_table_first (its slot indices point into this table) finish first
+        for (Slot &o : ctx->slot) if (o.stream) CK_CUDA(ctx, cudaStreamSynchronize(o.stream));
+        u64 exact = 0;
+        CK_CUDA(ctx, cudaMemcpy(&exact, ctx->d_keys, 8, cudaMemcpyDeviceToHost));
+        ctx->known_keys = exact; ctx->known_rec = ctx->submitted_rec;
+        const u64 need = exact + n;
+        if (need > cap) {
+            if (need > ctx->grow_max) return fail(ctx, CK_ERR_TABLE_FULL, "uniq batch would take the table past max_keys");
+            const int rc = table_grow(ctx, s.stream, table_slots_for(std::min(ctx->grow_max, 2 * need + 2 * n)));
+            if (rc) return rc;
+        }
+    }
+    ctx->submitted_rec += n;
+    s.rec_mark = ctx->submitted_rec;
+    return CK_OK;
+}
+
+// a collected uniq batch brings the device's key count as of its table_first back in h_counts[18..19]
+void note_keys(ck_ctx *ctx, const Slot &s)
+{
+    if (s.rec_mark <= ctx->known_rec) return;     // an older count than the one known (or the batch was not counted)
+    memcpy(&ctx->known_keys, s.h_counts + 18, 8);
+    ctx->known_rec = s.rec_mark;
 }
 
 // The hash-range exchange of multi-GPU uniq, fused into the kernels around it (SURVEY 8e; replaces the single `seen` map of
@@ -611,7 +680,7 @@ int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_reco
     if (n_records && (!offsets || (!have_bytes && offsets[n_records] != offsets[0])))
         return fail(ctx, CK_ERR_ARG, "null batch pointers");
     if (uniq && !ctx->table) return fail(ctx, CK_ERR_STATE, "context was created with table_capacity 0");
-    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.text = false; s.total = 0;
+    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.text = false; s.total = 0; s.rec_mark = 0;
     if (n_records == 0) return CK_OK;
     if (offsets[0] != 0) return fail(ctx, CK_ERR_ARG, "offsets[0] must be 0");
     const u64 total = offsets[n_records];
@@ -762,7 +831,7 @@ int submit_tail(ck_ctx *ctx, Slot &s, bool lens_given, uint64_t base_index)
         CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 16, ctx->d_overflow, 4, cudaMemcpyDeviceToHost, st));
     } else if (s.uniq) {
         rc = table_insert(ctx, st, ctx->table, ctx->table_slots, ctx->side, ctx->d_overflow, s.d_hash, nullptr,
-                          base_index, n_records, s.d_slotof);
+                          base_index, n_records, s.d_slotof, 1, ctx->d_keys);
         if (rc) return rc;
         CK_CUDA(ctx, cudaEventRecord(s.inserted, st));
         // first_index of this batch may point into the previous batch: wait for that batch's insert
@@ -770,7 +839,7 @@ int submit_tail(ck_ctx *ctx, Slot &s, bool lens_given, uint64_t base_index)
         ctx->last_insert = s.inserted; ctx->have_last_insert = true;
         rc = table_first(ctx, st, ctx->table, ctx->table_slots, ctx->side, s.d_slotof, n_records, s.d_first);
         if (rc) return rc;
-        CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 16, ctx->d_overflow, 4, cudaMemcpyDeviceToHost, st));
+        CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts + 16, ctx->d_overflow, 16, cudaMemcpyDeviceToHost, st));   // + d_keys
     }
     CK_CUDA(ctx, cudaMemcpyAsync(s.h_counts, s.d_counts, 16 * 4, cudaMemcpyDeviceToHost, st));
     if (s.uniq && (flags & CK_F_SURVIVORS)) {
@@ -820,6 +889,7 @@ int submit_common(ck_ctx *ctx, int slot, const uint8_t *bytes, const uint64_t *o
     const u64 total = s.total;
     cudaStream_t st = s.stream;
     CK_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (uniq && !ctx->peer.attached && (rc = table_reserve(ctx, s, n_records))) return rc;
     CK_CUDA(ctx, cudaMemcpyAsync(s.d_off, offsets, (size_t)(n_records + 1) * 8, cudaMemcpyHostToDevice, st));
     if (total) CK_CUDA(ctx, cudaMemcpyAsync(s.d_raw, bytes, total, cudaMemcpyHostToDevice, st));
     return enqueue_canon(ctx, s, base_index);
@@ -841,6 +911,7 @@ int submit_packed(ck_ctx *ctx, int slot, const ck_packed_batch *b, uint32_t flag
     if (b->lane_bytes_total > ctx->cfg.max_batch_bytes) return fail(ctx, CK_ERR_ARG, "lane_bytes exceed max_batch_bytes");
     cudaStream_t st = s.stream;
     CK_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (uniq && !ctx->peer.attached && (rc = table_reserve(ctx, s, n_records))) return rc;
     CK_CUDA(ctx, cudaMemcpyAsync(s.d_off, b->offsets, (size_t)(n_records + 1) * 8, cudaMemcpyHostToDevice, st));
     CK_CUDA(ctx, cudaMemcpyAsync(s.d_len, b->lens, (size_t)n_records * 4, cudaMemcpyHostToDevice, st));
     CK_CUDA(ctx, cudaMemcpyAsync(s.d_lane, b->lane, (size_t)n_records, cudaMemcpyHostToDevice, st));
@@ -879,6 +950,7 @@ int wait_common(ck_ctx *ctx, int slot, bool uniq, uint8_t *out_bytes, uint32_t *
     if (out_hash) CK_CUDA(ctx, cudaMemcpyAsync(out_hash, s.d_hash, n * 8, cudaMemcpyDeviceToHost, st));
     if (out_first && uniq) CK_CUDA(ctx, cudaMemcpyAsync(out_first, s.d_first, n * 8, cudaMemcpyDeviceToHost, st));
     CK_CUDA(ctx, cudaStreamSynchronize(st));
+    if (uniq) note_keys(ctx, s);
     if (s.h_counts[CLS_HUGE]) return fail(ctx, CK_ERR_TOO_LONG, "batch holds a record beyond the staged-length classes");
     if (uniq && s.h_counts[16]) return fail(ctx, CK_ERR_TABLE_FULL, "uniq table is full; raise table_capacity");
     return CK_OK;
@@ -964,8 +1036,9 @@ int ck_init(const ck_config *cfg, ck_ctx **out)
         }
     }
     CK_INIT(cudaMalloc(&ctx->side, 8));
-    CK_INIT(cudaMalloc(&ctx->d_overflow, 4));
-    CK_INIT(cudaMemset(ctx->d_overflow, 0, 4));
+    CK_INIT(cudaMalloc(&ctx->d_overflow, 16));
+    CK_INIT(cudaMemset(ctx->d_overflow, 0, 16));
+    ctx->d_keys = reinterpret_cast<u64 *>(ctx->d_overflow + 2);
     if (cfg->table_capacity) {
         ctx->table_slots = table_slots_for(cfg->table_capacity);
         CK_INIT(cudaMalloc(&ctx->table, ctx->table_slots * sizeof(TableSlot)));
@@ -1054,6 +1127,7 @@ int ck_peer_export(ck_ctx *ctx, uint32_t world, uint32_t rank, uint32_t max_reco
         return ctx ? fail(ctx, CK_ERR_ARG, "bad peer group arguments") : CK_ERR_ARG;
     PeerGroup &P = ctx->peer;
     if (P.exported) return fail(ctx, CK_ERR_STATE, "peer block already exported");
+    if (ctx->grow_max) return fail(ctx, CK_ERR_STATE, "a context whose uniq table grows (ck_uniq_grow) cannot join a peer group");
     CK_CUDA(ctx, cudaSetDevice(ctx->device));
     P.world = world; P.rank = rank; P.cap = max_records;
     P.recv_bytes = ((u64)world * P.cap * 16 + 255) & ~255ull;
@@ -1116,6 +1190,7 @@ int ck_uniq_wait_survivors(ck_ctx *ctx, int slot, uint32_t *out_n_survivors, uin
     if (out_first_index) CK_CUDA(ctx, cudaMemcpyAsync(out_first_index, s.d_first, n * 8, cudaMemcpyDeviceToHost, st));
     CK_CUDA(ctx, cudaStreamSynchronize(st));
     s.busy = false;
+    note_keys(ctx, s);
     if (s.h_counts[CLS_HUGE]) return fail(ctx, CK_ERR_TOO_LONG, "batch holds a record beyond the staged-length classes");
     if (s.h_counts[16]) return fail(ctx, CK_ERR_TABLE_FULL, "uniq table is full; raise table_capacity");
     // ... then what the survivors need, sized by their number
@@ -1141,9 +1216,34 @@ int ck_uniq_reset(ck_ctx *ctx)
     CK_CUDA(ctx, cudaDeviceSynchronize());
     k_table_clear<<<ctx->num_sms * 4, 256>>>(ctx->table, ctx->table_slots, ctx->side);
     ctx->launches++;
-    CK_CUDA(ctx, cudaMemset(ctx->d_overflow, 0, 4));
+    CK_CUDA(ctx, cudaMemset(ctx->d_overflow, 0, 16));   // and d_keys
     CK_CUDA(ctx, cudaDeviceSynchronize());
     ctx->have_last_insert = false;
+    ctx->known_keys = 0; ctx->known_rec = ctx->submitted_rec;
+    return CK_OK;
+}
+
+int ck_uniq_grow(ck_ctx *ctx, uint64_t max_keys)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (!ctx->table) return fail(ctx, CK_ERR_STATE, "context was created with table_capacity 0");
+    if (ctx->peer.exported) return fail(ctx, CK_ERR_STATE, "the tables of a peer group do not grow");
+    ctx->grow_max = max_keys;
+    return CK_OK;
+}
+
+int ck_uniq_table_info(ck_ctx *ctx, uint64_t *out_keys, uint64_t *out_capacity_keys, uint64_t *out_grows)
+{
+    if (!ctx) return CK_ERR_ARG;
+    u64 keys = 0;
+    if (ctx->table) {
+        CK_CUDA(ctx, cudaSetDevice(ctx->device));
+        for (Slot &o : ctx->slot) if (o.stream) CK_CUDA(ctx, cudaStreamSynchronize(o.stream));
+        CK_CUDA(ctx, cudaMemcpy(&keys, ctx->d_keys, 8, cudaMemcpyDeviceToHost));
+    }
+    if (out_keys) *out_keys = keys;
+    if (out_capacity_keys) *out_capacity_keys = table_capacity_keys(ctx->table_slots);
+    if (out_grows) *out_grows = ctx->grows;
     return CK_OK;
 }
 
@@ -1303,6 +1403,8 @@ int ck_fasta_submit(ck_ctx *ctx, int slot, const uint8_t *text, uint64_t text_by
     if (is_mono && longest > kMonoMaxRecord) return fail(ctx, CK_ERR_TOO_LONG, "record longer than 2^32 - 1024 bytes");
     if (!is_mono && longest > (1ull << 30)) return fail(ctx, CK_ERR_TOO_LONG, "record longer than 2^30 symbols");
     s.n = n; s.longest = longest; s.dbl = longest > 512 ? 1u : 0u;   // as submit_check
+    s.rec_mark = 0;
+    if (uniq && (rc = table_reserve(ctx, s, n))) return rc;
     Compaction c;
     if ((rc = compaction_carve(ctx, s, c))) return rc;
     // the arena of the seq bytes, as the host-buffer entries receive it
@@ -1349,6 +1451,7 @@ int ck_fasta_wait(ck_ctx *ctx, int slot, uint8_t *out_fasta, uint64_t *out_fasta
     if (out_full_len && s.mono) CK_CUDA(ctx, cudaMemcpyAsync(out_full_len, s.d_slotof, n * 4, cudaMemcpyDeviceToHost, st));
     if (out_monomer_len && s.mono) CK_CUDA(ctx, cudaMemcpyAsync(out_monomer_len, s.d_hash, n * 4, cudaMemcpyDeviceToHost, st));
     CK_CUDA(ctx, cudaStreamSynchronize(st));
+    if (s.uniq) note_keys(ctx, s);
     if (!s.mono && s.h_counts[CLS_HUGE]) return fail(ctx, CK_ERR_TOO_LONG, "batch holds a record beyond the staged-length classes");
     if (s.uniq && s.h_counts[16]) return fail(ctx, CK_ERR_TABLE_FULL, "uniq table is full; raise table_capacity");
     const u32 nw = s.h_counts[20];

@@ -62,7 +62,8 @@ typedef struct ck_config {
     int32_t device;            /* CUDA device ordinal */
     uint64_t max_batch_bytes;  /* largest `bytes` a batch may carry (staging is sized once) */
     uint32_t max_batch_records;
-    uint64_t table_capacity;   /* distinct canonical forms the uniq table must hold (0: uniq unused) */
+    uint64_t table_capacity;   /* distinct canonical forms the uniq table holds (0: uniq unused); with ck_uniq_grow, the
+                                  initial size */
 } ck_config;
 
 /* ---- context ------------------------------------------------------------------------------- */
@@ -98,7 +99,21 @@ int ck_uniq_wait(ck_ctx *ctx, int slot, uint8_t *out_bytes, uint32_t *out_len, u
  * Size out_index for n_records entries, out_compact_offsets for n_records + 1 and out_compact_bytes for offsets[n] + 16 n_records. */
 int ck_uniq_wait_survivors(ck_ctx *ctx, int slot, uint32_t *out_n_survivors, uint32_t *out_index, uint64_t *out_compact_offsets,
                            uint8_t *out_compact_bytes, uint32_t *out_len, uint64_t *out_hash64, uint64_t *out_first_index);
-int ck_uniq_reset(ck_ctx *ctx);   /* forget every key (new input file) */
+int ck_uniq_reset(ck_ctx *ctx);   /* forget every key (new input file); a grown table keeps its size */
+/* Let the context's first-occurrence table grow as distinct keys arrive: before a uniq batch is enqueued, the table is
+ * enlarged (rehashed on the device) whenever the batch could push it past 2/3 load.  max_keys bounds the distinct keys it
+ * may hold (UINT64_MAX: as many as device memory allows); 0 turns growth off (the default).  A batch that would need more
+ * than max_keys, or whose growth cannot be allocated, is refused by its submit with CK_ERR_TABLE_FULL before anything is
+ * enqueued: the table and its contents are unchanged, the slot stays usable.  Not with a peer group (CK_ERR_STATE, either
+ * order); needs a context created with table_capacity >= 1.
+ * The submit looks at the device's key count only when a host-side bound (the count collected with the last waited batch
+ * plus the records submitted since) could pass 2/3 load; it then synchronises both slots, and grows when the exact count
+ * plus the batch needs it, to twice the keys plus two batches.  A growth holds the old and the new table (16 bytes per
+ * slot, 1.5 slots per key) for the time of the rehash. */
+int ck_uniq_grow(ck_ctx *ctx, uint64_t max_keys);
+/* distinct keys in the table (exact; synchronises both slots), the keys it can hold at 2/3 load, and how many times it has
+ * grown; any output may be NULL */
+int ck_uniq_table_info(ck_ctx *ctx, uint64_t *out_keys, uint64_t *out_capacity_keys, uint64_t *out_grows);
 
 /* ---- packed host input: 2 bits per base over PCIe instead of 8 -----------------------------------
  * The host side the reference keeps (FASTA reader threads, src/uniq.rs:29-41) packs while it parses: ck_pack2_host applies
