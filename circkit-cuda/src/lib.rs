@@ -75,6 +75,9 @@ pub mod ffi {
     pub const CK_CMD_UNIQ: u32 = 2;
     pub const CK_CMD_MONOMERIZE: u32 = 3;
     pub const CK_F_CANONICAL_BODY: u32 = 64;
+    /// ck_deflate_submit: largest input of one call, largest dictionary
+    pub const CK_DEFLATE_MAX_BYTES: u64 = 64 << 20;
+    pub const CK_DEFLATE_DICT_BYTES: u32 = 32768;
     extern "C" {
         pub fn ck_init(cfg: *const CkConfig, out: *mut *mut CkCtx) -> c_int;
         pub fn ck_destroy(ctx: *mut CkCtx);
@@ -114,6 +117,10 @@ pub mod ffi {
         pub fn ck_fasta_wait(ctx: *mut CkCtx, slot: c_int, out_fasta: *mut u8, out_fasta_bytes: *mut u64, out_n_written: *mut u32,
                              out_index: *mut u32, out_head: *mut u64, out_first_index: *mut u64, out_full_len: *mut u32,
                              out_monomer_len: *mut u32) -> c_int;
+        pub fn ck_deflate_bound(n: u64) -> u64;
+        pub fn ck_deflate_submit(ctx: *mut CkCtx, slot: c_int, bytes: *const u8, n: u64, dict: *const u8, dict_bytes: u32,
+                                 crc_in: u32) -> c_int;
+        pub fn ck_deflate_wait(ctx: *mut CkCtx, slot: c_int, out: *mut u8, out_bytes: *mut u64, crc_out: *mut u32) -> c_int;
         pub fn ck_peer_export(ctx: *mut CkCtx, world: u32, rank: u32, max_records: u32, handle_out: *mut c_void) -> c_int;
         pub fn ck_peer_attach(ctx: *mut CkCtx, all_handles: *const c_void) -> c_int;
         pub fn ck_lmsr_index(ctx: *mut CkCtx, s: *const u8, n: usize, out_index: *mut usize) -> c_int;

@@ -15,6 +15,7 @@ CK_PEER_HANDLE_BYTES = 64
 CK_MONO_SENSITIVE, CK_MONO_FIRST_ONLY, CK_MONO_KEEP_ALL, CK_MONO_NONE = 1, 2, 4, 0xFFFFFFFF
 CK_CMD_CANONICALIZE, CK_CMD_UNIQ, CK_CMD_MONOMERIZE = 1, 2, 3
 CK_F_CANONICAL_BODY = 64
+CK_DEFLATE_MAX_BYTES, CK_DEFLATE_DICT_BYTES = 64 << 20, 32768
 CK_CLASS_2BIT_LE_512, CK_CLASS_2BIT_LE_2048, CK_CLASS_2BIT_LE_65536, CK_CLASS_2BIT_LE_425984 = 1, 2, 4, 8
 CK_CLASS_2BIT_LE_4096, CK_CLASS_2BIT_LE_8192 = 1 << 10, 1 << 11
 
@@ -90,6 +91,9 @@ SIGNATURES = {
     "ck_fasta_out_bytes": (_u64, [_u64, _u32]),
     "ck_fasta_submit": (_i, [_vp, _i, _vp, _u64, _u32, _u32, _u64, C.POINTER(CkMonoOptions), C.POINTER(_u32)]),
     "ck_fasta_wait": (_i, [_vp, _i, _vp, C.POINTER(_u64), C.POINTER(_u32), _vp, _vp, _vp, _vp, _vp]),
+    "ck_deflate_bound": (_u64, [_u64]),
+    "ck_deflate_submit": (_i, [_vp, _i, _vp, _u64, _vp, _u32, _u32]),
+    "ck_deflate_wait": (_i, [_vp, _i, _vp, C.POINTER(_u64), C.POINTER(_u32)]),
     "ck_launch_count": (_u64, [_vp]),
     "ck_kernel_timing": (_i, [_vp, _i]),
     "ck_kernel_times": (_i, [_vp, _vp, _vp, _u32]),

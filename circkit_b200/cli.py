@@ -26,10 +26,12 @@ import ctypes.util
 import gzip
 import lzma
 import os
+import struct
 import sys
 
 import numpy as np
 
+from . import _native as N
 from .core import Context
 
 
@@ -289,16 +291,75 @@ def iter_input(path: str | None, chunk_bytes: int = CHUNK_BYTES):
             f.close()
 
 
-class Writer:
-    """src/utils.rs:29-72 as a stream: stdout, or a file compressed by its suffix (gz 6, bz2 9, xz 6, zst 1; else plain)"""
+def _suffix(path: str | None) -> str:
+    return path.rsplit(".", 1)[-1] if path is not None and "." in os.path.basename(path) else ""
 
-    def __init__(self, path: str | None):
-        self.path, self.zst = path, None
+
+# one gzip member (RFC 1952) with no name, mtime 0 and OS unknown, so that the same output gives the same file
+GZIP_HEADER = b"\x1f\x8b\x08\x00\x00\x00\x00\x00\x00\xff"
+
+
+class DeviceDeflate:
+    """Raw DEFLATE on the GPU for Writer's gzip output (ck_deflate_submit / ck_deflate_wait): deflate(data, dict, crc) ->
+    (fragment, crc) compresses up to max_bytes bytes after `dict` (the <= 32 KiB before them) into blocks that end with a
+    sync flush (00 00 ff ff), and continues the CRC-32.  The context (no batch staging, so the pump's slots are untouched)
+    and the pinned buffers are created by the first call."""
+
+    max_bytes = N.CK_DEFLATE_MAX_BYTES
+
+    def __init__(self, device: int = 0):
+        self.device, self.ctx, self.pinned = device, None, {}
+
+    def _buf(self, which: int, size: int) -> np.ndarray:
+        p = self.pinned.get(which)
+        if p is None or len(p[1]) < size:
+            if p is not None:
+                self.ctx._lib.ck_free_pinned(self.ctx.handle, p[0])
+            size = (size + (16 << 20) - 1) & ~((16 << 20) - 1)
+            ptr = self.ctx._lib.ck_alloc_pinned(self.ctx.handle, size)
+            if not ptr:
+                raise MemoryError("cannot allocate %d bytes of pinned host memory" % size)
+            p = (ptr, np.ctypeslib.as_array((ctypes.c_uint8 * size).from_address(ptr)))
+            self.pinned[which] = p
+        return p[1]
+
+    def deflate(self, data, dict: bytes, crc: int) -> "tuple[bytes, int]":
+        if self.ctx is None:
+            self.ctx = Context(self.device, max_batch_bytes=0, max_batch_records=0)
+        n = len(data)
+        src = self._buf(0, n)[:n]
+        src[:] = np.frombuffer(data, dtype=np.uint8)
+        out = self._buf(1, self.ctx.deflate_bound(n))
+        self.ctx.deflate_submit(0, src, dict, crc)
+        return self.ctx.deflate_wait(0, out)
+
+    def close(self):
+        if self.ctx is not None:
+            for p, _ in self.pinned.values():
+                self.ctx._lib.ck_free_pinned(self.ctx.handle, p)
+            self.pinned = {}
+            self.ctx.close()
+            self.ctx = None
+
+
+class Writer:
+    """src/utils.rs:29-72 as a stream: stdout, or a file compressed by its suffix (gz 6, bz2 9, xz 6, zst 1; else plain).
+    gzip_encoder (gz only; e.g. DeviceDeflate()): an object with max_bytes, deflate(data, dict, crc) -> (raw deflate
+    fragment ending in a sync flush, crc) and close().  Writer then frames the gzip member itself: GZIP_HEADER, one
+    fragment per call of at most max_bytes bytes, each given the last 32 KiB written before it as its dictionary, and at
+    close the final empty block (03 00), the CRC-32 and ISIZE.  Without it, gz goes through gzip.GzipFile at level 6."""
+
+    def __init__(self, path: str | None, gzip_encoder=None):
+        self.path, self.zst, self.gz = path, None, None
         if path is None:
             self.f = sys.stdout.buffer
             return
-        ext = path.rsplit(".", 1)[-1] if "." in os.path.basename(path) else ""
-        if ext == "gz":
+        ext = _suffix(path)
+        if ext == "gz" and gzip_encoder is not None:
+            self.f, self.gz = open(path, "wb"), gzip_encoder
+            self.crc, self.size, self.tail = 0, 0, b""
+            self.f.write(GZIP_HEADER)
+        elif ext == "gz":
             self.f = gzip.GzipFile(path, "wb", compresslevel=6)
         elif ext == "bz2":
             self.f = bz2.BZ2File(path, "wb", compresslevel=9)
@@ -312,7 +373,15 @@ class Writer:
     def write(self, data: bytes):
         if not data:
             return
-        if self.zst is not None:
+        if self.gz is not None:
+            mv = memoryview(data).cast("B")
+            for lo in range(0, len(mv), self.gz.max_bytes):
+                piece = mv[lo:lo + self.gz.max_bytes]
+                frag, self.crc = self.gz.deflate(piece, self.tail, self.crc)
+                self.f.write(frag)
+                self.size += len(piece)
+                self.tail = (self.tail + piece[-32768:].tobytes())[-32768:]
+        elif self.zst is not None:
             self.f.write(_zstd_compress(data, 1))             # concatenated frames are one valid zstd stream
         else:
             self.f.write(data)
@@ -320,8 +389,16 @@ class Writer:
     def close(self):
         if self.path is None:
             self.f.flush()
-        else:
-            self.f.close()
+            return
+        try:
+            if self.gz is not None:                          # final empty fixed block, CRC-32, ISIZE (RFC 1952)
+                self.f.write(b"\x03\x00" + struct.pack("<II", self.crc, self.size & 0xFFFFFFFF))
+        finally:
+            try:
+                if self.gz is not None:
+                    self.gz.close()
+            finally:
+                self.f.close()
 
 
 def iter_text(chunks):
@@ -657,7 +734,7 @@ def main(argv=None) -> int:
             if first is not None:
                 yield first
             yield from pieces
-        w = Writer(args.output)
+        w = Writer(args.output, gzip_encoder=DeviceDeflate() if _suffix(args.output) == "gz" else None)
         tf = None
         try:
             ext = None

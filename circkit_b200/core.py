@@ -82,6 +82,7 @@ class Context:
         self.max_batch_bytes = max_batch_bytes
         self.max_batch_records = max_batch_records
         self._text_batch = {}           # slot -> (records, text bytes) of its text batch in flight
+        self._deflate_batch = {}        # slot -> (input bytes, input, dict) of its deflate call in flight
 
     # -- plumbing
     @property
@@ -283,6 +284,35 @@ class Context:
         k = int(nw.value)
         return dict(fasta=out[:int(nbytes.value)].tobytes(), n_written=k, index=index[:k], head=head[:n], first=first[:n],
                     full_len=full_len[:n], monomer_len=mono_len[:n])
+
+    # -- DEFLATE on the device (ck_deflate_submit / ck_deflate_wait): raw, sync-flushed fragments of one deflate stream
+    def deflate_bound(self, n: int) -> int:
+        return int(self._lib.ck_deflate_bound(n))
+
+    def deflate_submit(self, slot: int, data, dict=b"", crc: int = 0):
+        """ck_deflate_submit: `data` (bytes-like or a uint8 array, e.g. pinned; 1 .. CK_DEFLATE_MAX_BYTES bytes) after `dict`
+        (<= 32 KiB: the bytes that came before it in the stream); crc = the CRC-32 of everything before `data`"""
+        a = data if isinstance(data, np.ndarray) else np.frombuffer(data, dtype=np.uint8)
+        d = dict if isinstance(dict, np.ndarray) else np.frombuffer(dict, dtype=np.uint8)
+        self._check(self._lib.ck_deflate_submit(self._h, slot, a.ctypes.data if len(a) else None, len(a),
+                                                d.ctypes.data if len(d) else None, len(d), crc & 0xFFFFFFFF))
+        self._deflate_batch[slot] = (len(a), a, d)      # pinned inputs must outlive the copy
+
+    def deflate_wait(self, slot: int, out: "np.ndarray | None" = None) -> "tuple[bytes, int]":
+        """ck_deflate_wait -> (raw deflate bytes ending in 00 00 ff ff, CRC-32 continued from the submit's crc).
+        `out`: optional uint8 buffer (pinned, for speed) of at least deflate_bound(n) bytes."""
+        n = self._deflate_batch.pop(slot, (0, None, None))[0]
+        need = self.deflate_bound(n)
+        if out is None or len(out) < need:
+            out = np.empty(need, dtype=np.uint8)
+        nbytes, crc = C.c_uint64(0), C.c_uint32(0)
+        self._check(self._lib.ck_deflate_wait(self._h, slot, out.ctypes.data, C.byref(nbytes), C.byref(crc)))
+        return out[:int(nbytes.value)].tobytes(), int(crc.value)
+
+    def deflate(self, data, dict=b"", crc: int = 0) -> "tuple[bytes, int]":
+        """deflate_submit + deflate_wait on slot 0"""
+        self.deflate_submit(0, data, dict, crc)
+        return self.deflate_wait(0)
 
     def uniq_batch(self, arena: np.ndarray, offsets: np.ndarray, base_index: int = 0, *, normalize: bool = False,
                    want_bytes=True, aligned=False):

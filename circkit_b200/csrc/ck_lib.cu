@@ -25,6 +25,7 @@
 #include "ck_synth.cuh"
 #include "ck_monomerize.cuh"
 #include "ck_fasta.cuh"
+#include "ck_deflate.cuh"
 
 using namespace ck;
 
@@ -112,6 +113,20 @@ struct Slot {
     u32 *sel = nullptr; u64 *coff = nullptr;    // CK_F_SURVIVORS: survivor indices / compact offsets of the batch in flight
     u32 n = 0, flags = 0; u64 total = 0;
     u64 rec_mark = 0;                   // uniq batch in flight: ck_ctx::submitted_rec once it was counted (0: not counted)
+    bool defl = false;                  // ck_deflate_submit's call (ck_deflate_wait collects it)
+    // ck_deflate_*: own stream and buffers, allocated by the slot's first deflate call and grown to the largest since
+    struct Deflate {
+        cudaStream_t stream = nullptr;
+        u64 cap = 0;                    // input bytes the buffers hold
+        u8 *buf = nullptr;              // dict || input
+        u32 *kA = nullptr, *kB = nullptr, *vA = nullptr, *vB = nullptr;   // sort buffers; then match table / tokens
+        u32 *prev8 = nullptr, *prev4 = nullptr;
+        u32 *seg = nullptr;             // per segment: freq, table, header, meta, CRC, token count, offset
+        u32 *out = nullptr, *result = nullptr;
+        u32 *h_result = nullptr;        // pinned
+        void *tmp = nullptr; size_t tmp_bytes = 0;
+        u64 n = 0;
+    } z;
 };
 
 // Multi-GPU uniq through the C ABI: this rank's exchange block (exported by CUDA IPC) and every peer's, mapped here.
@@ -680,7 +695,7 @@ int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_reco
     if (n_records && (!offsets || (!have_bytes && offsets[n_records] != offsets[0])))
         return fail(ctx, CK_ERR_ARG, "null batch pointers");
     if (uniq && !ctx->table) return fail(ctx, CK_ERR_STATE, "context was created with table_capacity 0");
-    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.text = false; s.total = 0; s.rec_mark = 0;
+    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.text = false; s.defl = false; s.total = 0; s.rec_mark = 0;
     if (n_records == 0) return CK_OK;
     if (offsets[0] != 0) return fail(ctx, CK_ERR_ARG, "offsets[0] must be 0");
     const u64 total = offsets[n_records];
@@ -933,7 +948,7 @@ int wait_common(ck_ctx *ctx, int slot, bool uniq, uint8_t *out_bytes, uint32_t *
     if (!ctx) return CK_ERR_ARG;
     if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
     Slot &s = ctx->slot[slot];
-    if (!s.busy || s.uniq != uniq || s.mono || s.text) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    if (!s.busy || s.uniq != uniq || s.mono || s.text || s.defl) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
     s.busy = false;
     if (s.n == 0) {
         if (uniq && ctx->peer.attached && ctx->peer.world > 1) CK_CUDA(ctx, cudaStreamSynchronize(s.stream));
@@ -1064,6 +1079,13 @@ void ck_destroy(ck_ctx *ctx)
         for (void *p : ptrs) if (p) cudaFree(p);
         if (s.h_counts) cudaFreeHost(s.h_counts);
         if (s.stream) cudaStreamDestroy(s.stream);
+        {
+            Slot::Deflate &z = s.z;
+            void *zp[] = {z.buf, z.kA, z.kB, z.vA, z.vB, z.prev8, z.prev4, z.seg, z.out, z.result, z.tmp};
+            for (void *p : zp) if (p) cudaFree(p);
+            if (z.h_result) cudaFreeHost(z.h_result);
+            if (z.stream) cudaStreamDestroy(z.stream);
+        }
         if (s.inserted) cudaEventDestroy(s.inserted);
         free_scratch(s.scr);
     }
@@ -1388,7 +1410,7 @@ int ck_fasta_submit(ck_ctx *ctx, int slot, const uint8_t *text, uint64_t text_by
     if (is_mono && (rc = mono_options_check(ctx, mono))) return rc;
     CK_CUDA(ctx, cudaSetDevice(ctx->device));
     if ((rc = text_alloc(ctx, s))) return rc;
-    s.n = 0; s.total = 0; s.uniq = uniq; s.mono = is_mono; s.text = true; s.cmd = command;
+    s.n = 0; s.total = 0; s.uniq = uniq; s.mono = is_mono; s.text = true; s.defl = false; s.cmd = command;
     s.flags = CK_F_NORMALIZE | (is_mono ? 0u : CK_F_ALIGNED_OUT) | (uniq && !(flags & CK_F_CANONICAL_BODY) ? CK_F_NO_BYTES : 0u);
     if (text_bytes == 0) return submit_empty(ctx, s, base_index);
     cudaStream_t st = s.stream;
@@ -1462,6 +1484,123 @@ int ck_fasta_wait(ck_ctx *ctx, int slot, uint8_t *out_fasta, uint64_t *out_fasta
     if (out_index && nw) CK_CUDA(ctx, cudaMemcpyAsync(out_index, s.sel, (size_t)nw * 4, cudaMemcpyDeviceToHost, st));
     if (out_fasta && bytes) CK_CUDA(ctx, cudaMemcpyAsync(out_fasta, s.d_frame, bytes, cudaMemcpyDeviceToHost, st));
     CK_CUDA(ctx, cudaStreamSynchronize(st));
+    return CK_OK;
+}
+
+// ---- DEFLATE (ck_deflate_submit / ck_deflate_wait; csrc/ck_deflate.cuh) ------------------------------------------------
+// stored blocks of 65 535 bytes (two per segment), an empty stored block after the last segment, and whole words for the
+// pack kernel's edge stores
+uint64_t ck_deflate_bound(uint64_t n) { return n + 10 * ((n + CKZ_SEG - 1) / CKZ_SEG) + 16; }
+
+static u64 cap_segs(const Slot::Deflate &z) { return z.cap / CKZ_SEG; }
+
+static int deflate_alloc(ck_ctx *ctx, Slot::Deflate &z, u64 n)
+{
+    if (!z.stream) CK_CUDA(ctx, cudaStreamCreateWithFlags(&z.stream, cudaStreamNonBlocking));
+    if (!z.h_result) CK_CUDA(ctx, cudaMallocHost(&z.h_result, 16));
+    if (z.cap >= n) return CK_OK;
+    u64 cap = 1ull << 20;
+    while (cap < n) cap <<= 1;
+    cap = std::min<u64>(cap, CK_DEFLATE_MAX_BYTES);
+    CK_CUDA(ctx, cudaStreamSynchronize(z.stream));
+    void *zp[] = {z.buf, z.kA, z.kB, z.vA, z.vB, z.prev8, z.prev4, z.seg, z.out, z.result, z.tmp};
+    for (void *p : zp) if (p) cudaFree(p);
+    cudaStream_t keep_stream = z.stream;
+    u32 *keep_result = z.h_result;
+    z = Slot::Deflate{};
+    z.stream = keep_stream; z.h_result = keep_result;
+    const u64 N = cap + CK_DEFLATE_DICT_BYTES, segs = cap / CKZ_SEG;
+    CK_CUDA(ctx, cudaMalloc(&z.buf, N + 64));
+    for (u32 **p : {&z.kA, &z.kB, &z.vA, &z.vB, &z.prev8, &z.prev4}) CK_CUDA(ctx, cudaMalloc(p, N * 4));
+    CK_CUDA(ctx, cudaMalloc(&z.seg, segs * (2 * CKZ_SYMS + CKZ_HDR_WORDS + 8) * 4 + 64));
+    CK_CUDA(ctx, cudaMalloc(&z.out, (ck_deflate_bound(cap) + 7) / 4 * 4));
+    CK_CUDA(ctx, cudaMalloc(&z.result, 16));
+    cub::DoubleBuffer<u32> k(z.kA, z.kB), v(z.vA, z.vB);
+    size_t tb = 0;
+    CK_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, tb, k, v, (int)N, 0, CKZ_HBITS, z.stream));
+    CK_CUDA(ctx, cudaMalloc(&z.tmp, tb));
+    z.tmp_bytes = tb;
+    z.cap = cap;
+    return CK_OK;
+}
+
+// hash chains of one key width over buf[0, N): keys, stable radix sort, links
+static int deflate_chain(ck_ctx *ctx, Slot::Deflate &z, u32 N, u32 width, u32 *prev)
+{
+    cudaStream_t st = z.stream;
+    const u32 g = (N + 255) / 256;
+    k_defl_keys<<<g, 256, 0, st>>>(z.buf, N, width, z.kA, z.vA);
+    cub::DoubleBuffer<u32> k(z.kA, z.kB), v(z.vA, z.vB);
+    size_t tb = z.tmp_bytes;
+    CK_CUDA(ctx, cub::DeviceRadixSort::SortPairs(z.tmp, tb, k, v, (int)N, 0, CKZ_HBITS, st));
+    k_defl_links<<<g, 256, 0, st>>>(k.Current(), v.Current(), N, prev);
+    ctx->launches += 3;
+    CK_CUDA(ctx, cudaGetLastError());
+    return CK_OK;
+}
+
+int ck_deflate_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, uint64_t n, const uint8_t *dict, uint32_t dict_bytes,
+                      uint32_t crc_in)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    if (n == 0 || n > CK_DEFLATE_MAX_BYTES) return fail(ctx, CK_ERR_ARG, "n must be 1 .. CK_DEFLATE_MAX_BYTES");
+    if (dict_bytes > CK_DEFLATE_DICT_BYTES) return fail(ctx, CK_ERR_ARG, "dict_bytes exceeds CK_DEFLATE_DICT_BYTES");
+    if (!bytes || (dict_bytes && !dict)) return fail(ctx, CK_ERR_ARG, "null argument");
+    Slot &s = ctx->slot[slot];
+    if (s.busy) return fail(ctx, CK_ERR_STATE, "slot already holds a batch; call the matching wait first");
+    CK_CUDA(ctx, cudaSetDevice(ctx->device));
+    Slot::Deflate &z = s.z;
+    int rc;
+    if ((rc = deflate_alloc(ctx, z, n))) return rc;
+    cudaStream_t st = z.stream;
+    const u32 D = dict_bytes, N = (u32)(D + n), nseg = (u32)((n + CKZ_SEG - 1) / CKZ_SEG);
+    if (D) CK_CUDA(ctx, cudaMemcpyAsync(z.buf, dict, D, cudaMemcpyHostToDevice, st));
+    CK_CUDA(ctx, cudaMemcpyAsync(z.buf + D, bytes, n, cudaMemcpyHostToDevice, st));
+    CK_CUDA(ctx, cudaMemsetAsync(z.buf + N, 0, 64, st));
+    if ((rc = deflate_chain(ctx, z, N, 8, z.prev8))) return rc;
+    if ((rc = deflate_chain(ctx, z, N, 4, z.prev4))) return rc;
+    DeflateArgs a{};
+    a.buf = z.buf; a.dict = D; a.n = (u32)n; a.nseg = nseg;
+    a.prev8 = z.prev8; a.prev4 = z.prev4;
+    a.match = z.kA; a.tok = z.kB;                       // the sort buffers are free again
+    const u64 S = cap_segs(z);
+    a.freq = z.seg; a.table = a.freq + S * CKZ_SYMS; a.hdr = a.table + S * CKZ_SYMS; a.meta = a.hdr + S * CKZ_HDR_WORDS;
+    a.seg_crc = a.meta + 4 * S; a.ntok = a.seg_crc + S;
+    a.off = reinterpret_cast<u64 *>(a.ntok + S);        // S is even: 8-byte aligned
+    a.out = z.out; a.result = z.result; a.crc_in = crc_in;
+    k_defl_match<<<nseg, 256, 0, st>>>(a);
+    k_defl_parse<<<nseg, 128, 0, st>>>(a);
+    k_defl_huff<<<nseg, 256, 0, st>>>(a);
+    CK_CUDA(ctx, cudaMemsetAsync(z.out, 0, (ck_deflate_bound(n) + 7) / 4 * 4, st));
+    k_defl_place<<<1, 1024, 0, st>>>(a);
+    k_defl_pack<<<nseg, 256, 0, st>>>(a);
+    ctx->launches += 5;
+    CK_CUDA(ctx, cudaGetLastError());
+    CK_CUDA(ctx, cudaMemcpyAsync(z.h_result, z.result, 12, cudaMemcpyDeviceToHost, st));
+    z.n = n;
+    s.busy = true; s.defl = true; s.uniq = false; s.mono = false; s.text = false;
+    return CK_OK;
+}
+
+int ck_deflate_wait(ck_ctx *ctx, int slot, uint8_t *out, uint64_t *out_bytes, uint32_t *crc_out)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    Slot &s = ctx->slot[slot];
+    if (!s.busy || !s.defl) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    s.busy = false; s.defl = false;
+    if (out_bytes) *out_bytes = 0;
+    Slot::Deflate &z = s.z;
+    CK_CUDA(ctx, cudaStreamSynchronize(z.stream));
+    const u64 bytes = (u64)z.h_result[0] | (u64)z.h_result[1] << 32;
+    if (bytes > ck_deflate_bound(z.n)) return fail(ctx, CK_ERR_CUDA, "deflate output exceeds its bound");
+    if (out && bytes) {
+        CK_CUDA(ctx, cudaMemcpyAsync(out, z.out, bytes, cudaMemcpyDeviceToHost, z.stream));
+        CK_CUDA(ctx, cudaStreamSynchronize(z.stream));
+    }
+    if (out_bytes) *out_bytes = bytes;
+    if (crc_out) *crc_out = z.h_result[2];
     return CK_OK;
 }
 

@@ -351,6 +351,28 @@ int ck_fasta_submit(ck_ctx *ctx, int slot, const uint8_t *text, uint64_t text_by
 int ck_fasta_wait(ck_ctx *ctx, int slot, uint8_t *out_fasta, uint64_t *out_fasta_bytes, uint32_t *out_n_written,
                   uint32_t *out_index, uint64_t *out_head, uint64_t *out_first_index, uint32_t *out_full_len,
                   uint32_t *out_monomer_len);
+/* ---- DEFLATE on the device: the `.gz` output of `circkit ... -o out.gz` (src/utils.rs:29-72, flate2 at level 6) ---------
+ * ck_deflate_submit compresses n bytes (1 .. CK_DEFLATE_MAX_BYTES) on one of the two slots into raw DEFLATE (RFC 1951):
+ * blocks none of which has BFINAL set, ending byte-aligned with an empty stored block (00 00 ff ff, zlib's Z_SYNC_FLUSH).
+ * `dict` (dict_bytes <= CK_DEFLATE_DICT_BYTES; may be NULL when 0) is what came before `bytes` in the stream: matches may reach
+ * into it, and never further than 32 768 bytes back or before its start, so consecutive calls, each given the last 32 KiB of
+ * the input before it, concatenate into one deflate stream (one gzip member: a header, the fragments, 03 00, CRC-32 and
+ * ISIZE).  zlib.decompressobj(-15, zdict=dict).decompress(out) == bytes.  The output is a function of (bytes, dict) only.
+ * ck_deflate_wait copies *out_bytes (<= ck_deflate_bound(n)) bytes to `out` and gives the CRC-32 of `bytes` continued from
+ * crc_in (== zlib.crc32(bytes, crc_in)); out_bytes and crc_out may be NULL.
+ * A deflate call occupies its slot like any other batch (CK_ERR_STATE when busy, or for a wait without a submit); it runs on a
+ * stream of its own, so it works on a context created with max_batch_bytes = max_batch_records = 0 (no batch staging).  n == 0,
+ * n > CK_DEFLATE_MAX_BYTES, dict_bytes > CK_DEFLATE_DICT_BYTES or a NULL pointer -> CK_ERR_ARG, nothing is enqueued and the
+ * slot stays usable.  The slot's first deflate call allocates its buffers (about 30 bytes of HBM per input byte of the largest
+ * call so far, rounded up to a power of two), so contexts that never deflate use no more device memory.  `bytes` and `dict`
+ * may be reused once the submit returns when they are pageable; pinned buffers must stay untouched until the wait. */
+#define CK_DEFLATE_MAX_BYTES (64ull << 20)
+#define CK_DEFLATE_DICT_BYTES 32768u
+uint64_t ck_deflate_bound(uint64_t n);   /* out bytes to provide for n input bytes */
+int ck_deflate_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, uint64_t n, const uint8_t *dict, uint32_t dict_bytes,
+                      uint32_t crc_in);
+int ck_deflate_wait(ck_ctx *ctx, int slot, uint8_t *out, uint64_t *out_bytes, uint32_t *crc_out);
+
 /* number of kernels this context has launched so far (bench.py's gpu_launches) */
 uint64_t ck_launch_count(const ck_ctx *ctx);
 /* per-class kernel timing for the roofline: when enabled, every length/alphabet-class launch is bracketed
