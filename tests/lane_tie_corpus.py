@@ -278,15 +278,15 @@ def doubled_corpus(seed: int = 2) -> list[Rec]:
     return out
 
 
-def rotations_and_revcomps(seqs: list[bytes], rng) -> list[bytes]:
+def rotations_and_revcomps(seqs: list[bytes], rng, run: bytes = b"AAAA") -> list[bytes]:
     """seqs, followed by duplicates that must collapse onto them: rotations (half of them starting inside the run of the key,
-    i.e. inside a tie), reverse complements, and both"""
+    i.e. inside a tie; `run` finds it), reverse complements, and both"""
     out = list(seqs)
     for s in seqs:
         n = len(s)
         if not n or rng.random() < 0.5:
             continue
-        a = s.find(b"AAAA")
+        a = s.find(run)
         r = (a + int(rng.integers(0, 8))) % n if a >= 0 and rng.random() < 0.5 else int(rng.integers(n))
         t = s[r:] + s[:r]
         out.append(revcomp(t) if rng.random() < 0.5 else t)
