@@ -78,6 +78,8 @@ pub mod ffi {
     /// ck_deflate_submit: largest input of one call, largest dictionary
     pub const CK_DEFLATE_MAX_BYTES: u64 = 64 << 20;
     pub const CK_DEFLATE_DICT_BYTES: u32 = 32768;
+    /// ck_bzip2_submit: largest input of one call
+    pub const CK_BZIP2_MAX_BYTES: u64 = 64 << 20;
     extern "C" {
         pub fn ck_init(cfg: *const CkConfig, out: *mut *mut CkCtx) -> c_int;
         pub fn ck_destroy(ctx: *mut CkCtx);
@@ -121,6 +123,12 @@ pub mod ffi {
         pub fn ck_deflate_submit(ctx: *mut CkCtx, slot: c_int, bytes: *const u8, n: u64, dict: *const u8, dict_bytes: u32,
                                  crc_in: u32) -> c_int;
         pub fn ck_deflate_wait(ctx: *mut CkCtx, slot: c_int, out: *mut u8, out_bytes: *mut u64, crc_out: *mut u32) -> c_int;
+        pub fn ck_bzip2_bound(n: u64) -> u64;
+        pub fn ck_bzip2_submit(ctx: *mut CkCtx, slot: c_int, bytes: *const u8, n: u64, final_: c_int, bits_in: u32,
+                               nbits_in: u32, crc_in: u32) -> c_int;
+        pub fn ck_bzip2_wait(ctx: *mut CkCtx, slot: c_int, out: *mut u8, out_bytes: *mut u64, consumed: *mut u64,
+                             bits_out: *mut u32, nbits_out: *mut u32, crc_out: *mut u32) -> c_int;
+        pub fn ck_bzip2_stats(ctx: *mut CkCtx, slot: c_int, stage_ms: *mut f32, bwt_rounds: *mut u32) -> c_int;
         pub fn ck_peer_export(ctx: *mut CkCtx, world: u32, rank: u32, max_records: u32, handle_out: *mut c_void) -> c_int;
         pub fn ck_peer_attach(ctx: *mut CkCtx, all_handles: *const c_void) -> c_int;
         pub fn ck_lmsr_index(ctx: *mut CkCtx, s: *const u8, n: usize, out_index: *mut usize) -> c_int;

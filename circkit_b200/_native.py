@@ -16,6 +16,7 @@ CK_MONO_SENSITIVE, CK_MONO_FIRST_ONLY, CK_MONO_KEEP_ALL, CK_MONO_NONE = 1, 2, 4,
 CK_CMD_CANONICALIZE, CK_CMD_UNIQ, CK_CMD_MONOMERIZE = 1, 2, 3
 CK_F_CANONICAL_BODY = 64
 CK_DEFLATE_MAX_BYTES, CK_DEFLATE_DICT_BYTES = 64 << 20, 32768
+CK_BZIP2_MAX_BYTES = 64 << 20
 CK_CLASS_2BIT_LE_512, CK_CLASS_2BIT_LE_2048, CK_CLASS_2BIT_LE_65536, CK_CLASS_2BIT_LE_425984 = 1, 2, 4, 8
 CK_CLASS_2BIT_LE_4096, CK_CLASS_2BIT_LE_8192 = 1 << 10, 1 << 11
 
@@ -94,6 +95,11 @@ SIGNATURES = {
     "ck_deflate_bound": (_u64, [_u64]),
     "ck_deflate_submit": (_i, [_vp, _i, _vp, _u64, _vp, _u32, _u32]),
     "ck_deflate_wait": (_i, [_vp, _i, _vp, C.POINTER(_u64), C.POINTER(_u32)]),
+    "ck_bzip2_bound": (_u64, [_u64]),
+    "ck_bzip2_submit": (_i, [_vp, _i, _vp, _u64, _i, _u32, _u32, _u32]),
+    "ck_bzip2_wait": (_i, [_vp, _i, _vp, C.POINTER(_u64), C.POINTER(_u64), C.POINTER(_u32), C.POINTER(_u32),
+                           C.POINTER(_u32)]),
+    "ck_bzip2_stats": (_i, [_vp, _i, C.POINTER(C.c_float), C.POINTER(_u32)]),
     "ck_launch_count": (_u64, [_vp]),
     "ck_kernel_timing": (_i, [_vp, _i]),
     "ck_kernel_times": (_i, [_vp, _vp, _vp, _u32]),

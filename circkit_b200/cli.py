@@ -342,15 +342,50 @@ class DeviceDeflate:
             self.ctx = None
 
 
+class DeviceBzip2:
+    """bzip2 on the GPU for Writer's bz2 output (ck_bzip2_submit / ck_bzip2_wait), libbzip2's bytes at level 9:
+    bzip2(data, final, bits, nbits, crc) -> (bytes, consumed, bits, nbits, crc) writes the blocks that are complete in
+    `data` (all of them when final) after the nbits pending bits, and continues the combined CRC.  The context (no batch
+    staging, so the pump's slots are untouched) and the pinned buffers are created by the first call."""
+
+    max_bytes = N.CK_BZIP2_MAX_BYTES
+
+    def __init__(self, device: int = 0):
+        self.device, self.ctx, self.pinned = device, None, {}
+
+    _buf = DeviceDeflate._buf
+
+    def bzip2(self, data, final: bool, bits: int, nbits: int, crc: int):
+        if self.ctx is None:
+            self.ctx = Context(self.device, max_batch_bytes=0, max_batch_records=0)
+        n = len(data)
+        src = self._buf(0, n)[:n]
+        src[:] = np.frombuffer(data, dtype=np.uint8)
+        out = self._buf(1, self.ctx.bzip2_bound(n))
+        self.ctx.bzip2_submit(0, src, final, bits, nbits, crc)
+        return self.ctx.bzip2_wait(0, out)
+
+    close = DeviceDeflate.close
+
+
+BZIP2_HEADER = b"BZh9"
+BZIP2_EOS = 0x177245385090
+
+
 class Writer:
     """src/utils.rs:29-72 as a stream: stdout, or a file compressed by its suffix (gz 6, bz2 9, xz 6, zst 1; else plain).
     gzip_encoder (gz only; e.g. DeviceDeflate()): an object with max_bytes, deflate(data, dict, crc) -> (raw deflate
     fragment ending in a sync flush, crc) and close().  Writer then frames the gzip member itself: GZIP_HEADER, one
     fragment per call of at most max_bytes bytes, each given the last 32 KiB written before it as its dictionary, and at
-    close the final empty block (03 00), the CRC-32 and ISIZE.  Without it, gz goes through gzip.GzipFile at level 6."""
+    close the final empty block (03 00), the CRC-32 and ISIZE.  Without it, gz goes through gzip.GzipFile at level 6.
+    bzip2_encoder (bz2 only; e.g. DeviceBzip2()): an object with max_bytes, bzip2(data, final, bits, nbits, crc) ->
+    (bytes, consumed, bits, nbits, crc) as ck_bzip2_wait gives them, and close().  Writer writes BZIP2_HEADER, buffers
+    until a call can take max_bytes, keeps each call's unconsumed tail for the next, and at close makes the final call and
+    writes the end-of-stream marker, the combined CRC and the padding: the bytes of bz2.compress(all, 9).  Without it, bz2
+    goes through bz2.BZ2File at level 9."""
 
-    def __init__(self, path: str | None, gzip_encoder=None):
-        self.path, self.zst, self.gz = path, None, None
+    def __init__(self, path: str | None, gzip_encoder=None, bzip2_encoder=None):
+        self.path, self.zst, self.gz, self.bz = path, None, None, None
         if path is None:
             self.f = sys.stdout.buffer
             return
@@ -359,6 +394,10 @@ class Writer:
             self.f, self.gz = open(path, "wb"), gzip_encoder
             self.crc, self.size, self.tail = 0, 0, b""
             self.f.write(GZIP_HEADER)
+        elif ext == "bz2" and bzip2_encoder is not None:
+            self.f, self.bz = open(path, "wb"), bzip2_encoder
+            self.crc, self.bits, self.nbits, self.pending = 0, 0, 0, bytearray()
+            self.f.write(BZIP2_HEADER)
         elif ext == "gz":
             self.f = gzip.GzipFile(path, "wb", compresslevel=6)
         elif ext == "bz2":
@@ -381,10 +420,23 @@ class Writer:
                 self.f.write(frag)
                 self.size += len(piece)
                 self.tail = (self.tail + piece[-32768:].tobytes())[-32768:]
+        elif self.bz is not None:
+            self.pending += data
+            while len(self.pending) >= self.bz.max_bytes:
+                self._bzip2_call(memoryview(self.pending)[:self.bz.max_bytes], False)
         elif self.zst is not None:
             self.f.write(_zstd_compress(data, 1))             # concatenated frames are one valid zstd stream
         else:
             self.f.write(data)
+
+    def _bzip2_call(self, data, final: bool):
+        n = len(data)
+        out, consumed, self.bits, self.nbits, self.crc = self.bz.bzip2(data, final, self.bits, self.nbits, self.crc)
+        data.release()
+        if consumed == 0 and n >= self.bz.max_bytes or final and consumed != n:
+            raise RuntimeError("bzip2 encoder consumed %d of %d bytes" % (consumed, n))
+        self.f.write(out)
+        del self.pending[:consumed]
 
     def close(self):
         if self.path is None:
@@ -393,10 +445,18 @@ class Writer:
         try:
             if self.gz is not None:                          # final empty fixed block, CRC-32, ISIZE (RFC 1952)
                 self.f.write(b"\x03\x00" + struct.pack("<II", self.crc, self.size & 0xFFFFFFFF))
+            elif self.bz is not None:                        # the last blocks, end-of-stream marker, combined CRC, padding
+                if self.pending:
+                    self._bzip2_call(memoryview(self.pending), True)
+                nb = self.nbits + 80
+                v = (self.bits << 80 | BZIP2_EOS << 32 | self.crc) << (-nb % 8)
+                self.f.write(v.to_bytes((nb + 7) // 8, "big"))
         finally:
             try:
                 if self.gz is not None:
                     self.gz.close()
+                if self.bz is not None:
+                    self.bz.close()
             finally:
                 self.f.close()
 
@@ -734,7 +794,9 @@ def main(argv=None) -> int:
             if first is not None:
                 yield first
             yield from pieces
-        w = Writer(args.output, gzip_encoder=DeviceDeflate() if _suffix(args.output) == "gz" else None)
+        suffix = _suffix(args.output)
+        w = Writer(args.output, gzip_encoder=DeviceDeflate() if suffix == "gz" else None,
+                   bzip2_encoder=DeviceBzip2() if suffix == "bz2" else None)
         tf = None
         try:
             ext = None

@@ -83,6 +83,7 @@ class Context:
         self.max_batch_records = max_batch_records
         self._text_batch = {}           # slot -> (records, text bytes) of its text batch in flight
         self._deflate_batch = {}        # slot -> (input bytes, input, dict) of its deflate call in flight
+        self._bzip2_batch = {}          # slot -> input bytes of its bzip2 call in flight
 
     # -- plumbing
     @property
@@ -313,6 +314,44 @@ class Context:
         """deflate_submit + deflate_wait on slot 0"""
         self.deflate_submit(0, data, dict, crc)
         return self.deflate_wait(0)
+
+    # -- bzip2 on the device (ck_bzip2_submit / ck_bzip2_wait): the blocks of one bzip2 stream, as libbzip2 writes at level 9
+    def bzip2_bound(self, n: int) -> int:
+        return int(self._lib.ck_bzip2_bound(n))
+
+    def bzip2_submit(self, slot: int, data, final: bool, bits: int = 0, nbits: int = 0, crc: int = 0):
+        """ck_bzip2_submit: `data` (bytes-like or a uint8 array; 1 .. CK_BZIP2_MAX_BYTES bytes) is the stream from its first
+        byte not yet in a written block; (bits, nbits) the pending bits before it (nbits < 8, in the low bits of `bits`);
+        crc the combined CRC of the blocks before it.  `final` writes every block, ending the stream's last run."""
+        a = data if isinstance(data, np.ndarray) else np.frombuffer(data, dtype=np.uint8)
+        self._check(self._lib.ck_bzip2_submit(self._h, slot, a.ctypes.data if len(a) else None, len(a), 1 if final else 0,
+                                              bits & 0xFF, nbits, crc & 0xFFFFFFFF))
+        self._bzip2_batch[slot] = len(a)
+
+    def bzip2_wait(self, slot: int, out: "np.ndarray | None" = None) -> "tuple[bytes, int, int, int, int]":
+        """ck_bzip2_wait -> (whole bytes of the blocks written, consumed input bytes, pending bits, their count, combined
+        CRC).  `out`: optional uint8 buffer (pinned, for speed) of at least bzip2_bound(n) bytes."""
+        n = self._bzip2_batch.pop(slot, 0)
+        need = self.bzip2_bound(n)
+        if out is None or len(out) < need:
+            out = np.empty(need, dtype=np.uint8)
+        nbytes, consumed = C.c_uint64(0), C.c_uint64(0)
+        bits, nbits, crc = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+        self._check(self._lib.ck_bzip2_wait(self._h, slot, out.ctypes.data, C.byref(nbytes), C.byref(consumed),
+                                            C.byref(bits), C.byref(nbits), C.byref(crc)))
+        return (out[:int(nbytes.value)].tobytes(), int(consumed.value), int(bits.value), int(nbits.value),
+                int(crc.value))
+
+    def bzip2(self, data, final: bool, bits: int = 0, nbits: int = 0, crc: int = 0):
+        """bzip2_submit + bzip2_wait on slot 0"""
+        self.bzip2_submit(0, data, final, bits, nbits, crc)
+        return self.bzip2_wait(0)
+
+    def bzip2_stats(self, slot: int = 0) -> "tuple[list[float], int]":
+        """ck_bzip2_stats of the last call: device ms of (RLE1 and cuts, BWT, MTF, tables, pack), BWT sort rounds"""
+        ms, rounds = (C.c_float * 5)(), C.c_uint32(0)
+        self._check(self._lib.ck_bzip2_stats(self._h, slot, ms, C.byref(rounds)))
+        return list(ms), int(rounds.value)
 
     def uniq_batch(self, arena: np.ndarray, offsets: np.ndarray, base_index: int = 0, *, normalize: bool = False,
                    want_bytes=True, aligned=False):

@@ -26,6 +26,7 @@
 #include "ck_monomerize.cuh"
 #include "ck_fasta.cuh"
 #include "ck_deflate.cuh"
+#include "ck_bzip2.cuh"
 
 using namespace ck;
 
@@ -127,6 +128,23 @@ struct Slot {
         void *tmp = nullptr; size_t tmp_bytes = 0;
         u64 n = 0;
     } z;
+    bool bz = false;                    // ck_bzip2_submit's call (ck_bzip2_wait collects it)
+    // ck_bzip2_*: own stream and buffers, allocated by the slot's first bzip2 call and grown to the largest since
+    struct Bzip2 {
+        cudaStream_t stream = nullptr;
+        cudaEvent_t ev[6] = {};         // stage boundaries of the last call
+        u64 cap = 0, rcap = 0;          // raw input bytes / RLE1 bytes the buffers hold
+        u8 *in = nullptr, *rle = nullptr, *bid = nullptr, *flag = nullptr;
+        u32 *rank = nullptr, *sa = nullptr, *pos = nullptr, *pos2 = nullptr, *valA = nullptr, *valB = nullptr;
+        u32 *hp = nullptr, *hs = nullptr;
+        u64 *keyA = nullptr, *keyB = nullptr;
+        u8 *small = nullptr;            // blocks, meta, freq, selectors, codes, headers, heap scratch
+        u32 *out = nullptr, *result = nullptr;
+        u32 *h_host = nullptr;          // pinned: [0..3] Bzip2Meta, [4..7] result, [8] selected count
+        void *tmp = nullptr; size_t tmp_bytes = 0;
+        u64 n = 0;
+        u32 nblk = 0, consumed = 0, rounds = 0, bits_in = 0, nbits_in = 0, crc_in = 0;
+    } bz2;
 };
 
 // Multi-GPU uniq through the C ABI: this rank's exchange block (exported by CUDA IPC) and every peer's, mapped here.
@@ -695,7 +713,7 @@ int submit_check(ck_ctx *ctx, int slot, const uint64_t *offsets, uint32_t n_reco
     if (n_records && (!offsets || (!have_bytes && offsets[n_records] != offsets[0])))
         return fail(ctx, CK_ERR_ARG, "null batch pointers");
     if (uniq && !ctx->table) return fail(ctx, CK_ERR_STATE, "context was created with table_capacity 0");
-    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.text = false; s.defl = false; s.total = 0; s.rec_mark = 0;
+    s.n = n_records; s.flags = flags; s.uniq = uniq; s.mono = false; s.text = false; s.defl = false; s.bz = false; s.total = 0; s.rec_mark = 0;
     if (n_records == 0) return CK_OK;
     if (offsets[0] != 0) return fail(ctx, CK_ERR_ARG, "offsets[0] must be 0");
     const u64 total = offsets[n_records];
@@ -948,7 +966,7 @@ int wait_common(ck_ctx *ctx, int slot, bool uniq, uint8_t *out_bytes, uint32_t *
     if (!ctx) return CK_ERR_ARG;
     if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
     Slot &s = ctx->slot[slot];
-    if (!s.busy || s.uniq != uniq || s.mono || s.text || s.defl) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    if (!s.busy || s.uniq != uniq || s.mono || s.text || s.defl || s.bz) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
     s.busy = false;
     if (s.n == 0) {
         if (uniq && ctx->peer.attached && ctx->peer.world > 1) CK_CUDA(ctx, cudaStreamSynchronize(s.stream));
@@ -1084,6 +1102,15 @@ void ck_destroy(ck_ctx *ctx)
             void *zp[] = {z.buf, z.kA, z.kB, z.vA, z.vB, z.prev8, z.prev4, z.seg, z.out, z.result, z.tmp};
             for (void *p : zp) if (p) cudaFree(p);
             if (z.h_result) cudaFreeHost(z.h_result);
+            if (z.stream) cudaStreamDestroy(z.stream);
+        }
+        {
+            Slot::Bzip2 &z = s.bz2;
+            void *zp[] = {z.in, z.rle, z.bid, z.flag, z.rank, z.sa, z.pos, z.pos2, z.valA, z.valB, z.hp, z.hs, z.keyA, z.keyB,
+                          z.small, z.out, z.result, z.tmp};
+            for (void *p : zp) if (p) cudaFree(p);
+            if (z.h_host) cudaFreeHost(z.h_host);
+            for (cudaEvent_t e : z.ev) if (e) cudaEventDestroy(e);
             if (z.stream) cudaStreamDestroy(z.stream);
         }
         if (s.inserted) cudaEventDestroy(s.inserted);
@@ -1410,7 +1437,7 @@ int ck_fasta_submit(ck_ctx *ctx, int slot, const uint8_t *text, uint64_t text_by
     if (is_mono && (rc = mono_options_check(ctx, mono))) return rc;
     CK_CUDA(ctx, cudaSetDevice(ctx->device));
     if ((rc = text_alloc(ctx, s))) return rc;
-    s.n = 0; s.total = 0; s.uniq = uniq; s.mono = is_mono; s.text = true; s.defl = false; s.cmd = command;
+    s.n = 0; s.total = 0; s.uniq = uniq; s.mono = is_mono; s.text = true; s.defl = false; s.bz = false; s.cmd = command;
     s.flags = CK_F_NORMALIZE | (is_mono ? 0u : CK_F_ALIGNED_OUT) | (uniq && !(flags & CK_F_CANONICAL_BODY) ? CK_F_NO_BYTES : 0u);
     if (text_bytes == 0) return submit_empty(ctx, s, base_index);
     cudaStream_t st = s.stream;
@@ -1579,7 +1606,7 @@ int ck_deflate_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, uint64_t n, c
     CK_CUDA(ctx, cudaGetLastError());
     CK_CUDA(ctx, cudaMemcpyAsync(z.h_result, z.result, 12, cudaMemcpyDeviceToHost, st));
     z.n = n;
-    s.busy = true; s.defl = true; s.uniq = false; s.mono = false; s.text = false;
+    s.busy = true; s.defl = true; s.bz = false; s.uniq = false; s.mono = false; s.text = false;
     return CK_OK;
 }
 
@@ -1601,6 +1628,213 @@ int ck_deflate_wait(ck_ctx *ctx, int slot, uint8_t *out, uint64_t *out_bytes, ui
     }
     if (out_bytes) *out_bytes = bytes;
     if (crc_out) *crc_out = z.h_result[2];
+    return CK_OK;
+}
+
+// ---- bzip2 (ck_bzip2_submit / ck_bzip2_wait; csrc/ck_bzip2.cuh) --------------------------------------------------------
+// at most 17 bits per MTF symbol, at most 5/4 RLE1 bytes per raw byte, and a header per block; every block but the last
+// covers >= 4/5 * CKB_BLOCK_MAX raw bytes
+uint64_t ck_bzip2_bound(uint64_t n) { return 3 * n + (n / (CKB_BLOCK_MAX * 4 / 5) + 2) * (CKB_HDR_WORDS * 4) + 64; }
+
+// the fixed-size per-block arrays, carved from Slot::Bzip2::small
+static size_t bzip2_layout(u8 *p, Bzip2Args *a)
+{
+    u8 *const p0 = p;
+    auto take = [&p](size_t bytes) { u8 *q = p; p += (bytes + 255) / 256 * 256; return q; };
+    Bzip2Block *blk = reinterpret_cast<Bzip2Block *>(take(CKB_MAX_BLOCKS * sizeof(Bzip2Block)));
+    Bzip2Meta *meta = reinterpret_cast<Bzip2Meta *>(take(sizeof(Bzip2Meta)));
+    u32 *freq = reinterpret_cast<u32 *>(take((size_t)CKB_MAX_BLOCKS * CKB_ALPHA * 4));
+    u32 *code = reinterpret_cast<u32 *>(take((size_t)CKB_MAX_BLOCKS * CKB_GROUPS * CKB_ALPHA * 4));
+    u32 *hdr = reinterpret_cast<u32 *>(take((size_t)CKB_MAX_BLOCKS * CKB_HDR_WORDS * 4));
+    int *hb = reinterpret_cast<int *>(take((size_t)CKB_MAX_BLOCKS * CKB_GROUPS * sizeof(BzHeap)));
+    u8 *sel = take((size_t)CKB_MAX_BLOCKS * CKB_MAX_SEL);
+    if (a) { a->blk = blk; a->meta = meta; a->freq = freq; a->code = code; a->hdr = hdr; a->hb = hb; a->sel = sel; }
+    return (size_t)(p - p0);
+}
+
+static int bzip2_alloc(ck_ctx *ctx, Slot::Bzip2 &z, u64 n)
+{
+    if (!z.stream) CK_CUDA(ctx, cudaStreamCreateWithFlags(&z.stream, cudaStreamNonBlocking));
+    if (!z.h_host) CK_CUDA(ctx, cudaMallocHost(&z.h_host, 64));
+    if (!z.ev[0]) for (cudaEvent_t &e : z.ev) CK_CUDA(ctx, cudaEventCreate(&e));
+    if (!z.small) CK_CUDA(ctx, cudaMalloc(&z.small, bzip2_layout(nullptr, nullptr)));
+    if (z.cap >= n) return CK_OK;
+    u64 cap = 1ull << 20;
+    while (cap < n) cap <<= 1;
+    cap = std::min<u64>(cap, CK_BZIP2_MAX_BYTES);
+    CK_CUDA(ctx, cudaStreamSynchronize(z.stream));
+    void *zp[] = {z.in, z.rle, z.bid, z.flag, z.rank, z.sa, z.pos, z.pos2, z.valA, z.valB, z.hp, z.hs, z.keyA, z.keyB,
+                  z.out, z.result, z.tmp};
+    for (void *p : zp) if (p) cudaFree(p);
+    z.in = z.rle = z.bid = z.flag = nullptr;
+    z.rank = z.sa = z.pos = z.pos2 = z.valA = z.valB = z.hp = z.hs = nullptr;
+    z.keyA = z.keyB = nullptr; z.out = z.result = nullptr; z.tmp = nullptr; z.cap = 0;
+    const u64 R = cap + cap / 4 + 64;                   // RLE1 bytes: a run of 4 takes 5
+    CK_CUDA(ctx, cudaMalloc(&z.in, cap + 64));
+    for (u8 **p : {&z.rle, &z.bid, &z.flag}) CK_CUDA(ctx, cudaMalloc(p, R + 64));
+    for (u32 **p : {&z.rank, &z.sa, &z.pos, &z.pos2, &z.valA, &z.valB, &z.hp, &z.hs}) CK_CUDA(ctx, cudaMalloc(p, R * 4));
+    for (u64 **p : {&z.keyA, &z.keyB}) CK_CUDA(ctx, cudaMalloc(p, R * 8));
+    CK_CUDA(ctx, cudaMalloc(&z.out, (ck_bzip2_bound(cap) + 7) / 4 * 4));
+    CK_CUDA(ctx, cudaMalloc(&z.result, 16));
+    size_t tb = 0, t1 = 0;
+    cub::DoubleBuffer<u64> k(z.keyA, z.keyB);
+    cub::DoubleBuffer<u32> v(z.valA, z.valB);
+    CK_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, t1, k, v, (int)R, 0, 64, z.stream));
+    tb = std::max(tb, t1);
+    CK_CUDA(ctx, cub::DeviceScan::InclusiveScan(nullptr, t1, z.hp, z.hs, BzMax(), (int)R, z.stream));
+    tb = std::max(tb, t1);
+    CK_CUDA(ctx, cub::DeviceScan::InclusiveSum(nullptr, t1, z.pos2, z.valB, (int)R, z.stream));
+    tb = std::max(tb, t1);
+    CK_CUDA(ctx, cub::DeviceSelect::Flagged(nullptr, t1, z.pos, z.flag, z.pos2, z.result + 3, (int)R, z.stream));
+    tb = std::max(tb, t1);
+    CK_CUDA(ctx, cudaMalloc(&z.tmp, tb));
+    z.tmp_bytes = tb;
+    z.cap = cap; z.rcap = R;
+    return CK_OK;
+}
+
+int ck_bzip2_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, uint64_t n, int final, uint32_t bits_in,
+                    uint32_t nbits_in, uint32_t crc_in)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    if (n == 0 || n > CK_BZIP2_MAX_BYTES) return fail(ctx, CK_ERR_ARG, "n must be 1 .. CK_BZIP2_MAX_BYTES");
+    if (nbits_in > 7) return fail(ctx, CK_ERR_ARG, "nbits_in must be 0 .. 7");
+    if (!bytes) return fail(ctx, CK_ERR_ARG, "null argument");
+    Slot &s = ctx->slot[slot];
+    if (s.busy) return fail(ctx, CK_ERR_STATE, "slot already holds a batch; call the matching wait first");
+    CK_CUDA(ctx, cudaSetDevice(ctx->device));
+    Slot::Bzip2 &z = s.bz2;
+    int rc;
+    if ((rc = bzip2_alloc(ctx, z, n))) return rc;
+    cudaStream_t st = z.stream;
+    Bzip2Args a{};
+    bzip2_layout(z.small, &a);
+    a.in = z.in; a.n = (u32)n; a.final = final ? 1 : 0;
+    a.rs = z.hp; a.runst = z.hs; a.enc = z.pos2; a.cum = z.valB;     // stage 1 only: the sort buffers are free then
+    a.rle = z.rle; a.bid = z.bid; a.sa = z.sa; a.rank = z.rank; a.last = z.flag;
+    a.mtfv = reinterpret_cast<u16 *>(z.keyA);             // after the sort
+    a.out = z.out; a.result = z.result;
+    a.bits_in = bits_in & ((1u << nbits_in) - 1); a.nbits_in = nbits_in; a.crc_in = crc_in;
+    const u32 n32 = (u32)n, g = (n32 + 255) / 256;
+    CK_CUDA(ctx, cudaEventRecord(z.ev[0], st));
+    CK_CUDA(ctx, cudaMemcpyAsync(z.in, bytes, n, cudaMemcpyHostToDevice, st));
+    k_bz_runs<<<g, 256, 0, st>>>(z.in, n32, a.rs);
+    size_t tb = z.tmp_bytes;
+    CK_CUDA(ctx, cub::DeviceScan::InclusiveScan(z.tmp, tb, a.rs, a.runst, BzMax(), (int)n32, st));
+    k_bz_tok<<<g, 256, 0, st>>>(a);
+    tb = z.tmp_bytes;
+    CK_CUDA(ctx, cub::DeviceScan::InclusiveSum(z.tmp, tb, a.enc, a.cum, (int)n32, st));
+    k_bz_cuts<<<1, 1, 0, st>>>(a);
+    ctx->launches += 5;
+    CK_CUDA(ctx, cudaGetLastError());
+    CK_CUDA(ctx, cudaMemcpyAsync(z.h_host, a.meta, sizeof(Bzip2Meta), cudaMemcpyDeviceToHost, st));
+    CK_CUDA(ctx, cudaStreamSynchronize(st));
+    Bzip2Meta m;
+    memcpy(&m, z.h_host, sizeof m);
+    z.n = n; z.nblk = m.nblk; z.consumed = m.consumed; z.rounds = 0;
+    z.bits_in = a.bits_in; z.nbits_in = nbits_in; z.crc_in = crc_in;
+    if (m.nblk) {
+        const u32 N = m.nrle, nb = m.nblk, G = (N + 255) / 256;
+        k_bz_gather<<<(m.consumed + 255) / 256, 256, 0, st>>>(a, m.consumed);
+        k_bz_crc<<<nb, 1024, 0, st>>>(a);
+        CK_CUDA(ctx, cudaEventRecord(z.ev[1], st));
+        // BWT: the first sort over (block, 7 bytes), then rounds over the groups not yet split
+        u32 rbits = 1, bbits = 1;
+        while ((1ull << rbits) < N) rbits++;
+        while ((1u << bbits) < nb) bbits++;
+        u32 *pos = z.pos, *pos2 = z.pos2;
+        k_bz_key0<<<G, 256, 0, st>>>(a, nb, N, z.keyA, z.valA, pos);
+        ctx->launches += 3;
+        u32 mcount = N, sorted = CKB_KEY0_CHARS;
+        for (bool first = true; mcount; first = false) {
+            const u32 gm = (mcount + 255) / 256;
+            if (!first) { k_bz_key<<<gm, 256, 0, st>>>(a, mcount, pos, sorted, rbits, z.keyA, z.valA); ctx->launches++; }
+            const u32 after = first ? sorted : 2 * sorted;     // bytes the rotations are sorted by after this round
+            cub::DoubleBuffer<u64> kb(z.keyA, z.keyB);
+            cub::DoubleBuffer<u32> vb(z.valA, z.valB);
+            tb = z.tmp_bytes;
+            CK_CUDA(ctx, cub::DeviceRadixSort::SortPairs(z.tmp, tb, kb, vb, (int)mcount, 0,
+                                                         first ? (int)(8 * CKB_KEY0_CHARS + bbits) : (int)(2 * rbits), st));
+            k_bz_mark<<<gm, 256, 0, st>>>(a, mcount, kb.Current(), vb.Current(), pos, z.hp);
+            tb = z.tmp_bytes;
+            CK_CUDA(ctx, cub::DeviceScan::InclusiveScan(z.tmp, tb, z.hp, z.hs, BzMax(), (int)mcount, st));
+            k_bz_rank<<<gm, 256, 0, st>>>(a, mcount, kb.Current(), vb.Current(), pos, z.hs, after, z.flag);
+            tb = z.tmp_bytes;
+            CK_CUDA(ctx, cub::DeviceSelect::Flagged(z.tmp, tb, pos, z.flag, pos2, z.result + 3, (int)mcount, st));
+            ctx->launches += 5;
+            CK_CUDA(ctx, cudaGetLastError());
+            CK_CUDA(ctx, cudaMemcpyAsync(z.h_host + 8, z.result + 3, 4, cudaMemcpyDeviceToHost, st));
+            CK_CUDA(ctx, cudaStreamSynchronize(st));
+            mcount = z.h_host[8];
+            std::swap(pos, pos2);
+            sorted = after;
+            z.rounds++;
+        }
+        k_bz_orig<<<G, 256, 0, st>>>(a, N);
+        k_bz_periodic<<<nb, 1, 0, st>>>(a, z.hp);
+        CK_CUDA(ctx, cudaEventRecord(z.ev[2], st));
+        k_bz_mtf<<<nb, 256, 0, st>>>(a);
+        CK_CUDA(ctx, cudaEventRecord(z.ev[3], st));
+        k_bz_huff<<<nb, 256, 0, st>>>(a);
+        CK_CUDA(ctx, cudaEventRecord(z.ev[4], st));
+        CK_CUDA(ctx, cudaMemsetAsync(z.out, 0, (ck_bzip2_bound(n) + 7) / 4 * 4, st));
+        k_bz_place<<<1, CKB_MAX_BLOCKS, 0, st>>>(a, nb);
+        k_bz_pack<<<nb, 256, 0, st>>>(a);
+        CK_CUDA(ctx, cudaEventRecord(z.ev[5], st));
+        ctx->launches += 7;
+        CK_CUDA(ctx, cudaGetLastError());
+        CK_CUDA(ctx, cudaMemcpyAsync(z.h_host + 4, z.result, 12, cudaMemcpyDeviceToHost, st));
+    }
+    s.busy = true; s.bz = true; s.defl = false; s.uniq = false; s.mono = false; s.text = false;
+    return CK_OK;
+}
+
+int ck_bzip2_wait(ck_ctx *ctx, int slot, uint8_t *out, uint64_t *out_bytes, uint64_t *consumed, uint32_t *bits_out,
+                  uint32_t *nbits_out, uint32_t *crc_out)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    Slot &s = ctx->slot[slot];
+    if (!s.busy || !s.bz) return fail(ctx, CK_ERR_STATE, "no matching submit on this slot");
+    if (!out) return fail(ctx, CK_ERR_ARG, "null argument");
+    s.busy = false; s.bz = false;
+    Slot::Bzip2 &z = s.bz2;
+    CK_CUDA(ctx, cudaStreamSynchronize(z.stream));
+    u64 whole = 0, cons = 0;
+    u32 bits = z.bits_in, nbits = z.nbits_in, crc = z.crc_in;
+    if (z.nblk) {
+        const u64 total = (u64)z.h_host[4] | (u64)z.h_host[5] << 32, copy = (total + 7) / 8;
+        if (copy > ck_bzip2_bound(z.n)) return fail(ctx, CK_ERR_CUDA, "bzip2 output exceeds its bound");
+        CK_CUDA(ctx, cudaMemcpyAsync(out, z.out, copy, cudaMemcpyDeviceToHost, z.stream));
+        CK_CUDA(ctx, cudaStreamSynchronize(z.stream));
+        whole = total / 8;
+        nbits = (u32)(total % 8);
+        bits = nbits ? out[whole] >> (8 - nbits) : 0;
+        crc = z.h_host[6];
+        cons = z.consumed;
+    }
+    if (out_bytes) *out_bytes = whole;
+    if (consumed) *consumed = cons;
+    if (bits_out) *bits_out = bits;
+    if (nbits_out) *nbits_out = nbits;
+    if (crc_out) *crc_out = crc;
+    return CK_OK;
+}
+
+int ck_bzip2_stats(ck_ctx *ctx, int slot, float *stage_ms, uint32_t *bwt_rounds)
+{
+    if (!ctx) return CK_ERR_ARG;
+    if (slot < 0 || slot > 1) return fail(ctx, CK_ERR_ARG, "slot must be 0 or 1");
+    if (!stage_ms) return fail(ctx, CK_ERR_ARG, "null argument");
+    Slot &s = ctx->slot[slot];
+    if (s.busy && s.bz) return fail(ctx, CK_ERR_STATE, "call ck_bzip2_wait first");
+    const Slot::Bzip2 &z = s.bz2;
+    for (int k = 0; k < 5; k++) {
+        stage_ms[k] = 0.f;
+        if (z.nblk) CK_CUDA(ctx, cudaEventElapsedTime(&stage_ms[k], z.ev[k], z.ev[k + 1]));
+    }
+    if (bwt_rounds) *bwt_rounds = z.rounds;
     return CK_OK;
 }
 

@@ -373,6 +373,34 @@ int ck_deflate_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, uint64_t n, c
                       uint32_t crc_in);
 int ck_deflate_wait(ck_ctx *ctx, int slot, uint8_t *out, uint64_t *out_bytes, uint32_t *crc_out);
 
+/* ---- bzip2 on the device: the `.bz2` output of `circkit ... -o out.bz2` (src/utils.rs:29-72, the bzip2 crate at level 9) --
+ * The output is byte for byte that of libbzip2 1.0.8 at level 9 (Python's bz2.compress(data, 9)).
+ * ck_bzip2_submit takes n bytes (1 .. CK_BZIP2_MAX_BYTES) of one stream on one of the two slots: the stream from its first
+ * raw byte not yet in a written block (the previous call's unconsumed tail, then new bytes).  It writes every complete block
+ * of them -- every block when `final` is set, which also ends the last run -- as one bit string that starts after the
+ * nbits_in (0..7) pending bits held in the low bits of bits_in.  A block is complete when the RLE1 token that ends it is
+ * followed by another token; a call that is not final never uses the input's last token, which may still grow.
+ * ck_bzip2_wait copies the whole bytes of that bit string (*out_bytes of them; `out` must hold ck_bzip2_bound(n) bytes) and
+ * gives the bits left over (*nbits_out < 8 of them in the low bits of *bits_out), *consumed = the leading input bytes the
+ * written blocks cover (the caller keeps bytes[consumed:] as the next call's tail) and the stream's combined CRC continued
+ * from crc_in (crc = rotl(crc, 1) ^ block CRC per block).  The stream header "BZh9" and the end-of-stream marker, combined
+ * CRC and padding are the caller's.  A call that completes no block writes nothing: consumed 0, the bits and CRC unchanged.
+ * A tail is at most one block's raw extent (under 46 MB), so tail plus new bytes always fits one call.
+ * Slot state, return codes and the stream of its own are as for ck_deflate_*: it works on a context with no batch staging;
+ * n == 0, n > CK_BZIP2_MAX_BYTES, nbits_in > 7 or a NULL pointer -> CK_ERR_ARG.  The submit runs the block cuts and the
+ * sort before it returns (so `bytes` may be reused then); move-to-front, the tables and the packing finish by the wait.
+ * The slot's first bzip2 call allocates its buffers (about 85 bytes of HBM per input byte of the largest call so far,
+ * rounded up to a power of two), so contexts that never write bzip2 use no more device memory.
+ * ck_bzip2_stats gives the device time of the last call's stages in ms (RLE1 and cuts, BWT, MTF, tables, pack) and its
+ * number of BWT sort rounds; call it after the wait. */
+#define CK_BZIP2_MAX_BYTES (64ull << 20)
+uint64_t ck_bzip2_bound(uint64_t n);     /* out bytes to provide for n input bytes */
+int ck_bzip2_submit(ck_ctx *ctx, int slot, const uint8_t *bytes, uint64_t n, int final, uint32_t bits_in,
+                    uint32_t nbits_in, uint32_t crc_in);
+int ck_bzip2_wait(ck_ctx *ctx, int slot, uint8_t *out, uint64_t *out_bytes, uint64_t *consumed, uint32_t *bits_out,
+                  uint32_t *nbits_out, uint32_t *crc_out);
+int ck_bzip2_stats(ck_ctx *ctx, int slot, float *stage_ms /* 5 */, uint32_t *bwt_rounds);
+
 /* number of kernels this context has launched so far (bench.py's gpu_launches) */
 uint64_t ck_launch_count(const ck_ctx *ctx);
 /* per-class kernel timing for the roofline: when enabled, every length/alphabet-class launch is bracketed
